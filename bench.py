@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our CUDA path (one rank per GPU under torchrun)
   python bench.py --impl reference [...]                         the reference-structured CPU path (oracle port)
+  python bench.py [...] --dump-outputs DIR                       also write the last timed step's outputs (see dump_outputs)
 
 One "step" = one pass of the fused step kernel over every env of every rank, actions read from HBM,
 obs / reward / reset / progress written to HBM (SURVEY 8d "mode A").  Workload = BASELINE configs[1]:
@@ -64,7 +65,50 @@ def parse():
                         "every rank only reads its own vector, as a one-GPU run does)")
     p.add_argument("--seed", type=int, default=0)
     p.add_argument("--roofline-only", action="store_true", help="profiling aid: run only the 1 Mi-env roofline region")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (see dump_outputs)")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    return a
+
+
+DUMP_MAX_BYTES = 64 << 20          # every file of one `--dump-outputs` run together (all ranks), .npy headers included
+
+
+def _npy_bytes(a):
+    """Size of the file `np.save` writes for `a`: the .npy header, then the raw data."""
+    import io
+    import numpy as np
+    f = io.BytesIO()
+    np.lib.format.write_array_header_1_0(f, np.lib.format.header_data_from_array_1_0(a))
+    return f.tell() + a.nbytes
+
+
+def dump_outputs(out_dir, per_env, whole=None, suffix="", max_bytes=DUMP_MAX_BYTES):
+    """Writes the arrays of `per_env` (name -> tensor with one row per env) and of `whole` (name -> small tensor, written whole)
+    as <out_dir>/<name><suffix>.npy, so that two builds can be compared output for output: float64 stays float64, other
+    floating outputs become float32 and integer / flag outputs float64.  When the files would exceed `max_bytes` together,
+    every per-env array keeps the same fixed, seeded sample of env rows (numpy default_rng(0), sorted)."""
+    import numpy as np
+
+    def host(t):
+        a = t.detach().cpu().numpy()
+        return a.astype(np.float64 if a.dtype == np.float64 or a.dtype.kind != "f" else np.float32)
+    rows_out = {name: host(t) for name, t in per_env.items()}
+    whole = {name: host(t) for name, t in (whole or {}).items()}
+    n = len(next(iter(rows_out.values())))
+    total = sum(_npy_bytes(a) for a in (*rows_out.values(), *whole.values()))
+    if total > max_bytes:
+        row_bytes = sum(a.nbytes // n for a in rows_out.values())
+        fixed = total - n * row_bytes                  # headers (not longer for fewer rows) and the whole arrays
+        rows = np.sort(np.random.default_rng(0).choice(n, (max_bytes - fixed) // row_bytes, replace=False))
+        rows_out = {name: a[rows] for name, a in rows_out.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in {**rows_out, **whole}.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
 
 
 def task_cfg_kwargs():
@@ -431,6 +475,19 @@ def run_ours(args):
         dist.all_reduce(tr, op=dist.ReduceOp.MAX)
     rot_ms = float(tr.item())
     value_rot = world * n * K / (rot_ms * 1e-3)
+    if args.dump_outputs:
+        # what the caller of the timed path holds after it: the per-env outputs of timed step K - 1 (its shard's buffers are not
+        # touched again before this), the last metrics vector read inside the timed graph and, with the peer exchange, the sum
+        # over the ranks it produced.  Graph 1 (steps 0 .. chunk_r - 1) is replayed reps_r times, then graph 2 runs the rest.
+        _, o_, r_, rs_, pg_, to_, er_ = shards[(K - 1) % S]
+        reads = [k for k in range(reps_r * chunk_r, K) if (k % METRICS_EVERY) == METRICS_PHASE] or \
+                [k for k in range(chunk_r) if (k % METRICS_EVERY) == METRICS_PHASE]
+        whole = {"metrics": metrics_ring[(reads[-1] // METRICS_EVERY) % n_reads]} if reads else {}
+        if peer is not None:
+            whole["metrics_sum"] = metrics_sum
+        dump_outputs(args.dump_outputs, {"obs": o_, "reward": r_, "reset": rs_, "progress": pg_, "time_outs": to_,
+                                         "episode_return": er_}, whole, f"_rank{rank}" if world > 1 else "",
+                     DUMP_MAX_BYTES // world)
     peer_check = None
     if peer is not None:
         # outside the timed region: the sum the last in-graph exchange produced equals an NCCL all-reduce of the vectors it was fed

@@ -282,8 +282,11 @@ def main():
     sd = {"sd__" + k: v.numpy() for k, v in actor.state_dict().items()}
     np.savez_compressed(os.path.join(OUT, "rpo_lstm_actor.npz"), obs=obs.numpy(), done=done.numpy(), h0=h0.numpy(), c0=c0.numpy(),
                         a1=a1.numpy(), lp1=lp1.numpy(), en1=en1.numpy(), h1=h1.numpy(), c1=c1.numpy(),
-                        aT=aT.numpy(), lpT=lpT.numpy(), enT=enT.numpy(), hT=hT.numpy(), cT=cT.numpy(), **sd)
-    made.append("rpo_lstm_actor.npz")
+                        aT=aT.numpy(), lpT=lpT.numpy(), enT=enT.numpy(), hT=hT.numpy(), cT=cT.numpy())
+    # the state dict goes into two more files so that every stored file stays under 1 MB
+    np.savez_compressed(os.path.join(OUT, "rpo_lstm_actor_sd_mlp.npz"), **{k: v for k, v in sd.items() if not k.startswith("sd__lstm.")})
+    np.savez_compressed(os.path.join(OUT, "rpo_lstm_actor_sd_lstm.npz"), **{k: v for k, v in sd.items() if k.startswith("sd__lstm.")})
+    made += ["rpo_lstm_actor.npz", "rpo_lstm_actor_sd_mlp.npz", "rpo_lstm_actor_sd_lstm.npz"]
     print("wrote", made)
 
 

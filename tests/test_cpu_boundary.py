@@ -11,13 +11,17 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.fixture(scope="module")
-def lib():
+def _build_script():
     import importlib.util
     spec = importlib.util.spec_from_file_location("_ozl_build", os.path.join(ROOT, "ouzelum_b200", "build.py"))
     build = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(build)
-    build.build()                      # no-op when the in-tree .so is newer than its sources
+    return build
+
+
+@pytest.fixture(scope="module")
+def lib():
+    _build_script().build()            # no-op when the in-tree .so is newer than its sources
     from ouzelum_b200 import _lib
     return _lib
 
@@ -41,10 +45,11 @@ def test_library_exports_every_declared_symbol(lib):
 
 def test_library_is_sm100a_only_and_uses_bulk_copy(lib):
     import subprocess
-    out = subprocess.run(["cuobjdump", "-lelf", lib.LIB_PATH], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(_build_script().NVCC), "cuobjdump")     # the toolkit that built the library, PATH or not
+    out = subprocess.run([cuobjdump, "-lelf", lib.LIB_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
-    sass = subprocess.run(["cuobjdump", "-sass", lib.LIB_PATH], capture_output=True, text=True).stdout
+    sass = subprocess.run([cuobjdump, "-sass", lib.LIB_PATH], capture_output=True, text=True).stdout
     assert "UBLKCP" in sass                      # TMA bulk store of the observation tile (Blackwell/Hopper async copy engine)
     assert "quad_step_kernel" in sass
 
@@ -98,11 +103,10 @@ def test_philox_known_answers():
     assert list(mulhi(r, 2000)) == [0, 0, 0, 1999]
 
 
-def test_product_refuses_to_run_without_cuda(lib):
+def test_product_refuses_to_run_without_cuda(lib, monkeypatch):
     import torch
     import ouzelum_b200
-    if torch.cuda.is_available():
-        pytest.skip("CUDA present")
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)       # on a machine with a GPU the product must see none
     with pytest.raises(RuntimeError, match="no CPU"):
         ouzelum_b200.make(0, "Ouzelum", 16, sim_device="cpu", rl_device="cpu")
     with pytest.raises(RuntimeError, match="no CUDA device|no CPU"):
@@ -121,6 +125,52 @@ def test_product_never_imports_the_oracle():
             if f.endswith((".py", ".cu", ".cuh", ".h")):
                 txt = open(os.path.join(dirpath, f)).read()
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", txt, flags=re.M), f"{f} imports the oracle"
+
+
+def _repository_files():
+    """Paths (relative to the root) of the repository's files: what git tracks in a checkout; in a copy of the tree without
+    .git, every file that the patterns of .gitignore do not exclude (last matching pattern wins, `!` re-includes)."""
+    import fnmatch
+    import subprocess
+    if os.path.isdir(os.path.join(ROOT, ".git")):
+        r = subprocess.run(["git", "-C", ROOT, "ls-files", "-z"], capture_output=True, text=True, timeout=120)
+        if r.returncode == 0:
+            return [f for f in r.stdout.split("\0") if f]
+    rules = []
+    for line in open(os.path.join(ROOT, ".gitignore")).read().splitlines():
+        line = line.strip()
+        if line and not line.startswith("#"):
+            rules.append((line.startswith("!"), line.lstrip("!")))
+
+    def ignored(rel):
+        parts, out = rel.split("/"), False
+        for negate, pat in rules:
+            dir_only, pat = pat.endswith("/"), pat.strip("/")
+            heads = parts[:-1] if dir_only else parts              # a directory pattern matches the directories above the file
+            if "/" in pat:                                         # anchored at the root
+                hit = any(fnmatch.fnmatchcase("/".join(parts[:i + 1]), pat) for i in range(len(heads)))
+            else:
+                hit = any(fnmatch.fnmatchcase(p, pat) for p in heads)
+            if hit:
+                out = not negate
+        return out
+    files = []
+    for dirpath, dirnames, filenames in os.walk(ROOT):
+        dirnames[:] = [d for d in dirnames if d != ".git"]
+        for f in filenames:
+            rel = os.path.relpath(os.path.join(dirpath, f), ROOT).replace(os.sep, "/")
+            if not ignored(rel):
+                files.append(rel)
+    return files
+
+
+def test_every_repository_file_is_at_most_1_mb():
+    """Stored test vectors are sampled or split so that no file of the repository exceeds 1 MB (10^6 bytes)."""
+    files = _repository_files()
+    assert "bench.py" in files and "tests/golden/rpo_lstm_actor.npz" in files and "ouzelum_b200/libouzelum_b200.so" not in files
+    sizes = {f: os.path.getsize(os.path.join(ROOT, f)) for f in files if os.path.isfile(os.path.join(ROOT, f))}
+    big = {f: s for f, s in sizes.items() if s > 1_000_000}
+    assert not big, big
 
 
 def test_task_config_mirrors_yaml():
@@ -152,13 +202,17 @@ def test_recurrent_actor_cell_equals_nn_lstm():
 
 def test_recurrent_actor_equals_reference_actor_fixture():
     """(f)1: `RecurrentActor` against the reference's UNMODIFIED `RPO-LSTM/model.py` Actor (tests/golden/rpo_lstm_actor.npz, made
-    by running that module on CPU): it must LOAD the reference's state dict (the `<tag>_actor` checkpoint format of
-    RPO-LSTM/agent.py:136-147) and reproduce log-prob, entropy and LSTM state of a single step and of a 3-step sequence to 1e-6."""
+    by running that module on CPU; its state dict is stored in rpo_lstm_actor_sd_{mlp,lstm}.npz): it must LOAD the reference's
+    state dict (the `<tag>_actor` checkpoint format of RPO-LSTM/agent.py:136-147) and reproduce log-prob, entropy and LSTM state
+    of a single step and of a 3-step sequence to 1e-6."""
     import os
     import torch
     from ouzelum_b200.rollout import RecurrentActor
-    d = np.load(os.path.join(os.path.dirname(__file__), "golden", "rpo_lstm_actor.npz"))
-    sd = {k[4:]: torch.from_numpy(d[k]) for k in d.files if k.startswith("sd__")}
+    d = {}
+    for f in ("rpo_lstm_actor.npz", "rpo_lstm_actor_sd_mlp.npz", "rpo_lstm_actor_sd_lstm.npz"):
+        with np.load(os.path.join(os.path.dirname(__file__), "golden", f)) as z:
+            d.update({k: z[k] for k in z.files})
+    sd = {k[4:]: torch.from_numpy(d[k]) for k in d if k.startswith("sd__")}
     a = RecurrentActor()
     assert set(sd) == set(a.state_dict())                       # same parameter names and shapes as the reference module
     a.load_state_dict(sd, strict=True)
@@ -263,18 +317,56 @@ def test_compat_shims_resolve_the_reference_trainer_imports(lib, tmp_path):
                 sys.modules[k] = v
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/isaacgymenvs/RPO-LSTM/main.py") or __import__("torch").cuda.is_available(),
-                    reason="needs the reference checkout (build container only) and no GPU")
-def test_reference_trainer_reaches_make_through_the_compat_launcher():
-    """The reference's own RPO-LSTM/main.py, unmodified, through `python -m ouzelum_b200.compat`: every import resolves and the
-    script gets as far as isaacgymenvs.make(), which refuses loudly here because there is no GPU (no CPU fallback)."""
+_TRAINER_MAIN = '''
+import argparse
+
+import gym
+import isaacgym  # noqa: F401
+import isaacgymenvs
+import torch
+from isaacgymenvs.utils.POMDP import POMDPWrapper
+from torch.utils.tensorboard import SummaryWriter
+
+from agent import PPO
+
+parser = argparse.ArgumentParser()
+parser.add_argument("--env", default="Landing")
+parser.add_argument("--num_envs", type=int, default=4096)
+parser.add_argument("--POMDP", default="flicker")
+parser.add_argument("--pomdp_prob", type=float, default=0.1)
+parser.add_argument("--total_steps", type=int, default=30000000)
+args = parser.parse_args()
+assert (args.env, args.num_envs, args.POMDP, args.pomdp_prob) == ("Landing", 4096, "flicker", 0.1)
+assert issubclass(PPO, gym.Wrapper) and SummaryWriter is not None
+POMDP = POMDPWrapper(pomdp=args.POMDP, pomdp_prob=args.pomdp_prob)
+# the call of RPO-LSTM/main.py:41 as SURVEY.md section 3.1 records it
+envs = isaacgymenvs.make(seed=0, task="Landing", num_envs=4096, sim_device="cuda:0", rl_device="cuda:0", graphics_device_id=-1, headless=True, force_render=True)
+'''
+
+_TRAINER_AGENT = '''
+import gym
+
+
+class PPO(gym.Wrapper):
+    pass
+'''
+
+
+def test_reference_trainer_reaches_make_through_the_compat_launcher(tmp_path):
+    """A trainer laid out like the reference's RPO-LSTM/main.py (the same gym / isaacgym / isaacgymenvs / POMDP / tensorboard
+    imports, `from agent import PPO` from a file beside it, the argparse flags and command line of SURVEY.md section 1, the
+    make() call of section 3.1) through `python -m ouzelum_b200.compat`: every import resolves and the script gets as far as
+    isaacgymenvs.make(), which refuses loudly because no CUDA device is visible to it (no CPU fallback)."""
     import subprocess
     import sys
-    import tempfile
-    with tempfile.TemporaryDirectory() as tmp:
-        r = subprocess.run([sys.executable, "-m", "ouzelum_b200.compat", "/root/reference/isaacgymenvs/RPO-LSTM/main.py",
-                            "--num_envs", "64", "--total_steps", "100"], cwd=tmp, capture_output=True, text=True, timeout=300,
-                           env={**os.environ, "PYTHONPATH": ROOT})
+    trainer = tmp_path / "trainer"
+    trainer.mkdir()
+    (trainer / "main.py").write_text(_TRAINER_MAIN)
+    (trainer / "agent.py").write_text(_TRAINER_AGENT)
+    r = subprocess.run([sys.executable, "-m", "ouzelum_b200.compat", str(trainer / "main.py"),
+                        "--env", "Landing", "--num_envs", "4096", "--POMDP", "flicker", "--pomdp_prob", "0.1"],
+                       cwd=tmp_path, capture_output=True, text=True, timeout=300,
+                       env={**os.environ, "PYTHONPATH": ROOT, "CUDA_VISIBLE_DEVICES": ""})
     assert r.returncode != 0
     assert "no CUDA device is visible and there is no CPU fallback" in r.stderr, r.stderr[-2000:]
     assert "isaacgymenvs.make" in r.stderr or "main.py" in r.stderr
