@@ -26,9 +26,10 @@
 extern "C" {
 #endif
 
-#define OZL_ABI_VERSION 4   /* 3: ozl_cfg.dr[] (domain-randomisation schema), per-env yaw_km (params8), wrench_warmup_steps,
+#define OZL_ABI_VERSION 5   /* 3: ozl_cfg.dr[] (domain-randomisation schema), per-env yaw_km (params8), wrench_warmup_steps,
                                ozl_ekf_lee_args.num_envs_total, i64 reset mirror in ozl_host_io
-                               4: (additive) ozl_metrics_xchg_* / ozl_metrics_push / ozl_metrics_sum, ozl_noise_lambda_apply */
+                               4: (additive) ozl_metrics_xchg_* / ozl_metrics_push / ozl_metrics_sum, ozl_noise_lambda_apply
+                               5: (additive) ozl_set_states_output, OZL_STATE_* layout of the privileged critic state */
 
 /* sensor-fault model of isaacgymenvs/utils/POMDP.py:4-42 */
 enum { OZL_POMDP_NONE = 0, OZL_POMDP_FLICKER = 1, OZL_POMDP_NOISE = 2, OZL_POMDP_FLICKER_NOISE = 3 };
@@ -184,6 +185,32 @@ int ozl_step_wrench(ozl_env* env, const float* wrench4, const float* target3, fl
  * counter are untouched.  Lets composite tasks see the post-reset state in their pre-physics code, as the reference does
  * (reset_idx runs first in pre_physics_step, tasks/ekf_lee_landed.py:312-314, lee_landed.py:267-270). */
 int ozl_apply_resets(ozl_env* env, const int64_t* reset, void* stream);
+
+/* Privileged critic state (asymmetric actor-critic: the reference's numStates / states_buf / obs_dict["states"],
+ * tasks/base/vec_task.py:104,121-122,145-151).  OZL_STATES_WIDTH float32 per env, row-major [N, OZL_STATES_WIDTH], written by
+ * the same launch as the observation, from the same post-step registers (an env flagged for reset shows its terminal state).
+ * Every slot is clamped to +-clip_obs like the observation.
+ *   OZL_STATE_OBS .. +12        the CLEAN observation: before the sensor-fault model (pomdp_mode), after the clamp
+ *   OZL_STATE_THRUST .. +3      rotor thrust state T0..T3 / thrust_max
+ *   OZL_STATE_EFF .. +3         per-rotor effectiveness applied this step: 1, except the faulted rotor's effectiveness while its
+ *                               fault is active (all 1 on wrench-actuated steps)
+ *   OZL_STATE_MASS .. _ARM      per-env mass, ixx, iyy, izz, arm / their ozl_cfg values (exactly 1 when not randomised)
+ *   OZL_STATE_THRUST_SCALE      per-env thrust scale (nominal 1)
+ *   OZL_STATE_YAW_KM            per-env yaw_km (raw: its nominal may be 0)
+ *   OZL_STATE_PROGRESS          progress after this step / max_episode_length
+ *   OZL_STATE_POS .. +2         absolute root position / 3 (the observation's scaling; z is the die_z criterion)
+ * Divisions are IEEE float32 divisions; the CPU reference (tests/states_ref.py, on the oracle's state) reproduces the row bit for bit. */
+enum { OZL_STATE_OBS = 0, OZL_STATE_THRUST = 13, OZL_STATE_EFF = 17, OZL_STATE_MASS = 21, OZL_STATE_IXX = 22, OZL_STATE_IYY = 23,
+       OZL_STATE_IZZ = 24, OZL_STATE_ARM = 25, OZL_STATE_THRUST_SCALE = 26, OZL_STATE_YAW_KM = 27, OZL_STATE_PROGRESS = 28,
+       OZL_STATE_POS = 29, OZL_STATES_WIDTH = 32 };
+
+/* Register a caller-owned [N, OZL_STATES_WIDTH] f32 buffer (16-byte aligned; any device-writable pointer) that every later
+ * launch of ozl_step, ozl_step_tracking, ozl_step_wrench, ozl_step_host*, ozl_landing_step and ozl_lee_landed_step fills with
+ * the privileged state above.  states = NULL unregisters (the steps then run the kernels without the output).
+ * `width` must be OZL_STATES_WIDTH.  A captured CUDA graph keeps the buffer that was registered when it was captured.
+ * While a buffer is registered, ozl_rollout and ozl_ekf_lee_landed_step refuse to run (non-zero return, ozl_last_error()):
+ * their kernels do not write the state. */
+int ozl_set_states_output(ozl_env* env, float* states, int32_t width);
 
 /* Mode-B throughput entry: K steps in ONE launch, state held in registers, actions a = 2u-1 drawn
  * in-kernel from the counter RNG; obs/rew are written for the LAST step only, reset/progress are

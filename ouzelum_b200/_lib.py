@@ -9,7 +9,20 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("OUZELUM_B200_LIB") or os.path.join(_HERE, "libouzelum_b200.so")   # override: kernel experiments only
 
-OZL_ABI_VERSION = 4
+OZL_ABI_VERSION = 5
+
+
+def _header_enum(prefix):
+    """`{name: value}` of the enumerators of include/ouzelum_b200.h whose name starts with `prefix` (the header is the one
+    statement of such layouts; the library is compiled from the same file)."""
+    import re
+    with open(os.path.join(_HERE, "..", "include", "ouzelum_b200.h")) as f:
+        return {k: int(v) for k, v in re.findall(r"\b(" + prefix + r"\w*)\s*=\s*(\d+)", f.read())}
+
+
+# privileged critic state written by the step kernels (ozl_set_states_output): slot indices OZL_STATE_* and the row width
+STATES_LAYOUT = _header_enum("OZL_STATE")
+STATES_WIDTH = STATES_LAYOUT["OZL_STATES_WIDTH"]
 
 
 DR_NONE, DR_UNIFORM, DR_LOGUNIFORM, DR_GAUSSIAN = 0, 1, 2, 3
@@ -164,6 +177,7 @@ _SIGS = {
     "ozl_step_tracking": (C.c_int, [_P] * 10),
     "ozl_step_wrench": (C.c_int, [_P] * 10),
     "ozl_rollout": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P]),
+    "ozl_set_states_output": (C.c_int, [_P, _P, C.c_int32]),
     "ozl_get_state": (C.c_int, [_P] * 6),
     "ozl_set_state": (C.c_int, [_P] * 6),
     "ozl_get_params": (C.c_int, [_P] * 4),

@@ -81,6 +81,10 @@ struct ozl_env {
     int chain_mode;                     // OZL_EKF_CHAIN: 0 = never chain, 1 = chain launches that are provably adjacent in a stream capture
     unsigned long long chain_capture_id;
     void* chain_last_node;
+    // privileged critic-state output (ozl_set_states_output): caller's [N, OZL_STATES_WIDTH] buffer or NULL, and the 2-D tensor
+    // map over it (box [128 rows][32], 128-byte swizzle) through which the step kernels store one states tile per 128 envs
+    float* states;
+    alignas(64) unsigned char states_tmap[128];
 };
 
 // Step launches go through cudaLaunchKernelEx so that they can carry the programmatic-stream-serialization attribute (PDL):

@@ -5,6 +5,7 @@
 #include <cstring>
 #include <cstdlib>
 #include <cmath>
+#include <cuda.h>              // CUtensorMap (types only: the encoder is looked up through cudaGetDriverEntryPoint)
 #include "internal.h"
 #include "bulk_copy.cuh"
 #include "quad_io.cuh"
@@ -51,14 +52,31 @@ struct FrontArgs {
     float4* wrench_out;  // optional [N] debug output
 };
 
-template <int BLOCK, int FRONT>
+// One env's row of the [kTile, OZL_STATES_WIDTH] states tile in shared memory, laid out as CU_TENSOR_MAP_SWIZZLE_128B expects
+// (16-byte chunk k of row r sits at chunk k ^ (r & 7); the tile is 1024-byte aligned): the eight 16-byte stores of a quarter-warp
+// land in eight different bank groups, where plain 128-byte rows would put all of them in the same four banks (8-way conflict).
+// The tensor-map store un-swizzles the tile into the caller's row-major [N, 32] buffer.
+__device__ __forceinline__ void stage_states_row(float* tile, int r, const float clean[13], const Env& e, const StepOut& o,
+                                                 const DevCfg& c) {
+    float s[OZL_STATES_WIDTH];
+    states_row(s, clean, e, o, c);
+    float4* row = reinterpret_cast<float4*>(tile + r * OZL_STATES_WIDTH);
+#pragma unroll
+    for (int k = 0; k < OZL_STATES_WIDTH / 4; ++k) row[k ^ (r & 7)] = make_float4(s[4 * k], s[4 * k + 1], s[4 * k + 2], s[4 * k + 3]);
+}
+
+// STATES: also write the privileged critic state (ozl_set_states_output) through `states_map`; the STATES = false instantiations
+// are the kernels without that output.
+template <int BLOCK, int FRONT, bool STATES>
 __global__ void __launch_bounds__(BLOCK, OZL_STEP_MINB)
 quad_step_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ actions, float* __restrict__ obs,
                  float* __restrict__ rew, int64_t* __restrict__ reset, int64_t* __restrict__ progress,
                  uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, const float* __restrict__ target_in,
                  const int act_mode, uint8_t* __restrict__ done_u8, int64_t* __restrict__ reset_mirror, const int obs_bulk,
-                 const int64_t env0, const FrontArgs fa, volatile unsigned int* host_done, const unsigned int host_seq) {
+                 const int64_t env0, const FrontArgs fa, volatile unsigned int* host_done, const unsigned int host_seq,
+                 const __grid_constant__ CUtensorMap states_map) {
     __shared__ __align__(16) float s_obs[BLOCK * 13];
+    __shared__ __align__(1024) float s_states[STATES ? BLOCK * OZL_STATES_WIDTH : 4];
     __shared__ uint64_t s_step;
 
     const int64_t base = env0 + (int64_t)blockIdx.x * BLOCK;
@@ -110,6 +128,7 @@ quad_step_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ act
         } else {
             env_step(e, act, prog, rst, genv, step, c, o, act_mode, tptr);
         }
+        if constexpr (STATES) stage_states_row(s_states, threadIdx.x, o.obs, e, o, c);
         obs_epilogue(o.obs, genv, step, flicker_blackout(step, c), c);
 
         store_dynamic(pl, i, e);
@@ -126,6 +145,8 @@ quad_step_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ act
     }
 #if OZL_OBS_BULK
     fence_proxy_async_smem();          // make the generic-proxy smem writes visible to the bulk-copy (async) proxy
+#else
+    if constexpr (STATES) fence_proxy_async_smem();
 #endif
     __syncthreads();
     // [N,13] row-major observation tile of this block is contiguous: write it with full 16-byte lanes
@@ -156,11 +177,17 @@ quad_step_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ act
             for (int k = threadIdx.x; k < nflt; k += BLOCK) dst[k] = s_obs[k];
         }
     }
+    // [BLOCK, 32] states tile: one tensor-map store (rows at and beyond num_envs are clipped)
+    if constexpr (STATES) {
+        if (threadIdx.x == 0) tma_store_2d(&states_map, 0, (int32_t)base, s_states);
+    }
     // one work unit per block; block 0 of the full-range launch also retires the padding (env0 != 0: ragged-tail launch
     // behind the TMA kernel, which has retired the padding already)
     block_epilogue<BLOCK>(c, pl, valid, o, n_here, 1ull + ((blockIdx.x == 0 && env0 == 0) ? (unsigned long long)c.step_pad : 0ull));
 #if OZL_OBS_BULK
-    if (threadIdx.x == 0) bulk_wait_read_all();   // s_obs must stay alive until the bulk copy has read it
+    if (threadIdx.x == 0) bulk_wait_read_all();   // s_obs (and s_states) must stay alive until the bulk copies have read them
+#else
+    if constexpr (STATES) { if (threadIdx.x == 0) bulk_wait_read_all(); }
 #endif
     // Host consumer: completion word.  Every block orders its zero-copy result stores before a ticket (the barrier makes the
     // block's stores visible to thread 0, the system-scope fence orders them before the ticket); the block that draws the last
@@ -169,6 +196,7 @@ quad_step_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ act
     if (host_done) {
         __syncthreads();
         if (threadIdx.x == 0) {
+            if constexpr (STATES) bulk_wait_all();     // the states tile has reached memory before the ticket
             __threadfence_system();
             const unsigned long long t = atomicAdd(pl.ctrl + 6, 1ull);
             if (t == (unsigned long long)gridDim.x - 1ull) {
@@ -198,12 +226,15 @@ constexpr int kTmaStageBytes = kTmaRstOff + kTile * 8;            // 19456
 #ifndef OZL_TMA_MINB
 #define OZL_TMA_MINB 5
 #endif
+template <bool STATES>
 __global__ void __launch_bounds__(kTile, OZL_TMA_MINB)
 quad_step_tma_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ actions, float* __restrict__ obs,
                      float* __restrict__ rew, int64_t* __restrict__ reset, int64_t* __restrict__ progress,
-                     uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, const int64_t full_tiles) {
+                     uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, const int64_t full_tiles,
+                     const __grid_constant__ CUtensorMap states_map) {
     __shared__ __align__(128) unsigned char s_stage[kTmaStageBytes];
     __shared__ __align__(16) float s_obs[kTile * 13];
+    __shared__ __align__(1024) float s_states[STATES ? kTile * OZL_STATES_WIDTH : 4];   // 16 KB: 5 CTAs/SM still fit
     __shared__ __align__(8) uint64_t s_bar;
     __shared__ double s_m[kTile / 32][11];
     const int tid = threadIdx.x;
@@ -260,7 +291,7 @@ quad_step_tma_kernel(const DevCfg c, const Planes pl, const float4* __restrict__
         const int64_t prog = reinterpret_cast<const int64_t*>(s_stage + kTmaProgOff)[tid];
         const bool rst = reinterpret_cast<const int64_t*>(s_stage + kTmaRstOff)[tid] != 0;
         if (tid == 0) {
-            bulk_wait_read_all();                // previous tile's observation store has finished reading s_obs
+            bulk_wait_read_all();                // previous tile's observation (and states) stores have finished reading s_obs
             s_next = nxt;
         }
         __syncthreads();                         // everyone has copied the stage out, s_obs is free, s_next is published
@@ -279,6 +310,7 @@ quad_step_tma_kernel(const DevCfg c, const Planes pl, const float4* __restrict__
         const uint32_t genv = c.env_id_base + (uint32_t)i;
         StepOut o;
         env_step(e, act, prog, rst, genv, step, c, o, ACT_ROTORS, nullptr);
+        if constexpr (STATES) stage_states_row(s_states, tid, o.obs, e, o, c);
         obs_epilogue(o.obs, genv, step, blackout, c);
         store_dynamic(pl, i, e);
         if (o.static_dirty) store_static(pl, i, e);
@@ -292,6 +324,9 @@ quad_step_tma_kernel(const DevCfg c, const Planes pl, const float4* __restrict__
         fence_proxy_async_smem();
         __syncthreads();
         if (tid == 0) bulk_store_s2g(obs + tile * (kTile * 13), s_obs, kTile * 13 * 4);
+        if constexpr (STATES) {
+            if (tid == 0) tma_store_2d(&states_map, 0, (int32_t)(tile * kTile), s_states);
+        }
         // metrics
         m_rew += (double)o.rew;
         if (o.reset) { m_ret += (double)o.ep_ret_done; m_len += (int)o.prog; }
@@ -723,6 +758,8 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
 
     ozl_env* e = new ozl_env();
     e->cfg = *cfg;
+    e->states = nullptr;
+    memset(e->states_tmap, 0, sizeof(e->states_tmap));
     derive_dev_cfg(*cfg, e->dev);
     e->device = device;
     e->sm_count = prop.multiProcessorCount;
@@ -807,10 +844,13 @@ extern "C" int ozl_reset_all(ozl_env* env, uint64_t seed, void* stream) {
 constexpr int kStepBlock = OZL_STEP_BLOCK;
 static_assert(kStepBlock == kTile, "the step counter retires one work unit per 128-env tile == one block of the generic kernel");
 
-static int launch_step(ozl_env* env, const float* actions, const float* target_in, int act_mode, float* obs, float* rew,
-                       int64_t* reset, int64_t* progress, uint8_t* timeout, float* ep_ret, void* stream, const char* who,
-                       uint8_t* done_u8 = nullptr, int obs_bulk = 1, int64_t* reset_mirror = nullptr, int host_flag = 0) {
-    if (!env) return set_error("%s: env is NULL", who);
+// The states tensor map of the handle (zeros while no states buffer is registered: the STATES = false kernels never read it)
+static inline const CUtensorMap& states_map(const ozl_env* env) { return *reinterpret_cast<const CUtensorMap*>(env->states_tmap); }
+
+template <bool STATES>
+static int launch_step_t(ozl_env* env, const float* actions, const float* target_in, int act_mode, float* obs, float* rew,
+                         int64_t* reset, int64_t* progress, uint8_t* timeout, float* ep_ret, void* stream, const char* who,
+                         uint8_t* done_u8, int obs_bulk, int64_t* reset_mirror, int host_flag) {
     cudaStream_t st = (cudaStream_t)stream;
     if (!actions || !obs || !rew || !reset || !progress) return set_error("%s: NULL buffer", who);
     if (((uintptr_t)actions & 15) || ((uintptr_t)obs & 15)) return set_error("%s: actions/obs must be 16-byte aligned", who);
@@ -823,22 +863,33 @@ static int launch_step(ozl_env* env, const float* actions, const float* target_i
         // large N: persistent TMA-pipelined kernel over the whole tiles, then one generic block for the ragged tail
         unsigned grid = (unsigned)(full_tiles < resident ? full_tiles : resident);
         while ((full_tiles + grid - 1) / grid > 8192) grid *= 2;     // 16-bit packed metric counters: keep tiles per CTA far below 65535
-        if (launch_pdl(env, quad_step_tma_kernel, dim3(grid), dim3(kTile), st, env->dev, env->pl, (const float4*)actions, obs, rew, reset,
-                       progress, timeout, ep_ret, full_tiles))
+        if (launch_pdl(env, quad_step_tma_kernel<STATES>, dim3(grid), dim3(kTile), st, env->dev, env->pl, (const float4*)actions, obs, rew,
+                       reset, progress, timeout, ep_ret, full_tiles, states_map(env)))
             return check_cuda(cudaGetLastError(), "quad_step_tma_kernel");
         if (tail)
-            quad_step_kernel<kStepBlock, FRONT_NONE><<<1, kStepBlock, 0, st>>>(env->dev, env->pl, (const float4*)actions, obs, rew, reset,
-                                                                              progress, timeout, ep_ret, nullptr, ACT_ROTORS, nullptr,
-                                                                              nullptr, 1, full_tiles * kTile, FrontArgs{},
-                                                                              (volatile unsigned int*)nullptr, 0u);
+            quad_step_kernel<kStepBlock, FRONT_NONE, STATES><<<1, kStepBlock, 0, st>>>(env->dev, env->pl, (const float4*)actions, obs, rew,
+                                                                                      reset, progress, timeout, ep_ret, nullptr, ACT_ROTORS,
+                                                                                      nullptr, nullptr, 1, full_tiles * kTile, FrontArgs{},
+                                                                                      (volatile unsigned int*)nullptr, 0u, states_map(env));
         return check_cuda(cudaGetLastError(), "quad_step_kernel(tail)");
     }
-    if (launch_pdl(env, quad_step_kernel<kStepBlock, FRONT_NONE>, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev, env->pl,
-                   (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, target_in, act_mode, done_u8, reset_mirror,
+    if (launch_pdl(env, quad_step_kernel<kStepBlock, FRONT_NONE, STATES>, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev,
+                   env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, target_in, act_mode, done_u8, reset_mirror,
                    obs_bulk, (int64_t)0, FrontArgs{}, (volatile unsigned int*)(host_flag ? env->host_done : nullptr),
-                   host_flag ? ++env->host_seq : 0u))
+                   host_flag ? ++env->host_seq : 0u, states_map(env)))
         return check_cuda(cudaGetLastError(), "quad_step_kernel");
     return 0;
+}
+
+// The kernels with the states output run whenever the handle has a states buffer registered.
+static int launch_step(ozl_env* env, const float* actions, const float* target_in, int act_mode, float* obs, float* rew,
+                       int64_t* reset, int64_t* progress, uint8_t* timeout, float* ep_ret, void* stream, const char* who,
+                       uint8_t* done_u8 = nullptr, int obs_bulk = 1, int64_t* reset_mirror = nullptr, int host_flag = 0) {
+    if (!env) return set_error("%s: env is NULL", who);
+    return env->states ? launch_step_t<true>(env, actions, target_in, act_mode, obs, rew, reset, progress, timeout, ep_ret, stream, who,
+                                             done_u8, obs_bulk, reset_mirror, host_flag)
+                       : launch_step_t<false>(env, actions, target_in, act_mode, obs, rew, reset, progress, timeout, ep_ret, stream, who,
+                                              done_u8, obs_bulk, reset_mirror, host_flag);
 }
 
 // Landing-family steps with the vehicle (and, for LeeLanded, the controller) in the same launch.
@@ -858,15 +909,16 @@ static int launch_front_step(ozl_env* env, int front, const float* actions, cons
     fa.h.step_ptr = env->pl.ctrl;            // the vehicle follows the handle's device step counter (graph-capturable)
     const int64_t n = env->cfg.num_envs;
     cudaStream_t st = (cudaStream_t)stream;
+#define OZL_LAUNCH_FRONT(F, S, MODE)                                                                                            \
+    launch_pdl(env, quad_step_kernel<kStepBlock, F, S>, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev, env->pl,     \
+               (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, (const float*)nullptr, (int)MODE, (uint8_t*)nullptr, \
+               (int64_t*)nullptr, 1, (int64_t)0, fa, (volatile unsigned int*)nullptr, 0u, states_map(env))
     int rc;
     if (front == FRONT_VEHICLE)
-        rc = launch_pdl(env, quad_step_kernel<kStepBlock, FRONT_VEHICLE>, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev,
-                        env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, (const float*)nullptr, (int)ACT_ROTORS,
-                        (uint8_t*)nullptr, (int64_t*)nullptr, 1, (int64_t)0, fa, (volatile unsigned int*)nullptr, 0u);
+        rc = env->states ? OZL_LAUNCH_FRONT(FRONT_VEHICLE, true, ACT_ROTORS) : OZL_LAUNCH_FRONT(FRONT_VEHICLE, false, ACT_ROTORS);
     else
-        rc = launch_pdl(env, quad_step_kernel<kStepBlock, FRONT_LEE>, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev,
-                        env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, (const float*)nullptr, (int)ACT_WRENCH,
-                        (uint8_t*)nullptr, (int64_t*)nullptr, 1, (int64_t)0, fa, (volatile unsigned int*)nullptr, 0u);
+        rc = env->states ? OZL_LAUNCH_FRONT(FRONT_LEE, true, ACT_WRENCH) : OZL_LAUNCH_FRONT(FRONT_LEE, false, ACT_WRENCH);
+#undef OZL_LAUNCH_FRONT
     if (rc) return check_cuda(cudaGetLastError(), who);
     return 0;
 }
@@ -963,12 +1015,51 @@ extern "C" int ozl_apply_resets(ozl_env* env, const int64_t* reset, void* stream
 extern "C" int ozl_rollout(ozl_env* env, int32_t K, float* obs, float* rew, int64_t* reset, int64_t* progress, void* stream) {
     OZL_ENV_CHECK("ozl_rollout");
     if (K <= 0) return set_error("ozl_rollout: K must be > 0");
+    if (env->states) return set_error("ozl_rollout: a states output is registered (ozl_set_states_output) and the K-step kernel does not write it");
     if (!obs || !rew || !reset || !progress) return set_error("ozl_rollout: NULL buffer");
     quad_rollout_kernel<kStepBlock><<<blocks_for(env->cfg.num_envs, kStepBlock), kStepBlock, 0, st>>>(
         env->dev, env->pl, K, obs, rew, reset, progress);
     if (check_cuda(cudaGetLastError(), "quad_rollout_kernel")) return 1;
     if (K > 1) add_steps_kernel<<<1, 1, 0, st>>>(env->pl, (unsigned long long)(K - 1));
     return check_cuda(cudaGetLastError(), "add_steps_kernel");
+}
+
+extern "C" int ozl_set_states_output(ozl_env* env, float* states, int32_t width) {
+    if (!env) return set_error("ozl_set_states_output: env is NULL");
+    if (width != OZL_STATES_WIDTH)
+        return set_error("ozl_set_states_output: width %d != OZL_STATES_WIDTH (%d)", (int)width, (int)OZL_STATES_WIDTH);
+    if (!states) {
+        env->states = nullptr;
+        memset(env->states_tmap, 0, sizeof(env->states_tmap));
+        return 0;
+    }
+    if ((uintptr_t)states & 15) return set_error("ozl_set_states_output: states must be 16-byte aligned");
+    typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                 const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                 CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+    static EncodeFn fn = nullptr;
+    if (!fn) {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
+            cudaGetLastError();
+            return set_error("ozl_set_states_output: cuTensorMapEncodeTiled is not available from the driver");
+        }
+        fn = (EncodeFn)p;
+    }
+    // [N][32] f32 rows of 128 bytes; box = one 128-env tile, 128-byte swizzle (stage_states_row writes the tile in that layout)
+    const cuuint64_t gdim[2] = {(cuuint64_t)OZL_STATES_WIDTH, (cuuint64_t)env->cfg.num_envs};
+    const cuuint64_t gstr[1] = {(cuuint64_t)OZL_STATES_WIDTH * sizeof(float)};
+    const cuuint32_t box[2] = {(cuuint32_t)OZL_STATES_WIDTH, (cuuint32_t)kTile};
+    const cuuint32_t estr[2] = {1u, 1u};
+    alignas(64) unsigned char m[sizeof(env->states_tmap)];
+    const CUresult r = fn(reinterpret_cast<CUtensorMap*>(m), CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, states, gdim, gstr, box, estr,
+                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) return set_error("ozl_set_states_output: cuTensorMapEncodeTiled failed (%d)", (int)r);
+    memcpy(env->states_tmap, m, sizeof(m));
+    env->states = states;
+    return 0;
 }
 
 extern "C" int ozl_get_state(ozl_env* env, float* root13, float* thrust4, float* target3, float* ep_ret, void* stream) {

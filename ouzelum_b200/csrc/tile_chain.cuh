@@ -26,6 +26,7 @@
 // launches included, runs in mode 0, which behaves exactly like a classic launch.
 #pragma once
 #include <stdint.h>
+#include "bulk_copy.cuh"       // bulk_wait_all
 
 namespace ozl {
 
@@ -37,7 +38,6 @@ __device__ __forceinline__ unsigned long long ld_acquire_u64(const unsigned long
 __device__ __forceinline__ void st_release_u64(unsigned long long* p, unsigned long long v) {
     asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
 }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
 
 // thread 0 of the CTA, after the trigger: wait until the tile's previous step has been released

@@ -84,13 +84,15 @@ class RecurrentActor(nn.Module):
 
 
 class RolloutStorage:
-    """The buffers of main.py:70-78 for any (rollout_steps, num_envs)."""
+    """The buffers of main.py:70-78 for any (rollout_steps, num_envs).  `num_states` > 0 adds `states` [T, N, num_states]: the
+    env's obs_dict["states"] (privileged critic input, env.asymmetric_observations) stored next to `obs`."""
 
-    def __init__(self, steps, num_envs, num_obs, num_actions, device):
+    def __init__(self, steps, num_envs, num_obs, num_actions, device, num_states=0):
         z = lambda *s: torch.zeros(*s, dtype=torch.float32, device=device)
         self.obs, self.pomdps = z(steps, num_envs, num_obs), z(steps, num_envs, num_obs)
         self.actions, self.logprobs = z(steps, num_envs, num_actions), z(steps, num_envs)
         self.rewards, self.dones = z(steps, num_envs), z(steps, num_envs)
+        self.states = z(steps, num_envs, num_states) if num_states > 0 else None
 
 
 @torch.no_grad()
@@ -99,22 +101,34 @@ def collect_rollout(env, actor, storage, state, pomdp=None):
     carried between calls.  Returns the updated state; env-side episode statistics accumulate in `env.metrics()`."""
     steps = storage.obs.shape[0]
     next_obs, pomdp_obs, next_done, lstm_state = state["next_obs"], state["pomdp_obs"], state["next_done"], state["lstm_state"]
+    next_states = state.get("next_states")
     for t in range(steps):
         storage.obs[t], storage.pomdps[t], storage.dones[t] = next_obs, pomdp_obs, next_done
+        if storage.states is not None:
+            storage.states[t] = next_states
         action, logp, _, lstm_state = actor(pomdp_obs, lstm_state, next_done)
         storage.actions[t], storage.logprobs[t] = action, logp
         obs_dict, rew, done, _ = env.step(action)
         next_obs = obs_dict["obs"]
+        if storage.states is not None:
+            next_states = obs_dict["states"]
         storage.rewards[t] = rew
         next_done = done.to(torch.float32)
         pomdp_obs = pomdp.observation(next_obs) if pomdp is not None else next_obs
-    return dict(next_obs=next_obs, pomdp_obs=pomdp_obs, next_done=next_done, lstm_state=lstm_state)
+    out = dict(next_obs=next_obs, pomdp_obs=pomdp_obs, next_done=next_done, lstm_state=lstm_state)
+    if next_states is not None:
+        out["next_states"] = next_states
+    return out
 
 
 def initial_rollout_state(env, actor):
-    obs = env.reset()["obs"]
-    return dict(next_obs=obs, pomdp_obs=obs.clone(), next_done=torch.zeros(env.num_envs, device=obs.device),
-                lstm_state=actor.initial_state(env.num_envs, obs.device))
+    first = env.reset()
+    obs = first["obs"]
+    out = dict(next_obs=obs, pomdp_obs=obs.clone(), next_done=torch.zeros(env.num_envs, device=obs.device),
+               lstm_state=actor.initial_state(env.num_envs, obs.device))
+    if "states" in first:            # a copy: the env's states buffer is overwritten by every step
+        out["next_states"] = first["states"].clone()
+    return out
 
 
 class GraphedRollout:
@@ -145,6 +159,8 @@ class GraphedRollout:
         s["next_done"].copy_(new["next_done"])
         s["lstm_state"][0].copy_(new["lstm_state"][0])
         s["lstm_state"][1].copy_(new["lstm_state"][1])
+        if "next_states" in s:
+            s["next_states"].copy_(new["next_states"])
 
     def run(self):
         self.graph.replay()

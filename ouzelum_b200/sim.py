@@ -69,6 +69,14 @@ class QuadSim:
         check(lib.ozl_step_wrench(self._h, wrench.data_ptr(), ptr(target), obs.data_ptr(), rew.data_ptr(),
                                   reset.data_ptr(), progress.data_ptr(), ptr(timeout), ptr(ep_ret), _stream()))
 
+    def set_states_output(self, states):
+        """ozl_set_states_output: every later step launch also writes the privileged critic state into `states`
+        ([N, STATES_WIDTH] f32 CUDA tensor, kept alive by the caller); None unregisters."""
+        if states is not None and (tuple(states.shape) != (self.num_envs, _lib.STATES_WIDTH) or states.dtype != torch.float32
+                                   or not states.is_contiguous() or states.device != self.device):
+            raise ValueError(f"states must be a contiguous float32 [{self.num_envs}, {_lib.STATES_WIDTH}] tensor on {self.device}")
+        check(lib.ozl_set_states_output(self._h, ptr(states), _lib.STATES_WIDTH))
+
     def rollout(self, k, obs, rew, reset, progress):
         check(lib.ozl_rollout(self._h, int(k), obs.data_ptr(), rew.data_ptr(), reset.data_ptr(), progress.data_ptr(),
                               _stream()))

@@ -30,6 +30,7 @@ from .ouzelum import _POMDP, x500_cfg_from_task
 class EKFLeeLanded(_VehicleTargetTask):
     x_offset = -0.08                                   # ekf_lee_landed.py:629
     land_cutoff = 0.25                                 # ekf_lee_landed.py:508
+    supports_states = False                            # the fused estimator step kernel has no states output
 
     def __init__(self, cfg, *a, **k):
         env = cfg["env"]

@@ -100,11 +100,27 @@ def x500_cfg_from_task(cfg, num_envs, **over):
     return _lib.default_cfg(num_envs, **kw)
 
 
+def asymmetric_states(task_name, env_cfg, supported):
+    """`env.asymmetric_observations` (the stock IsaacGymEnvs name of the numStates critic input): True -> set numStates to the
+    kernel's privileged-state width before VecTask reads it.  Raises ValueError for a task whose step kernel has no states output
+    or for an explicit numStates of another width."""
+    if not bool(env_cfg.get("asymmetric_observations", False)):
+        return False
+    if not supported:
+        raise ValueError(f"{task_name}: asymmetric_observations is not supported (its step kernel does not write a states output)")
+    ns = env_cfg.get("numStates")
+    if ns is not None and int(ns) != _lib.STATES_WIDTH:
+        raise ValueError(f"{task_name}: asymmetric_observations writes {_lib.STATES_WIDTH} states per env, but numStates = {ns}")
+    env_cfg["numStates"] = _lib.STATES_WIDTH
+    return True
+
+
 class X500Task(VecTask):
     """Shared machinery of the x500 tasks: owns the `QuadSim` handle and launches the fused step."""
 
     num_x500_obs = 13
     num_x500_actions = 4
+    supports_states = True             # the step kernels can write the privileged critic state (ozl_set_states_output)
 
     def __init__(self, cfg, rl_device, sim_device, graphics_device_id, headless,
                  virtual_screen_capture=False, force_render=False):
@@ -113,9 +129,13 @@ class X500Task(VecTask):
         self.debug_viz = self.cfg["env"].get("enableDebugVis", False)
         self.cfg["env"]["numObservations"] = self.num_x500_obs     # ouzelum.py:50
         self.cfg["env"]["numActions"] = self.num_x500_actions      # ouzelum.py:55
+        asym = asymmetric_states(type(self).__name__, self.cfg["env"], self.supports_states)
         super().__init__(config=self.cfg, rl_device=rl_device, sim_device=sim_device,
                          graphics_device_id=graphics_device_id, headless=headless,
                          virtual_screen_capture=virtual_screen_capture, force_render=force_render)
+        if asym:                       # registered once: the buffer never moves, so captured graphs keep writing it
+            self.sim.set_states_output(self.states_buf)
+            self._states_from_kernel = True
         self.dt = float(self.cfg.get("sim", {}).get("dt", 0.01))
         self._timeout_u8 = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
         self.timeout_buf = self._timeout_u8.view(torch.bool)
@@ -259,7 +279,8 @@ class X500Task(VecTask):
                 "params": params.cpu(), "fault": fault.cpu(), "step_count": self.sim.step_count,
                 "reset_buf": self.reset_buf.cpu(), "progress_buf": self.progress_buf.cpu(), "obs_buf": self.obs_buf.cpu(),
                 "rew_buf": self.rew_buf.cpu(), "timeout_buf": self._timeout_u8.cpu(), "episode_return_buf": self.episode_return_buf.cpu(),
-                "seed": int(self.native_cfg.seed), "num_envs": self.num_envs, "task": type(self).__name__}
+                "seed": int(self.native_cfg.seed), "num_envs": self.num_envs, "task": type(self).__name__,
+                **({"states_buf": self.states_buf.cpu()} if self.num_states > 0 else {})}
 
     def load_state_dict(self, sd):
         if sd["num_envs"] != self.num_envs:
@@ -276,6 +297,8 @@ class X500Task(VecTask):
         if "timeout_buf" in sd:
             self._timeout_u8.copy_(sd["timeout_buf"])
             self.episode_return_buf.copy_(sd["episode_return_buf"])
+        if self.num_states > 0 and "states_buf" in sd:
+            self.states_buf.copy_(sd["states_buf"])
         if sd.get("task", type(self).__name__) != type(self).__name__:
             raise ValueError(f"checkpoint of task {sd['task']!r} loaded into {type(self).__name__!r}")
         self._graph = None

@@ -73,6 +73,7 @@ class VecTask(Env):
     metadata = {"render.modes": ["human", "rgb_array"], "video.frames_per_second": 24}
     reward_range = (-float("inf"), float("inf"))
     spec = None
+    _states_from_kernel = False        # True once the task's step kernel writes states_buf (env.asymmetric_observations)
 
     def __init__(self, config, rl_device, sim_device, graphics_device_id, headless,
                  virtual_screen_capture: bool = False, force_render: bool = False):
@@ -119,6 +120,8 @@ class VecTask(Env):
 
     # ---- surface ------------------------------------------------------------------------------------
     def get_state(self):
+        if self._states_from_kernel:       # clamped in the kernel: no torch op on the step path
+            return self.states_buf if self._rl_on_sim_device else self.states_buf.to(self.rl_device)
         return torch.clamp(self.states_buf, -self.clip_obs, self.clip_obs).to(self.rl_device)
 
     def step(self, actions: torch.Tensor) -> Tuple[Dict[str, torch.Tensor], torch.Tensor, torch.Tensor, Dict[str, Any]]:
