@@ -26,10 +26,11 @@
 extern "C" {
 #endif
 
-#define OZL_ABI_VERSION 5   /* 3: ozl_cfg.dr[] (domain-randomisation schema), per-env yaw_km (params8), wrench_warmup_steps,
+#define OZL_ABI_VERSION 6   /* 3: ozl_cfg.dr[] (domain-randomisation schema), per-env yaw_km (params8), wrench_warmup_steps,
                                ozl_ekf_lee_args.num_envs_total, i64 reset mirror in ozl_host_io
                                4: (additive) ozl_metrics_xchg_* / ozl_metrics_push / ozl_metrics_sum, ozl_noise_lambda_apply
-                               5: (additive) ozl_set_states_output, OZL_STATE_* layout of the privileged critic state */
+                               5: (additive) ozl_set_states_output, OZL_STATE_* layout of the privileged critic state
+                               6: (additive) ozl_set_scenarios, OZL_SCN_* layout of a scenario row */
 
 /* sensor-fault model of isaacgymenvs/utils/POMDP.py:4-42 */
 enum { OZL_POMDP_NONE = 0, OZL_POMDP_FLICKER = 1, OZL_POMDP_NOISE = 2, OZL_POMDP_FLICKER_NOISE = 3 };
@@ -211,6 +212,44 @@ enum { OZL_STATE_OBS = 0, OZL_STATE_THRUST = 13, OZL_STATE_EFF = 17, OZL_STATE_M
  * While a buffer is registered, ozl_rollout and ozl_ekf_lee_landed_step refuse to run (non-zero return, ozl_last_error()):
  * their kernels do not write the state. */
 int ozl_set_states_output(ozl_env* env, float* states, int32_t width);
+
+/* Scenario table: per-env episode conditions that every reset of the env applies in place of the random draws, so that the
+ * conditions of an episode no longer depend on the step at which the previous one ended (i.e. on the policy).  One float32 row
+ * of OZL_SCENARIO_WIDTH per local env, row-major [N, OZL_SCENARIO_WIDTH]:
+ *   OZL_SCN_POS .. +2          root position (absolute)                                      group "position"
+ *   OZL_SCN_QUAT .. +3         attitude quaternion xyzw, unit                                group "attitude"
+ *   OZL_SCN_LINVEL .. +2       linear velocity (world)                                       group "linear velocity"
+ *   OZL_SCN_ANGVEL .. +2       angular velocity (world)                                      group "angular velocity"
+ *   OZL_SCN_TARGET .. +2       target                                                        group "target"
+ *   OZL_SCN_FAULT_ROTOR, _ONSET, _EFF   faulted rotor (0..3, or -1: no fault this episode), onset (progress step, an integer
+ *                              in [0, 2^24)), effectiveness in [0, 1]                        group "fault"
+ *   OZL_SCN_MASS .. _YAW_KM    mass, ixx, iyy, izz, arm, thrust_scale, yaw_km (absolute values, as params8 of ozl_set_params),
+ *                              one group each
+ *   OZL_SCN_RESERVED .. 31     must be NaN
+ * Slots 0-12 are laid out as root13 of ozl_set_state.  A group is either all NaN -- the env gets exactly what it gets without a
+ * table: the draw, identity / zero for attitude and velocities, an unchanged value for a body parameter that is not randomised --
+ * or all set, and then its values are used at every reset of the env.  An all-NaN table therefore gives results bit-identical to
+ * no table.  A set target also holds through the periodic re-samples of the episode (target_period).  Not pinned by a table:
+ * the per-step sensor-fault draws (flicker / noise), the observation and action noise lambdas, and the ground vehicle's
+ * trajectory draws of the landing family.
+ * The rows apply at the resets of ozl_step, ozl_step_tracking, ozl_step_wrench, ozl_step_host*, ozl_landing_step,
+ * ozl_lee_landed_step and ozl_apply_resets; the landed flag and the episode bookkeeping are unchanged. */
+enum { OZL_SCN_POS = 0, OZL_SCN_QUAT = 3, OZL_SCN_LINVEL = 7, OZL_SCN_ANGVEL = 10, OZL_SCN_TARGET = 13, OZL_SCN_FAULT_ROTOR = 16,
+       OZL_SCN_FAULT_ONSET = 17, OZL_SCN_FAULT_EFF = 18, OZL_SCN_MASS = 19, OZL_SCN_IXX = 20, OZL_SCN_IYY = 21, OZL_SCN_IZZ = 22,
+       OZL_SCN_ARM = 23, OZL_SCN_THRUST_SCALE = 24, OZL_SCN_YAW_KM = 25, OZL_SCN_RESERVED = 26, OZL_SCENARIO_WIDTH = 32 };
+
+/* Register the scenario table: `rows_host` is HOST memory, [N, OZL_SCENARIO_WIDTH] f32; `width` must be OZL_SCENARIO_WIDTH.
+ * Every row is validated first and nothing is registered if one fails: reserved slots NaN; each group all NaN or all finite;
+ * |x^2 + y^2 + z^2 + w^2 - 1| <= 1e-6 for the quaternion (the integrator keeps a unit quaternion unit with one Newton step and
+ * needs a unit input); no target group when cfg.target_fixed is set (the target is driven by a vehicle or the caller); no fault
+ * group unless cfg.fault_mode is set; rotor in {-1, 0, 1, 2, 3}, onset an integer in [0, 2^24), effectiveness in [0, 1]; mass
+ * and inertias in (1e-30, 1e30) (the step's reciprocals need positive normal floats), arm > 0, thrust_scale >= 0, yaw_km finite.
+ * The rows are copied (stream-ordered on `stream`, which is then synchronised) into a device buffer the handle allocates on the
+ * first registration and frees in ozl_destroy.  A later call overwrites the contents at the same address, so a CUDA graph
+ * captured while a table is registered applies the new rows at its next resets.  rows_host = NULL unregisters.  Registering or
+ * unregistering after a capture is not seen by that graph (it keeps the kernels it captured), as for ozl_set_states_output.
+ * While a table is registered, ozl_rollout and ozl_ekf_lee_landed_step refuse to run (non-zero return, ozl_last_error()). */
+int ozl_set_scenarios(ozl_env* env, const float* rows_host, int32_t width, void* stream);
 
 /* Mode-B throughput entry: K steps in ONE launch, state held in registers, actions a = 2u-1 drawn
  * in-kernel from the counter RNG; obs/rew are written for the LAST step only, reset/progress are

@@ -9,7 +9,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("OUZELUM_B200_LIB") or os.path.join(_HERE, "libouzelum_b200.so")   # override: kernel experiments only
 
-OZL_ABI_VERSION = 5
+OZL_ABI_VERSION = 6
 
 
 def _header_enum(prefix):
@@ -23,6 +23,9 @@ def _header_enum(prefix):
 # privileged critic state written by the step kernels (ozl_set_states_output): slot indices OZL_STATE_* and the row width
 STATES_LAYOUT = _header_enum("OZL_STATE")
 STATES_WIDTH = STATES_LAYOUT["OZL_STATES_WIDTH"]
+# scenario rows applied at every reset (ozl_set_scenarios): slot indices OZL_SCN_* and the row width OZL_SCENARIO_WIDTH
+SCENARIO_LAYOUT = _header_enum("OZL_SC")
+SCENARIO_WIDTH = SCENARIO_LAYOUT["OZL_SCENARIO_WIDTH"]
 
 
 DR_NONE, DR_UNIFORM, DR_LOGUNIFORM, DR_GAUSSIAN = 0, 1, 2, 3
@@ -178,6 +181,7 @@ _SIGS = {
     "ozl_step_wrench": (C.c_int, [_P] * 10),
     "ozl_rollout": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P]),
     "ozl_set_states_output": (C.c_int, [_P, _P, C.c_int32]),
+    "ozl_set_scenarios": (C.c_int, [_P, _P, C.c_int32, _P]),
     "ozl_get_state": (C.c_int, [_P] * 6),
     "ozl_set_state": (C.c_int, [_P] * 6),
     "ozl_get_params": (C.c_int, [_P] * 4),

@@ -507,6 +507,8 @@ extern "C" int ozl_ekf_lee_landed_step(ozl_env* env, const ozl_ekf_lee_args* in,
     if (!husky) return set_error("ozl_ekf_lee_landed_step: husky args are NULL");
     if (env && env->states)
         return set_error("ozl_ekf_lee_landed_step: a states output is registered (ozl_set_states_output) and the fused estimator step does not write it");
+    if (env && env->scn)
+        return set_error("ozl_ekf_lee_landed_step: a scenario table is registered (ozl_set_scenarios) and the fused estimator step does not apply it");
     return launch_ekf_lee(env, in, husky, StepIo{obs, rew, reset, progress, timeout, ep_ret}, stream);
 }
 

@@ -85,6 +85,11 @@ struct ozl_env {
     // map over it (box [128 rows][32], 128-byte swizzle) through which the step kernels store one states tile per 128 envs
     float* states;
     alignas(64) unsigned char states_tmap[128];
+    // scenario table (ozl_set_scenarios): device copy of the caller's [N, OZL_SCENARIO_WIDTH] rows, allocated on the first
+    // registration and kept until ozl_destroy (re-registration overwrites it in place); `scn` is that buffer while a table is
+    // registered and NULL otherwise -- the step launches pick the kernels that read it by this pointer
+    float* scn_buf;
+    float* scn;
 };
 
 // Step launches go through cudaLaunchKernelEx so that they can carry the programmatic-stream-serialization attribute (PDL):

@@ -66,15 +66,17 @@ __device__ __forceinline__ void stage_states_row(float* tile, int r, const float
 }
 
 // STATES: also write the privileged critic state (ozl_set_states_output) through `states_map`; the STATES = false instantiations
-// are the kernels without that output.
-template <int BLOCK, int FRONT, bool STATES>
-__global__ void __launch_bounds__(BLOCK, OZL_STEP_MINB)
-quad_step_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ actions, float* __restrict__ obs,
-                 float* __restrict__ rew, int64_t* __restrict__ reset, int64_t* __restrict__ progress,
-                 uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, const float* __restrict__ target_in,
-                 const int act_mode, uint8_t* __restrict__ done_u8, int64_t* __restrict__ reset_mirror, const int obs_bulk,
-                 const int64_t env0, const FrontArgs fa, volatile unsigned int* host_done, const unsigned int host_seq,
-                 const __grid_constant__ CUtensorMap states_map) {
+// are the kernels without that output.  SCN: lay the scenario table `scn` (ozl_set_scenarios) over the reset draws; the body
+// is instantiated by two kernels, quad_step_kernel (no table, `scn` unused) and quad_step_scn_kernel.
+#define OZL_STEP_PARAMS                                                                                                         \
+    const DevCfg c, const Planes pl, const float4* __restrict__ actions, float* __restrict__ obs, float* __restrict__ rew,       \
+        int64_t* __restrict__ reset, int64_t* __restrict__ progress, uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, \
+        const float* __restrict__ target_in, const int act_mode, uint8_t* __restrict__ done_u8, int64_t* __restrict__ reset_mirror, \
+        const int obs_bulk, const int64_t env0, const FrontArgs fa, volatile unsigned int* host_done, const unsigned int host_seq
+#define OZL_STEP_ARGS c, pl, actions, obs, rew, reset, progress, timeout, ep_ret_out, target_in, act_mode, done_u8, reset_mirror, \
+                      obs_bulk, env0, fa, host_done, host_seq, states_map, scn
+template <int BLOCK, int FRONT, bool STATES, bool SCN>
+__device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMap& states_map, const float* __restrict__ scn) {
     __shared__ __align__(16) float s_obs[BLOCK * 13];
     __shared__ __align__(1024) float s_states[STATES ? BLOCK * OZL_STATES_WIDTH : 4];
     __shared__ uint64_t s_step;
@@ -117,8 +119,9 @@ quad_step_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ act
         }
         float act[4] = {a4.x, a4.y, a4.z, a4.w};
         const uint32_t genv = c.env_id_base + (uint32_t)i;
+        const float* scn_row = SCN ? scn + i * OZL_SCENARIO_WIDTH : nullptr;
         if (FRONT == FRONT_LEE) {
-            const int64_t prog1 = env_reset_phase(e, prog, rst, genv, step, c, o);
+            const int64_t prog1 = env_reset_phase<SCN>(e, prog, rst, genv, step, c, o, scn_row);
             const float cmd[4] = {fa.cmd[0] * fa.g.scale[0], fa.cmd[1] * fa.g.scale[1], fa.cmd[2] * fa.g.scale[2], fa.cmd[3] * fa.g.scale[3]};
             float th, tq[3];
             lee_control(LEE_POSITION, e.p, e.q, e.v, e.w, cmd, fa.g, th, tq);                  // lee_landed.py:311
@@ -126,7 +129,7 @@ quad_step_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ act
             if (fa.wrench_out) fa.wrench_out[i] = make_float4(act[0], act[1], act[2], act[3]);
             env_act_phase(e, act, prog1, rst, genv, step, c, o, ACT_WRENCH, tptr, fa.cmd);       // detector on the controller target, :305,318-322
         } else {
-            env_step(e, act, prog, rst, genv, step, c, o, act_mode, tptr);
+            env_step<SCN>(e, act, prog, rst, genv, step, c, o, act_mode, tptr, scn_row);
         }
         if constexpr (STATES) stage_states_row(s_states, threadIdx.x, o.obs, e, o, c);
         obs_epilogue(o.obs, genv, step, flicker_blackout(step, c), c);
@@ -208,6 +211,17 @@ quad_step_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ act
     }
 }
 
+template <int BLOCK, int FRONT, bool STATES>
+__global__ void __launch_bounds__(BLOCK, OZL_STEP_MINB)
+quad_step_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
+    quad_step_body<BLOCK, FRONT, STATES, false>(OZL_STEP_ARGS);
+}
+template <int BLOCK, int FRONT, bool STATES>
+__global__ void __launch_bounds__(BLOCK, OZL_STEP_MINB)
+quad_step_scn_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
+    quad_step_body<BLOCK, FRONT, STATES, true>(OZL_STEP_ARGS);
+}
+
 // ------------------------------------------------------------------------------------------------ K1, TMA-pipelined
 // Persistent variant for large N (rotor-action mode, stored target): one CTA per (SM x 8) slot loops over tiles of
 // kTile = 128 envs.  Thanks to the tiled state layout a tile's whole state is ONE contiguous 15 KiB region, so thread 0
@@ -226,12 +240,13 @@ constexpr int kTmaStageBytes = kTmaRstOff + kTile * 8;            // 19456
 #ifndef OZL_TMA_MINB
 #define OZL_TMA_MINB 5
 #endif
-template <bool STATES>
-__global__ void __launch_bounds__(kTile, OZL_TMA_MINB)
-quad_step_tma_kernel(const DevCfg c, const Planes pl, const float4* __restrict__ actions, float* __restrict__ obs,
-                     float* __restrict__ rew, int64_t* __restrict__ reset, int64_t* __restrict__ progress,
-                     uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, const int64_t full_tiles,
-                     const __grid_constant__ CUtensorMap states_map) {
+#define OZL_TMA_PARAMS                                                                                                          \
+    const DevCfg c, const Planes pl, const float4* __restrict__ actions, float* __restrict__ obs, float* __restrict__ rew,       \
+        int64_t* __restrict__ reset, int64_t* __restrict__ progress, uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, \
+        const int64_t full_tiles
+#define OZL_TMA_ARGS c, pl, actions, obs, rew, reset, progress, timeout, ep_ret_out, full_tiles, states_map, scn
+template <bool STATES, bool SCN>
+__device__ __forceinline__ void quad_step_tma_body(OZL_TMA_PARAMS, const CUtensorMap& states_map, const float* __restrict__ scn) {
     __shared__ __align__(128) unsigned char s_stage[kTmaStageBytes];
     __shared__ __align__(16) float s_obs[kTile * 13];
     __shared__ __align__(1024) float s_states[STATES ? kTile * OZL_STATES_WIDTH : 4];   // 16 KB: 5 CTAs/SM still fit
@@ -309,7 +324,7 @@ quad_step_tma_kernel(const DevCfg c, const Planes pl, const float4* __restrict__
         const float act[4] = {a4.x, a4.y, a4.z, a4.w};
         const uint32_t genv = c.env_id_base + (uint32_t)i;
         StepOut o;
-        env_step(e, act, prog, rst, genv, step, c, o, ACT_ROTORS, nullptr);
+        env_step<SCN>(e, act, prog, rst, genv, step, c, o, ACT_ROTORS, nullptr, SCN ? scn + i * OZL_SCENARIO_WIDTH : nullptr);
         if constexpr (STATES) stage_states_row(s_states, tid, o.obs, e, o, c);
         obs_epilogue(o.obs, genv, step, blackout, c);
         store_dynamic(pl, i, e);
@@ -366,6 +381,17 @@ quad_step_tma_kernel(const DevCfg c, const Planes pl, const float4* __restrict__
         // launch of quad_step_kernel that follows on the stream
         retire_units(pl.ctrl, (unsigned long long)m_valid + (blockIdx.x == 0 ? (unsigned long long)c.step_pad : 0ull));
     }
+}
+
+template <bool STATES>
+__global__ void __launch_bounds__(kTile, OZL_TMA_MINB)
+quad_step_tma_kernel(OZL_TMA_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
+    quad_step_tma_body<STATES, false>(OZL_TMA_ARGS);
+}
+template <bool STATES>
+__global__ void __launch_bounds__(kTile, OZL_TMA_MINB)
+quad_step_tma_scn_kernel(OZL_TMA_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
+    quad_step_tma_body<STATES, true>(OZL_TMA_ARGS);
 }
 
 // ------------------------------------------------------------------------------------------------ mode B
@@ -525,8 +551,8 @@ __global__ void set_params_kernel(const Planes pl, int64_t n, const float* param
     store_static(pl, i, e);
 }
 
-// reset phase only (see ozl_apply_resets): same draws as env_step, no physics, no bookkeeping
-__global__ void apply_resets_kernel(const DevCfg c, const Planes pl, const int64_t* __restrict__ reset) {
+// reset phase only (see ozl_apply_resets): same draws as env_step, no physics, no bookkeeping; `scn`: the scenario table or NULL
+__global__ void apply_resets_kernel(const DevCfg c, const Planes pl, const int64_t* __restrict__ reset, const float* __restrict__ scn) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= c.num_envs || reset[i] == 0) return;
     const uint64_t step = read_step(pl.ctrl);
@@ -541,6 +567,7 @@ __global__ void apply_resets_kernel(const DevCfg c, const Planes pl, const int64
         e.tgt[0] = u01(r.x) * c.target_scale[0] + c.target_off[0];
         e.tgt[1] = u01(r.y) * c.target_scale[1] + c.target_off[1];
         e.tgt[2] = u01(r.z) * c.target_scale[2] + c.target_off[2];
+        if (scn) scn_target(e, scn + i * OZL_SCENARIO_WIDTH);
     }
     const uint4 r = draw(c.seed, genv, step, P_SPAWN);
     e.p[0] = c.spawn_base[0] + (c.spawn_range[0] * u01(r.x) + c.spawn_lo[0]);
@@ -554,6 +581,7 @@ __global__ void apply_resets_kernel(const DevCfg c, const Planes pl, const int64
         e.eff = c.fault_eff_lo + c.fault_eff_range * u01(f.z);
     }
     if (c.dr_enable) dr_draw_all(e, genv, step, c);
+    if (scn) scn_respawn(e, scn + i * OZL_SCENARIO_WIDTH);
     store_dynamic(pl, i, e);
     store_static(pl, i, e);
 }
@@ -760,6 +788,7 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
     e->cfg = *cfg;
     e->states = nullptr;
     memset(e->states_tmap, 0, sizeof(e->states_tmap));
+    e->scn_buf = e->scn = nullptr;
     derive_dev_cfg(*cfg, e->dev);
     e->device = device;
     e->sm_count = prop.multiProcessorCount;
@@ -820,6 +849,7 @@ extern "C" int ozl_destroy(ozl_env* env) {
     if (!env) return 0;
     cudaSetDevice(env->device);
     cudaFree(env->arena);
+    if (env->scn_buf) cudaFree(env->scn_buf);
     if (env->host_done) cudaFreeHost((void*)env->host_done);
     delete env;
     return 0;
@@ -847,7 +877,7 @@ static_assert(kStepBlock == kTile, "the step counter retires one work unit per 1
 // The states tensor map of the handle (zeros while no states buffer is registered: the STATES = false kernels never read it)
 static inline const CUtensorMap& states_map(const ozl_env* env) { return *reinterpret_cast<const CUtensorMap*>(env->states_tmap); }
 
-template <bool STATES>
+template <bool STATES, bool SCN>
 static int launch_step_t(ozl_env* env, const float* actions, const float* target_in, int act_mode, float* obs, float* rew,
                          int64_t* reset, int64_t* progress, uint8_t* timeout, float* ep_ret, void* stream, const char* who,
                          uint8_t* done_u8, int obs_bulk, int64_t* reset_mirror, int host_flag) {
@@ -858,38 +888,40 @@ static int launch_step_t(ozl_env* env, const float* actions, const float* target
     const int64_t full_tiles = n / kTile, tail = n % kTile;
     const int64_t resident = (int64_t)env->sm_count * OZL_TMA_MINB;
     const bool plain = (target_in == nullptr) && act_mode == ACT_ROTORS && done_u8 == nullptr && reset_mirror == nullptr && obs_bulk;
+    const auto tma_kernel = SCN ? quad_step_tma_scn_kernel<STATES> : quad_step_tma_kernel<STATES>;
+    const auto kernel = SCN ? quad_step_scn_kernel<kStepBlock, FRONT_NONE, STATES> : quad_step_kernel<kStepBlock, FRONT_NONE, STATES>;
     if (plain && env->tma_min_tiles > 0 && full_tiles >= env->tma_min_tiles &&
         !(((uintptr_t)progress | (uintptr_t)reset) & 15)) {
         // large N: persistent TMA-pipelined kernel over the whole tiles, then one generic block for the ragged tail
         unsigned grid = (unsigned)(full_tiles < resident ? full_tiles : resident);
         while ((full_tiles + grid - 1) / grid > 8192) grid *= 2;     // 16-bit packed metric counters: keep tiles per CTA far below 65535
-        if (launch_pdl(env, quad_step_tma_kernel<STATES>, dim3(grid), dim3(kTile), st, env->dev, env->pl, (const float4*)actions, obs, rew,
-                       reset, progress, timeout, ep_ret, full_tiles, states_map(env)))
+        if (launch_pdl(env, tma_kernel, dim3(grid), dim3(kTile), st, env->dev, env->pl, (const float4*)actions, obs, rew,
+                       reset, progress, timeout, ep_ret, full_tiles, states_map(env), (const float*)env->scn))
             return check_cuda(cudaGetLastError(), "quad_step_tma_kernel");
         if (tail)
-            quad_step_kernel<kStepBlock, FRONT_NONE, STATES><<<1, kStepBlock, 0, st>>>(env->dev, env->pl, (const float4*)actions, obs, rew,
-                                                                                      reset, progress, timeout, ep_ret, nullptr, ACT_ROTORS,
-                                                                                      nullptr, nullptr, 1, full_tiles * kTile, FrontArgs{},
-                                                                                      (volatile unsigned int*)nullptr, 0u, states_map(env));
+            kernel<<<1, kStepBlock, 0, st>>>(env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, nullptr,
+                                             ACT_ROTORS, nullptr, nullptr, 1, full_tiles * kTile, FrontArgs{},
+                                             (volatile unsigned int*)nullptr, 0u, states_map(env), (const float*)env->scn);
         return check_cuda(cudaGetLastError(), "quad_step_kernel(tail)");
     }
-    if (launch_pdl(env, quad_step_kernel<kStepBlock, FRONT_NONE, STATES>, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev,
+    if (launch_pdl(env, kernel, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev,
                    env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, target_in, act_mode, done_u8, reset_mirror,
                    obs_bulk, (int64_t)0, FrontArgs{}, (volatile unsigned int*)(host_flag ? env->host_done : nullptr),
-                   host_flag ? ++env->host_seq : 0u, states_map(env)))
+                   host_flag ? ++env->host_seq : 0u, states_map(env), (const float*)env->scn))
         return check_cuda(cudaGetLastError(), "quad_step_kernel");
     return 0;
 }
 
-// The kernels with the states output run whenever the handle has a states buffer registered.
+// The kernels with the states output run whenever the handle has a states buffer registered, the scenario kernels whenever it
+// has a scenario table registered.
 static int launch_step(ozl_env* env, const float* actions, const float* target_in, int act_mode, float* obs, float* rew,
                        int64_t* reset, int64_t* progress, uint8_t* timeout, float* ep_ret, void* stream, const char* who,
                        uint8_t* done_u8 = nullptr, int obs_bulk = 1, int64_t* reset_mirror = nullptr, int host_flag = 0) {
     if (!env) return set_error("%s: env is NULL", who);
-    return env->states ? launch_step_t<true>(env, actions, target_in, act_mode, obs, rew, reset, progress, timeout, ep_ret, stream, who,
-                                             done_u8, obs_bulk, reset_mirror, host_flag)
-                       : launch_step_t<false>(env, actions, target_in, act_mode, obs, rew, reset, progress, timeout, ep_ret, stream, who,
-                                              done_u8, obs_bulk, reset_mirror, host_flag);
+    auto* f = env->states ? (env->scn ? launch_step_t<true, true> : launch_step_t<true, false>)
+                          : (env->scn ? launch_step_t<false, true> : launch_step_t<false, false>);
+    return f(env, actions, target_in, act_mode, obs, rew, reset, progress, timeout, ep_ret, stream, who, done_u8, obs_bulk, reset_mirror,
+             host_flag);
 }
 
 // Landing-family steps with the vehicle (and, for LeeLanded, the controller) in the same launch.
@@ -910,9 +942,10 @@ static int launch_front_step(ozl_env* env, int front, const float* actions, cons
     const int64_t n = env->cfg.num_envs;
     cudaStream_t st = (cudaStream_t)stream;
 #define OZL_LAUNCH_FRONT(F, S, MODE)                                                                                            \
-    launch_pdl(env, quad_step_kernel<kStepBlock, F, S>, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev, env->pl,     \
-               (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, (const float*)nullptr, (int)MODE, (uint8_t*)nullptr, \
-               (int64_t*)nullptr, 1, (int64_t)0, fa, (volatile unsigned int*)nullptr, 0u, states_map(env))
+    launch_pdl(env, env->scn ? quad_step_scn_kernel<kStepBlock, F, S> : quad_step_kernel<kStepBlock, F, S>, dim3(blocks_for(n, kStepBlock)), \
+               dim3(kStepBlock), st, env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret,          \
+               (const float*)nullptr, (int)MODE, (uint8_t*)nullptr, (int64_t*)nullptr, 1, (int64_t)0, fa,                           \
+               (volatile unsigned int*)nullptr, 0u, states_map(env), (const float*)env->scn)
     int rc;
     if (front == FRONT_VEHICLE)
         rc = env->states ? OZL_LAUNCH_FRONT(FRONT_VEHICLE, true, ACT_ROTORS) : OZL_LAUNCH_FRONT(FRONT_VEHICLE, false, ACT_ROTORS);
@@ -1008,7 +1041,7 @@ extern "C" int ozl_step_wrench(ozl_env* env, const float* wrench4, const float* 
 extern "C" int ozl_apply_resets(ozl_env* env, const int64_t* reset, void* stream) {
     OZL_ENV_CHECK("ozl_apply_resets");
     if (!reset) return set_error("ozl_apply_resets: reset is NULL");
-    apply_resets_kernel<<<blocks_for(env->cfg.num_envs, 256), 256, 0, st>>>(env->dev, env->pl, reset);
+    apply_resets_kernel<<<blocks_for(env->cfg.num_envs, 256), 256, 0, st>>>(env->dev, env->pl, reset, env->scn);
     return check_cuda(cudaGetLastError(), "apply_resets_kernel");
 }
 
@@ -1016,6 +1049,7 @@ extern "C" int ozl_rollout(ozl_env* env, int32_t K, float* obs, float* rew, int6
     OZL_ENV_CHECK("ozl_rollout");
     if (K <= 0) return set_error("ozl_rollout: K must be > 0");
     if (env->states) return set_error("ozl_rollout: a states output is registered (ozl_set_states_output) and the K-step kernel does not write it");
+    if (env->scn) return set_error("ozl_rollout: a scenario table is registered (ozl_set_scenarios) and the K-step kernel does not apply it");
     if (!obs || !rew || !reset || !progress) return set_error("ozl_rollout: NULL buffer");
     quad_rollout_kernel<kStepBlock><<<blocks_for(env->cfg.num_envs, kStepBlock), kStepBlock, 0, st>>>(
         env->dev, env->pl, K, obs, rew, reset, progress);
@@ -1059,6 +1093,74 @@ extern "C" int ozl_set_states_output(ozl_env* env, float* states, int32_t width)
     if (r != CUDA_SUCCESS) return set_error("ozl_set_states_output: cuTensorMapEncodeTiled failed (%d)", (int)r);
     memcpy(env->states_tmap, m, sizeof(m));
     env->states = states;
+    return 0;
+}
+
+// One scenario row against the rules of ozl_set_scenarios (include/ouzelum_b200.h); 0 = valid.
+static int check_scenario_row(const ozl_cfg& cfg, const float* r, int64_t row) {
+    static const struct { int first, count; const char* name; } groups[] = {
+        {OZL_SCN_POS, 3, "position"}, {OZL_SCN_QUAT, 4, "attitude"}, {OZL_SCN_LINVEL, 3, "linear velocity"},
+        {OZL_SCN_ANGVEL, 3, "angular velocity"}, {OZL_SCN_TARGET, 3, "target"}, {OZL_SCN_FAULT_ROTOR, 3, "fault"},
+        {OZL_SCN_MASS, 1, "mass"}, {OZL_SCN_IXX, 1, "ixx"}, {OZL_SCN_IYY, 1, "iyy"}, {OZL_SCN_IZZ, 1, "izz"}, {OZL_SCN_ARM, 1, "arm"},
+        {OZL_SCN_THRUST_SCALE, 1, "thrust_scale"}, {OZL_SCN_YAW_KM, 1, "yaw_km"}};
+    const char* who = "ozl_set_scenarios";
+    const long long k = (long long)row;
+    for (int j = OZL_SCN_RESERVED; j < OZL_SCENARIO_WIDTH; ++j)
+        if (!std::isnan(r[j])) return set_error("%s: row %lld: reserved slot %d must be NaN", who, k, j);
+    for (const auto& g : groups) {
+        int nan = 0;
+        for (int j = g.first; j < g.first + g.count; ++j) {
+            if (std::isnan(r[j])) ++nan;
+            else if (!std::isfinite(r[j])) return set_error("%s: row %lld: %s group has a non-finite value in slot %d", who, k, g.name, j);
+        }
+        if (nan != 0 && nan != g.count) return set_error("%s: row %lld: %s group must be all NaN or all set", who, k, g.name);
+    }
+    const auto set = [&](int slot) { return !std::isnan(r[slot]); };
+    if (set(OZL_SCN_QUAT)) {
+        const double x = r[OZL_SCN_QUAT], y = r[OZL_SCN_QUAT + 1], z = r[OZL_SCN_QUAT + 2], w = r[OZL_SCN_QUAT + 3];
+        if (!(std::fabs(x * x + y * y + z * z + w * w - 1.0) <= 1e-6))
+            return set_error("%s: row %lld: attitude quaternion is not unit (|q|^2 - 1 must be within 1e-6)", who, k);
+    }
+    if (set(OZL_SCN_TARGET) && cfg.target_fixed)
+        return set_error("%s: row %lld: target group set, but cfg.target_fixed is set (the target is driven by a vehicle or the caller)", who, k);
+    if (set(OZL_SCN_FAULT_ROTOR)) {
+        if (!cfg.fault_mode)
+            return set_error("%s: row %lld: fault group set, but the handle has no rotor-fault model (cfg.fault_mode, rotorFault.enable)", who, k);
+        const float rotor = r[OZL_SCN_FAULT_ROTOR], onset = r[OZL_SCN_FAULT_ONSET], eff = r[OZL_SCN_FAULT_EFF];
+        if (!(rotor == -1.0f || rotor == 0.0f || rotor == 1.0f || rotor == 2.0f || rotor == 3.0f))
+            return set_error("%s: row %lld: fault rotor %g is not one of -1, 0, 1, 2, 3", who, k, (double)rotor);
+        if (!(onset >= 0.0f && onset < 16777216.0f && onset == std::floor(onset)))
+            return set_error("%s: row %lld: fault onset %g is not an integer in [0, 2^24)", who, k, (double)onset);
+        if (!(eff >= 0.0f && eff <= 1.0f)) return set_error("%s: row %lld: fault effectiveness %g is not in [0, 1]", who, k, (double)eff);
+    }
+    for (int j = OZL_SCN_MASS; j <= OZL_SCN_IZZ; ++j)
+        if (set(j) && !(r[j] > 1e-30f && r[j] < 1e30f))
+            return set_error("%s: row %lld: slot %d (mass / inertia) must be a positive normal float in (1e-30, 1e30)", who, k, j);
+    if (set(OZL_SCN_ARM) && !(r[OZL_SCN_ARM] > 0.0f)) return set_error("%s: row %lld: arm must be > 0", who, k);
+    if (set(OZL_SCN_THRUST_SCALE) && !(r[OZL_SCN_THRUST_SCALE] >= 0.0f)) return set_error("%s: row %lld: thrust_scale must be >= 0", who, k);
+    return 0;
+}
+
+extern "C" int ozl_set_scenarios(ozl_env* env, const float* rows_host, int32_t width, void* stream) {
+    OZL_ENV_CHECK("ozl_set_scenarios");
+    if (width != OZL_SCENARIO_WIDTH)
+        return set_error("ozl_set_scenarios: width %d != OZL_SCENARIO_WIDTH (%d)", (int)width, (int)OZL_SCENARIO_WIDTH);
+    if (!rows_host) {
+        env->scn = nullptr;
+        return 0;
+    }
+    const int64_t n = env->cfg.num_envs;
+    for (int64_t i = 0; i < n; ++i)
+        if (check_scenario_row(env->cfg, rows_host + i * OZL_SCENARIO_WIDTH, i)) return 1;
+    const size_t bytes = (size_t)n * OZL_SCENARIO_WIDTH * sizeof(float);
+    if (!env->scn_buf && check_cuda(cudaMalloc(&env->scn_buf, bytes), "cudaMalloc(scenario table)")) {
+        env->scn_buf = nullptr;
+        return 1;
+    }
+    // stream-ordered behind any launch that still reads the old rows; synchronised so that the caller may free rows_host
+    if (check_cuda(cudaMemcpyAsync(env->scn_buf, rows_host, bytes, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(scenario table)")) return 1;
+    if (check_cuda(cudaStreamSynchronize(st), "cudaStreamSynchronize")) return 1;
+    env->scn = env->scn_buf;
     return 0;
 }
 

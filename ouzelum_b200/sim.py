@@ -77,6 +77,17 @@ class QuadSim:
             raise ValueError(f"states must be a contiguous float32 [{self.num_envs}, {_lib.STATES_WIDTH}] tensor on {self.device}")
         check(lib.ozl_set_states_output(self._h, ptr(states), _lib.STATES_WIDTH))
 
+    def set_scenarios(self, rows):
+        """ozl_set_scenarios: from now on every reset of env i applies row i of `rows` ([N, SCENARIO_WIDTH] float32, CPU or CUDA;
+        NaN groups keep the random draws) in place of the draws.  The rows are validated and copied; None unregisters."""
+        if rows is None:
+            check(lib.ozl_set_scenarios(self._h, None, _lib.SCENARIO_WIDTH, _stream()), ValueError)
+            return
+        if not isinstance(rows, torch.Tensor) or rows.dtype != torch.float32 or tuple(rows.shape) != (self.num_envs, _lib.SCENARIO_WIDTH):
+            raise ValueError(f"scenario rows must be a float32 [{self.num_envs}, {_lib.SCENARIO_WIDTH}] tensor")
+        host = rows.detach().to("cpu").contiguous()
+        check(lib.ozl_set_scenarios(self._h, host.data_ptr(), _lib.SCENARIO_WIDTH, _stream()), ValueError)
+
     def rollout(self, k, obs, rew, reset, progress):
         check(lib.ozl_rollout(self._h, int(k), obs.data_ptr(), rew.data_ptr(), reset.data_ptr(), progress.data_ptr(),
                               _stream()))

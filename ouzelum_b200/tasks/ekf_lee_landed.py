@@ -31,6 +31,7 @@ class EKFLeeLanded(_VehicleTargetTask):
     x_offset = -0.08                                   # ekf_lee_landed.py:629
     land_cutoff = 0.25                                 # ekf_lee_landed.py:508
     supports_states = False                            # the fused estimator step kernel has no states output
+    supports_scenarios = False                         # ... and does not apply a scenario table
 
     def __init__(self, cfg, *a, **k):
         env = cfg["env"]

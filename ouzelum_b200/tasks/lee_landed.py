@@ -28,6 +28,12 @@ class LeeLanded(_VehicleTargetTask):
                                   plate_z=TARGET_Z, plate_radius=0.35,
                                   land_cutoff=self.land_cutoff if bool(self.cfg["env"].get("fusedStep", True)) else 0.0)
 
+    def _check_scenarios(self, rows):
+        from .._lib import SCENARIO_LAYOUT
+        if not torch.isnan(rows[:, SCENARIO_LAYOUT["OZL_SCN_FAULT_ROTOR"]]).all():
+            raise ValueError("LeeLanded: scenario rows must leave the fault group NaN (the steps are wrench-actuated: rotor faults "
+                             "do not apply)")
+
     def create_sim(self):
         super().create_sim()
         self.controller = Controller(control(), self.device)

@@ -121,6 +121,7 @@ class X500Task(VecTask):
     num_x500_obs = 13
     num_x500_actions = 4
     supports_states = True             # the step kernels can write the privileged critic state (ozl_set_states_output)
+    supports_scenarios = True          # the step kernels can apply a scenario table at resets (ozl_set_scenarios)
 
     def __init__(self, cfg, rl_device, sim_device, graphics_device_id, headless,
                  virtual_screen_capture=False, force_render=False):
@@ -144,6 +145,7 @@ class X500Task(VecTask):
         self._host_io, self._host_keep = {}, []          # step_host: argument blocks cached by actions-buffer address
         self._graph = None
         self._static_actions = None
+        self.scenarios = None          # the registered scenario table (CPU copy), see set_scenarios
         self.use_cuda_graph = bool(self.cfg["env"].get("useCudaGraph", False))
 
     # ---- overridable pieces --------------------------------------------------------------------------
@@ -264,6 +266,30 @@ class X500Task(VecTask):
     def set_root_states(self, root):
         self.sim.set_state(root=root)
 
+    # ---- scenario table ----------------------------------------------------------------------------------------------------
+    def set_scenarios(self, rows):
+        """Pin per-env episode conditions: from now on every reset of env i applies row i of `rows` (float32 [num_envs,
+        SCENARIO_WIDTH] on CPU or CUDA, layout `_lib.SCENARIO_LAYOUT` / OZL_SCN_* in include/ouzelum_b200.h) in place of the random
+        draws -- spawn pose, velocities, target, rotor-fault schedule, body parameters.  An all-NaN group keeps the draw
+        (`ouzelum_b200.scenarios.empty`).  Not pinned: the per-step sensor-fault draws, the observation / action noise and the
+        ground vehicle's trajectory.  New contents reach a captured CUDA graph at its next resets; registering or unregistering
+        (rows = None) re-captures this task's own step graph.  Raises ValueError for an invalid table."""
+        if not self.supports_scenarios:
+            raise ValueError(f"{type(self).__name__}: scenario tables are not supported (its step kernel does not apply them)")
+        host = None
+        if rows is not None:
+            if not isinstance(rows, torch.Tensor):
+                raise ValueError("scenario rows must be a torch.Tensor")
+            host = rows.detach().to("cpu").contiguous()
+            self._check_scenarios(host)
+        self.sim.set_scenarios(host)
+        if (host is None) != (self.scenarios is None):
+            self._graph = None         # the captured step holds the kernels without (or with) the table
+        self.scenarios = None if host is None else host.clone()
+
+    def _check_scenarios(self, rows):
+        """Task-specific refusals of a scenario table (the library validates the rows themselves)."""
+
     def reset_idx(self, env_ids):
         """ouzelum.py:192-216.  The re-initialisation itself happens inside the next step's kernel (exactly when
         the reference's takes effect: pre_physics_step, ouzelum.py:226-229); here the request is recorded."""
@@ -280,6 +306,7 @@ class X500Task(VecTask):
                 "reset_buf": self.reset_buf.cpu(), "progress_buf": self.progress_buf.cpu(), "obs_buf": self.obs_buf.cpu(),
                 "rew_buf": self.rew_buf.cpu(), "timeout_buf": self._timeout_u8.cpu(), "episode_return_buf": self.episode_return_buf.cpu(),
                 "seed": int(self.native_cfg.seed), "num_envs": self.num_envs, "task": type(self).__name__,
+                "scenarios": None if self.scenarios is None else self.scenarios.clone(),
                 **({"states_buf": self.states_buf.cpu()} if self.num_states > 0 else {})}
 
     def load_state_dict(self, sd):
@@ -299,6 +326,8 @@ class X500Task(VecTask):
             self.episode_return_buf.copy_(sd["episode_return_buf"])
         if self.num_states > 0 and "states_buf" in sd:
             self.states_buf.copy_(sd["states_buf"])
+        if "scenarios" in sd and (sd["scenarios"] is not None or self.scenarios is not None):
+            self.set_scenarios(sd["scenarios"])
         if sd.get("task", type(self).__name__) != type(self).__name__:
             raise ValueError(f"checkpoint of task {sd['task']!r} loaded into {type(self).__name__!r}")
         self._graph = None

@@ -44,6 +44,9 @@ class Quadcopter(VecTask):
         self._timeout_u8 = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
         self.timeout_buf = self._timeout_u8.view(torch.bool)
 
+    def set_scenarios(self, rows):
+        raise ValueError("Quadcopter: scenario tables are not supported (its step kernel does not apply them)")
+
     def create_sim(self):
         n, dev = self.num_envs, self.device
         env, sim = self.cfg["env"], self.cfg.get("sim", {})
