@@ -15,13 +15,11 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libouzelum_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 # Floating-point contract: EVERY translation unit is compiled without FMA contraction (-fmad=false); fused multiply-adds are
 # written explicitly (fmaf / fma) where they pay.  The env-step arithmetic is therefore bit-exact against the op-ordered CPU
 # oracles wherever it is instantiated (quad_step.cu, quadcopter.cu AND the one-launch EKFLeeLanded step), and the estimator /
 # controller device functions give identical bits in the fused kernel and in the stand-alone companion kernels.
-FMAD_OFF = None          # all
-FMAD = os.environ.get("OZL_COMPANION_FMAD", "false")
+FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC", "-fmad=false"]
 
 
 def sources():
@@ -45,8 +43,7 @@ def build(force=False, verbose=False):
     for src in sources():
         name = os.path.basename(src)
         obj = os.path.join(objdir, name[:-3] + ".o")
-        fmad = "false" if (FMAD_OFF is None or name in FMAD_OFF) else FMAD
-        cmd = [NVCC] + FLAGS + ["-fmad=" + fmad] + (["-Xptxas", "-v"] if verbose else []) + ["-c", "-o", obj, src]
+        cmd = [NVCC] + FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", "-o", obj, src]
         procs.append((cmd, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)))
         objs.append(obj)
     for cmd, pr in procs:

@@ -7,10 +7,8 @@
 //     whole task step (vehicle kernel, this kernel, step kernel) takes no host-changing argument: CUDA-graph capturable
 //   * traffic per env: root 72 B + EKF 2x160 B + PV 2x360 B + ~100 B of glue  (config 3: ~1.3 KB / env-step with the step kernel;
 //     L2-resident in steady state at 65536 envs)
-// (OZL_PHILOX_NOINLINE would keep ONE out-of-line copy of the counter RNG for the ~22 draw sites of this kernel: 20 KB less code,
-//  but measured slower on B200 -- 28.2 vs 27.1 us per 65536-env step -- so the draws stay inline)
-#include <cstdlib>
-#include <cuda.h>              // CUtensorMap (types only: the encoder is looked up through cudaGetDriverEntryPoint, no libcuda link)
+// (the counter-RNG draws stay inline: one out-of-line copy shared by the ~22 draw sites of this kernel is 20 KB less code but
+//  measured slower on B200, 28.2 vs 27.1 us per 65536-env step)
 #include "internal.h"
 #include "bulk_copy.cuh"
 #include "quad_io.cuh"
@@ -20,19 +18,8 @@
 #include "lee_control.cuh"
 #include "tile_chain.cuh"
 
-// Profiling aid (profiles/build_variant.sh ... "-DOZL_ABLATE=<bits>"): drop one stage of the fused step to time the rest.  Results are
-// wrong with any bit set; the product build has OZL_ABLATE == 0 and the branches below fold away.
-#ifndef OZL_ABLATE
-#define OZL_ABLATE 0
-#endif
-// bits: 1 sensor faults, 2 EKF, 4 PV predict, 8 PV fixes, 16 Lee controller, 32 env step, 64 covariance tile in / out,
-//       128 EKF state loads / stores
-#define OZL_KEEP(bit) (!(OZL_ABLATE & (bit)))
-#ifndef OZL_PV_COOP
-#define OZL_PV_COOP 1       // warp-cooperative PV fixes (filters.cuh, pv_correct_coop); 0 = every thread runs its own fixes
-#endif
-constexpr int kEkfSmemRows = 81 + (OZL_PV_COOP ? 12 : 0);   // covariance tile (+ the cooperative fixes' scratch columns), floats per env
-constexpr int kWarpTile = kEkfSmemRows * 32;                // floats of shared memory per WARP: [81][32] tile (+ [12][32] scratch)
+constexpr int kEkfSmemRows = 81 + 12;                      // covariance tile + the cooperative fixes' scratch columns, floats per env
+constexpr int kWarpTile = kEkfSmemRows * 32;                // floats of shared memory per WARP: [81][32] tile + [12][32] scratch
 
 namespace ozl {
 
@@ -56,12 +43,13 @@ struct EkfLeeArgs {
     LeeGains g;
 };
 
-// Envs per CTA: 64 (8 CTAs / SM), 96 (5), 128 (4), 256 (2) or 512 (1) at 128 registers per thread.  Measured on B200 at config 3
+// Envs per CTA: 96 (5 CTAs per SM at 128 registers per thread; 64-env CTAs fit 8, 128 fit 4, 256 fit 2, 512 fit 1).  Measured on B200 at config 3
 // (65536 envs, one wave): 96 -> 27.1 us, 128 -> 28.4 us, 64 -> 29.4 us, 256 -> +0.1 us over 128, 512 -> +1.3 us.  (Final kernel, warp-private
 // tiles: 96 -> 23.8 us, 64 -> 24.3 us, 128 -> 24.7 us, 32 -> 26.5 us.)  65536 envs
 // are 443 envs per SM: with 128-env CTAs the SMs hold 3 or 4 of them (12 or 16 warps) and the launch lasts as long as the SMs
-// with 16; 96-env CTAs spread the same envs as 4 or 5 CTAs (12 or 15 warps).  See ozl_ekf_lee_block().
-constexpr int ekf_minb(int block) { return block <= 64 ? 8 : (block <= 96 ? 5 : (block <= 128 ? 4 : (block <= 256 ? 2 : 1))); }
+// with 16; 96-env CTAs spread the same envs as 4 or 5 CTAs (12 or 15 warps).
+constexpr int kEkfLeeBlock = 96;
+constexpr int kEkfLeeMinBlocks = 5;
 
 // Layout of the work inside a CTA (one env per thread, kEkfBlock envs per CTA, shared memory WARP-PRIVATE):
 //   * each warp's [81][32] slice of the PV covariance planes is brought into its own shared-memory tile by ONE 2-D tensor-map copy
@@ -86,16 +74,10 @@ struct StepIo {
     float* obs; float* rew; int64_t* reset; int64_t* progress; uint8_t* timeout; float* ep_ret;
 };
 
-#ifdef OZL_EKF_MAXNREG
-#define OZL_EKF_BOUNDS(B) __maxnreg__(OZL_EKF_MAXNREG)
-#else
-#define OZL_EKF_BOUNDS(B) __launch_bounds__(B, ekf_minb(B))
-#endif
 template <int kEkfBlock, bool WITH_STEP>
-__global__ void OZL_EKF_BOUNDS(kEkfBlock)
-ekf_lee_fused_kernel(const __grid_constant__ DevCfg c, const Planes pl, const EkfLeeArgs a, const int use_tma_arg, const HuskyArgs h, const StepIo io,
+__global__ void __launch_bounds__(kEkfBlock, kEkfLeeMinBlocks)
+ekf_lee_fused_kernel(const __grid_constant__ DevCfg c, const Planes pl, const EkfLeeArgs a, const int use_tma, const HuskyArgs h, const StepIo io,
                      const int chain, const __grid_constant__ CUtensorMap tmap) {
-    const int use_tma = OZL_KEEP(64) ? use_tma_arg : 0;
     static_assert(kEkfBlock % 32 == 0, "whole warps");
     // Shared memory is WARP-PRIVATE: warp w owns [81][32] floats of covariance tile (+ [12][32] of scratch for the cooperative
     // fixes), its own mbarrier, and later stages its [32][13] observation rows in the same tile.  Nothing after the step-index
@@ -163,7 +145,7 @@ ekf_lee_fused_kernel(const __grid_constant__ DevCfg c, const Planes pl, const Ek
             mbar_expect_tx(s_bar, 81u * 32u * 4u);
             tma_load_2d(s_P, &tmap, (int32_t)wbase, 0, s_bar);
         }
-    } else if (valid && OZL_KEEP(64)) {
+    } else if (valid) {
 #pragma unroll 3          // fallback path (N % 4 != 0 or no tensor map): kept small, this kernel is instruction-fetch bound
         for (int k = 0; k < 81; ++k) s_P[k * 32 + lane] = a.pv_P[(int64_t)k * a.n + i];
     }
@@ -191,9 +173,8 @@ ekf_lee_fused_kernel(const __grid_constant__ DevCfg c, const Planes pl, const Ek
         // ---- attitude-EKF state: loads issued here (L2 hits), consumed after the sensor front-end
         EKF4 s;
         if (warm || rst) { s.q[0] = q[3]; s.q[1] = q[0]; s.q[2] = q[1]; s.q[3] = q[2]; }
-        else if (OZL_KEEP(128)) { for (int k = 0; k < 4; ++k) s.q[k] = a.ekf_q[(int64_t)k * a.n + i]; }
-        else { s.q[0] = 1.0; s.q[1] = s.q[2] = s.q[3] = 0.0; }
-        for (int k = 0; k < 16; ++k) s.P[k / 4][k % 4] = OZL_KEEP(128) ? a.ekf_P[(int64_t)k * a.n + i] : (k % 5 == 0 ? 1.0 : 0.0);
+        else { for (int k = 0; k < 4; ++k) s.q[k] = a.ekf_q[(int64_t)k * a.n + i]; }
+        for (int k = 0; k < 16; ++k) s.P[k / 4][k % 4] = a.ekf_P[(int64_t)k * a.n + i];
         // ---- sensor front-end (:345-346,366-375,397-406)
         FaultCfg f = a.f;
         f.step = step;
@@ -206,13 +187,11 @@ ekf_lee_fused_kernel(const __grid_constant__ DevCfg c, const Planes pl, const Ek
         }
         acc[2] = acc[2] + 9.8f;
         for (int j = 0; j < 4; ++j) ang[j] = q[j];
-        if (OZL_KEEP(1)) {
-            sensor_fault(f, genv, 1, false, gyr, 3);
-            sensor_fault(f, genv, 3, true, ang, 4);
-            sensor_fault(f, genv, 4, false, acc, 3);
-            sensor_fault(f, genv, 5, false, pos, 3);
-            sensor_fault(f, genv, 6, false, vel, 3);
-        }
+        sensor_fault(f, genv, 1, false, gyr, 3);
+        sensor_fault(f, genv, 3, true, ang, 4);
+        sensor_fault(f, genv, 4, false, acc, 3);
+        sensor_fault(f, genv, 5, false, pos, 3);
+        sensor_fault(f, genv, 6, false, vel, 3);
         // ---- PV state: loads issued before the EKF arithmetic, consumed after it
         PVShared<32> pvs;
         pvs.P = s_P + lane;
@@ -222,35 +201,30 @@ ekf_lee_fused_kernel(const __grid_constant__ DevCfg c, const Planes pl, const Ek
         {
             const double gd[3] = {(double)gyr[0], (double)gyr[1], (double)gyr[2]};
             const double ad[4] = {(double)ang[3], (double)ang[0], (double)ang[1], (double)ang[2]};
-            if (OZL_KEEP(2)) ekf_update(s, gd, ad, a.ekf_Dt, a.ekf_g_noise, 0.0000001);
-            for (int k = 0; k < 4; ++k) { if (OZL_KEEP(128)) a.ekf_q[(int64_t)k * a.n + i] = s.q[k]; q32[k] = (float)s.q[k]; }
-            if (OZL_KEEP(128)) { for (int k = 0; k < 16; ++k) a.ekf_P[(int64_t)k * a.n + i] = s.P[k / 4][k % 4]; }
+            ekf_update(s, gd, ad, a.ekf_Dt, a.ekf_g_noise, 0.0000001);
+            for (int k = 0; k < 4; ++k) { a.ekf_q[(int64_t)k * a.n + i] = s.q[k]; q32[k] = (float)s.q[k]; }
+            for (int k = 0; k < 16; ++k) a.ekf_P[(int64_t)k * a.n + i] = s.P[k / 4][k % 4];
         }
         // ---- PV filter (:353-358,397-444) on the shared-memory covariance tile
         {
             if (rst) { for (int k = 0; k < 3; ++k) { pvs.x[k] = p[k]; pvs.x[3 + k] = v[k]; pvs.x[6 + k] = 0.f; } }
             const float qt[4] = {q[3], q[0], q[1], q[2]};
             if (use_tma) mbar_wait(s_bar, 0);                    // the covariance tile has landed
-            if (OZL_KEEP(4)) pv_predict(pvs, acc, warm ? qt : q32, a.dt, a.dt2, a.acc_var);
+            pv_predict(pvs, acc, warm ? qt : q32, a.dt, a.dt2, a.acc_var);
             // shared sensor-trigger counters (:425-440): the reference advances them once per env-iteration, i.e. the k-th
             // iteration overall is step * N_total + GLOBAL env id (invariant to how the envs are sharded over GPUs)
             const uint64_t k = a.per_env_triggers ? step : step * (uint64_t)a.n_total + (uint64_t)genv;
-            const bool fix_pos = OZL_KEEP(8) && a.pos_period && (k % a.pos_period) == a.pos_phase;
-            const bool fix_vel = OZL_KEEP(8) && a.vel_period && (k % a.vel_period) == a.vel_phase;
+            const bool fix_pos = a.pos_period && (k % a.pos_period) == a.pos_phase;
+            const bool fix_vel = a.vel_period && (k % a.vel_period) == a.vel_phase;
             const float zero3[3] = {0.f, 0.f, 0.f};                                                  // gps_var=None => R = 0
-#if OZL_PV_COOP
             // warp-cooperative fixes (filters.cuh): first fix of every env, then the velocity fix of the envs that had both
             float* const scr = s_P + 81 * 32 + lane;
             pv_correct_coop(pvs, scr, wmask, lane, fix_pos ? 0 : (fix_vel ? 3 : -1), fix_pos ? pos : vel, a.pos_var, zero3);
             pv_correct_coop(pvs, scr, wmask, lane, (fix_pos && fix_vel) ? 3 : -1, vel, a.pos_var, zero3);
-#else
-            if (fix_pos) pv_correct<0>(pvs, pos, a.pos_var);
-            if (fix_vel) pv_correct<3>(pvs, vel, zero3);
-#endif
             for (int kk = 0; kk < 9; ++kk) a.pv_x[(int64_t)kk * a.n + i] = pvs.x[kk];
             for (int kk = 0; kk < 3; ++kk) { est_p[kk] = pvs.x[kk]; est_v[kk] = pvs.x[3 + kk]; }
         }
-        if (!use_tma && OZL_KEEP(64)) {
+        if (!use_tma) {
 #pragma unroll 3
             for (int k = 0; k < 81; ++k) a.pv_P[(int64_t)k * a.n + i] = s_P[k * 32 + lane];
         }
@@ -284,7 +258,7 @@ ekf_lee_fused_kernel(const __grid_constant__ DevCfg c, const Planes pl, const Ek
     }
     float4 wr = make_float4(0.f, 0.f, 0.f, 0.f);
     if (valid) {
-        if (warm || !OZL_KEEP(16)) {
+        if (warm) {
             wr = make_float4(a.hover, 0.f, 0.f, 0.f);                                     // :526-528
         } else {
             float th, tq[3];
@@ -306,10 +280,8 @@ ekf_lee_fused_kernel(const __grid_constant__ DevCfg c, const Planes pl, const Ek
         Env e;
         unpack(L, e);
         const float act[4] = {wr.x, wr.y, wr.z, wr.w};
-        if (OZL_KEEP(32)) {
-            env_step(e, act, prog, rst, genv, step, c, o, ACT_WRENCH, tgt);
-            obs_epilogue(o.obs, genv, step, flicker_blackout(step, c), c);
-        }
+        env_step(e, act, prog, rst, genv, step, c, o, ACT_WRENCH, tgt);
+        obs_epilogue(o.obs, genv, step, flicker_blackout(step, c), c);
         store_dynamic(pl, i, e);
         store_static(pl, i, e);
         io.rew[i] = o.rew;
@@ -350,44 +322,17 @@ ekf_lee_fused_kernel(const __grid_constant__ DevCfg c, const Planes pl, const Ek
 
 using namespace ozl;
 
-// Envs per CTA of the fused kernel (default 96, see above); OZL_EKF_BLOCK (64 / 96 / 128 / 256 / 512) overrides it for experiments.
-static int ozl_ekf_lee_block(const ozl_env* env, int64_t n) {
-    static int forced = -1;
-    if (forced < 0) {
-        const char* v = getenv("OZL_EKF_BLOCK");
-        forced = v ? atoi(v) : 0;
-        if (forced != 0 && forced != 64 && forced != 96 && forced != 128 && forced != 256 && forced != 512) forced = 0;
-    }
-    if (forced) return forced;
-    (void)env; (void)n;
-    return 96;
-}
-
 // 2-D tensor map over the caller's [81][N] covariance planes, box = [81][32] = one warp's envs (cached in the handle: the pointer is
 // fixed per task).
-// Returns 0 when env->pv_tmap is valid for (P, block).
+// Returns 0 when env->pv_tmap is valid for P.
 static int ozl_encode_pv_tmap(ozl_env* env, const float* P, int64_t n) {
-    const int block = 32;                                         // one box per warp
-    if (env->pv_tmap_ptr == P && env->pv_tmap_block == block) return 0;
-    if (n < block) return 1;
-    typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                 const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                 CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    static EncodeFn fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = (EncodeFn)p;
-        else
-            cudaGetLastError();
-    }
+    if (env->pv_tmap_ptr == P) return 0;
+    if (n < 32) return 1;
+    const PFN_cuTensorMapEncodeTiled fn = tensor_map_encoder();
     if (!fn) return 1;
     const cuuint64_t gdim[2] = {(cuuint64_t)n, 81ull};
     const cuuint64_t gstr[1] = {(cuuint64_t)n * sizeof(float)};
-    const cuuint32_t box[2] = {(cuuint32_t)block, 81u};
+    const cuuint32_t box[2] = {32u, 81u};
     const cuuint32_t estr[2] = {1u, 1u};
     if (fn(reinterpret_cast<CUtensorMap*>(env->pv_tmap), CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(P), gdim, gstr, box, estr,
            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
@@ -396,7 +341,6 @@ static int ozl_encode_pv_tmap(ozl_env* env, const float* P, int64_t n) {
         return 1;
     }
     env->pv_tmap_ptr = P;
-    env->pv_tmap_block = block;
     return 0;
 }
 
@@ -442,16 +386,11 @@ static int launch_ekf_lee(ozl_env* env, const ozl_ekf_lee_args* in, const ozl_hu
     // capture, with nothing captured in between (the stream's one dependency is that launch's node)
     // Chaining pays when the grid is several waves long (262144 envs: 125 -> 110 us per step); a ONE-wave grid runs in lockstep
     // either way and only pays the protocol's latency (65536 envs: 27.2 -> 33 us), so it keeps the classic launch (chain = -1).
-    const int block = ozl_ekf_lee_block(env, a.n);
-    const unsigned grid = (unsigned)((a.n + block - 1) / block);
-    const size_t smem = (size_t)kEkfSmemRows * block * sizeof(float);
-    {
-        static int tmap_mode = -1;                                  // OZL_EKF_TMAP=0: keep the 81 plane copies
-        if (tmap_mode < 0) { const char* v = getenv("OZL_EKF_TMAP"); tmap_mode = v ? atoi(v) : 1; }
-        if (tmap_mode && (a.n % 4 == 0) && (((uintptr_t)a.pv_P & 15) == 0) && ozl_encode_pv_tmap(env, a.pv_P, a.n) == 0) use_tma = 1;
-    }
-    const long long slots = (long long)env->sm_count * ekf_minb(block);
-    const bool may_chain = husky && env->use_pdl && (env->chain_mode == 2 || (env->chain_mode == 1 && (long long)grid > slots));
+    const unsigned grid = (unsigned)((a.n + kEkfLeeBlock - 1) / kEkfLeeBlock);
+    const size_t smem = (size_t)kEkfSmemRows * kEkfLeeBlock * sizeof(float);
+    if ((a.n % 4 == 0) && (((uintptr_t)a.pv_P & 15) == 0) && ozl_encode_pv_tmap(env, a.pv_P, a.n) == 0) use_tma = 1;
+    const long long slots = (long long)env->sm_count * kEkfLeeMinBlocks;
+    const bool may_chain = husky && (env->chain_mode == 2 || (env->chain_mode == 1 && (long long)grid > slots));
     int chain = may_chain ? 0 : -1;
     if (may_chain && env->chain_last_node) {
         cudaStreamCaptureStatus cs; unsigned long long cid = 0; size_t nd = 0;
@@ -463,27 +402,15 @@ static int launch_ekf_lee(ozl_env* env, const ozl_ekf_lee_args* in, const ozl_hu
             cudaGetLastError();
         }
     }
-    int rc;
-#define OZL_LAUNCH_EKF(B, WS)                                                                                                   \
-    do {                                                                                                                        \
-        static bool attr_set = false;                                                                                           \
-        if (!attr_set) {                                                                                                        \
-            if (check_cuda(cudaFuncSetAttribute(ekf_lee_fused_kernel<B, WS>, cudaFuncAttributeMaxDynamicSharedMemorySize,      \
-                                                kEkfSmemRows * B * (int)sizeof(float)), "cudaFuncSetAttribute")) return 1;     \
-            attr_set = true;                                                                                                    \
-        }                                                                                                                       \
-        rc = launch_pdl_smem(env, ekf_lee_fused_kernel<B, WS>, dim3(grid), dim3(B), smem, (cudaStream_t)stream, env->dev,       \
-                             env->pl, a, use_tma, h, io, chain, *reinterpret_cast<const CUtensorMap*>(env->pv_tmap));          \
-    } while (0)
-    if (husky) {
-        if (block == 512) OZL_LAUNCH_EKF(512, true); else if (block == 256) OZL_LAUNCH_EKF(256, true);
-        else if (block == 64) OZL_LAUNCH_EKF(64, true); else if (block == 128) OZL_LAUNCH_EKF(128, true); else OZL_LAUNCH_EKF(96, true);
-    } else {
-        if (block == 512) OZL_LAUNCH_EKF(512, false); else if (block == 256) OZL_LAUNCH_EKF(256, false);
-        else if (block == 128) OZL_LAUNCH_EKF(128, false); else OZL_LAUNCH_EKF(96, false);
+    static bool attr_set[2] = {false, false};         // per kernel: the dynamic shared memory exceeds the 48 KB default
+    const auto kernel = husky ? ekf_lee_fused_kernel<kEkfLeeBlock, true> : ekf_lee_fused_kernel<kEkfLeeBlock, false>;
+    if (!attr_set[husky != nullptr]) {
+        if (check_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "cudaFuncSetAttribute")) return 1;
+        attr_set[husky != nullptr] = true;
     }
-#undef OZL_LAUNCH_EKF
-    if (rc) return check_cuda(cudaGetLastError(), "ekf_lee_fused_kernel");
+    if (launch_pdl_smem(kernel, dim3(grid), dim3(kEkfLeeBlock), smem, (cudaStream_t)stream, env->dev, env->pl, a, use_tma, h, io, chain,
+                        *reinterpret_cast<const CUtensorMap*>(env->pv_tmap)))
+        return check_cuda(cudaGetLastError(), "ekf_lee_fused_kernel");
     if (may_chain) {       // remember the node this launch became (if it was captured): the next launch may chain behind it
         cudaStreamCaptureStatus cs; unsigned long long cid = 0; size_t nd = 0;
         const cudaGraphNode_t* deps = nullptr;

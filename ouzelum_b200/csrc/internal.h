@@ -1,6 +1,7 @@
 // Internal (non-ABI) declarations shared by the translation units of libouzelum_b200.so.
 #pragma once
 #include <cuda_runtime.h>
+#include <cudaTypedefs.h>      // CUtensorMap and the encoder's type (no libcuda link: see tensor_map_encoder)
 #include <stdint.h>
 #include "../../include/ouzelum_b200.h"
 #include "quad_env.cuh"
@@ -9,51 +10,37 @@ namespace ozl {
 
 int set_error(const char* fmt, ...);   // stores a thread-local message, returns 1
 int check_cuda(cudaError_t e, const char* what);
+// cuTensorMapEncodeTiled, looked up once through cudaGetDriverEntryPoint; NULL if the driver does not provide it
+PFN_cuTensorMapEncodeTiled tensor_map_encoder();
 
-#ifndef OZL_METRIC_SLOTS
-#define OZL_METRIC_SLOTS 32
-#endif
-constexpr int kMetricSlots = OZL_METRIC_SLOTS;   // metric accumulators are striped over this many slots (256 B apart) to spread L2 atomics
+constexpr int kMetricSlots = 32;       // metric accumulators are striped over this many slots (256 B apart) to spread L2 atomics
 constexpr int kMetricStride = 32;      // doubles per slot (16 used)
 
 // Private state of one handle: float4-packed planes, so one env == one 16-byte lane per plane.
 //   dynamic (read+written every step):  d0 {px,py,pz,qx} d1 {qy,qz,qw,vx} d2 {vy,vz,wx,wy} d3 {wz,T0,T1,T2} d4 {T3,ep_ret}
 //   static  (read every step, written only on reset/resample):
 //           s0 {tx,ty,tz,fault_eff} s1 {mass,ixx,iyy,izz} s2 {arm,thrust_scale,fault_word,yaw_km}
-// Layout (OZL_TILED=1, default): tiles of kTile = 128 envs; inside a tile the planes are stored back to back
+// Layout: tiles of kTile = 128 envs; inside a tile the planes are stored back to back
 //   [d0 2 KiB][d1][d2][d3][d4 1 KiB][s0 2 KiB][s1][s2]  = 15360 bytes per tile
 // so the CTA that owns a tile reads ONE contiguous 15 KiB region and writes ONE contiguous 9 KiB region (long DRAM bursts,
 // 2 streams per CTA instead of 16), while a warp still touches 512 contiguous bytes per plane.
-// OZL_TILED=0 is the plain plane-major SoA ([plane][N]) kept for A/B measurements.
-#ifndef OZL_TILED
-#define OZL_TILED 1
-#endif
 constexpr int kTile = 128;
 constexpr int kTileBytes = kTile * (7 * 16 + 8);
 struct Planes {
     char* base;                 // arena
-    int64_t plane4, plane2;     // OZL_TILED=0: byte strides of the float4 / float2 planes
     unsigned long long* ctrl;   // [0..2] step-counter record {base, units, shift} (step_counter.cuh), [4] TMA-kernel tile scheduler (monotonic)
     double* metrics;            // kMetricSlots x kMetricStride
     unsigned long long* tile_seq;   // [tiles][2] {started, done}: per-tile step sequence of the tile-chained launches (tile_chain.cuh)
 };
 // k = 0..3: d0..d3, k = 4..6: s0..s2
 __device__ __forceinline__ float4* plane4_ptr(const Planes& pl, int k, int64_t i) {
-#if OZL_TILED
     const int64_t tile = i >> 7;
     const int lane = (int)(i & (kTile - 1));
     const int off = (k < 4 ? k * 2048 : 9216 + (k - 4) * 2048);
     return reinterpret_cast<float4*>(pl.base + tile * kTileBytes + off) + lane;
-#else
-    return reinterpret_cast<float4*>(pl.base + (int64_t)k * pl.plane4) + i;
-#endif
 }
 __device__ __forceinline__ float2* plane2_ptr(const Planes& pl, int64_t i) {
-#if OZL_TILED
     return reinterpret_cast<float2*>(pl.base + (i >> 7) * kTileBytes + 8192) + (int)(i & (kTile - 1));
-#else
-    return reinterpret_cast<float2*>(pl.base + 7 * pl.plane4) + i;
-#endif
 }
 
 }  // namespace ozl
@@ -65,19 +52,16 @@ struct ozl_env {
     int device;
     int sm_count;
     long long tma_min_tiles;    // >= this many whole tiles: use the persistent TMA-pipelined step kernel
-    int use_pdl;                // step launches carry the programmatic-stream-serialization attribute (see launch_step)
     void* arena;                // single cudaMalloc backing all planes
     size_t arena_bytes;
     // host-consumer steps: completion word in pinned host memory, written by the last block of a step kernel after all its
     // zero-copy result stores (ozl_step_host_sync / ozl_step_host_wait poll it instead of synchronising the stream)
-    volatile unsigned int* host_done;   // cudaHostAlloc'ed, one word
+    volatile unsigned int* host_done;   // cudaHostAlloc'ed, one word; NULL if that failed (stream synchronise instead)
     unsigned int host_seq;              // sequence number of the last host step launched
-    int use_host_flag;                  // OZL_HOST_FLAG=0 turns the completion word off (stream synchronise instead)
     // tile-chained step launches (tile_chain.cuh): the graph node of the last chained launch captured on this handle
-    // 2-D tensor map of the caller's [81][N] PV covariance planes with a [81][block] box (ekf_lee_fused.cu), cached per (pointer, block)
+    // 2-D tensor map of the caller's [81][N] PV covariance planes with a [81][32] box (ekf_lee_fused.cu), cached per pointer
     alignas(64) unsigned char pv_tmap[128];
     const void* pv_tmap_ptr;
-    int pv_tmap_block;
     int chain_mode;                     // OZL_EKF_CHAIN: 0 = never chain, 1 = chain launches that are provably adjacent in a stream capture
     unsigned long long chain_capture_id;
     void* chain_last_node;
@@ -96,7 +80,7 @@ struct ozl_env {
 // consecutive steps on a stream are strictly dependent, but the NEXT step's blocks can be made resident and parked in
 // griddep_wait() while the current step drains, which takes the launch latency off the critical path of short steps.
 template <typename... KArgs, typename... Args>
-static inline int launch_pdl_smem(ozl_env* env, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+static inline int launch_pdl_smem(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
                                   Args... args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
@@ -104,18 +88,11 @@ static inline int launch_pdl_smem(ozl_env* env, void (*kernel)(KArgs...), dim3 g
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = env->use_pdl ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...) != cudaSuccess;
 }
 template <typename... KArgs, typename... Args>
-static inline int launch_pdl(ozl_env* env, void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t st, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = 0; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = env->use_pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...) != cudaSuccess;
+static inline int launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t st, Args... args) {
+    return launch_pdl_smem(kernel, grid, block, 0, st, args...);
 }
 

@@ -253,7 +253,7 @@ extern "C" int ozl_metrics_push(ozl_env* env, ozl_metrics_xchg* x, double* local
     XDev d;
     if (xdev_of(x, d, "ozl_metrics_push")) return 1;
     if (x->device != env->device) return set_error("ozl_metrics_push: exchange on device %d, env on device %d", x->device, env->device);
-    if (launch_pdl(env, metrics_push_kernel, dim3(1), dim3(512), (cudaStream_t)stream, env->pl, d, local16, prev_sum16, (int)clear))
+    if (launch_pdl(metrics_push_kernel, dim3(1), dim3(512), (cudaStream_t)stream, env->pl, d, local16, prev_sum16, (int)clear))
         return check_cuda(cudaGetLastError(), "metrics_push_kernel");
     return 0;
 }
@@ -262,7 +262,7 @@ extern "C" int ozl_metrics_sum(ozl_env* env, ozl_metrics_xchg* x, double* sum16,
     if (!env || !sum16) return set_error("ozl_metrics_sum: NULL argument");
     XDev d;
     if (xdev_of(x, d, "ozl_metrics_sum")) return 1;
-    if (launch_pdl(env, metrics_sum_kernel, dim3(1), dim3(512), (cudaStream_t)stream, d, sum16))
+    if (launch_pdl(metrics_sum_kernel, dim3(1), dim3(512), (cudaStream_t)stream, d, sum16))
         return check_cuda(cudaGetLastError(), "metrics_sum_kernel");
     return 0;
 }

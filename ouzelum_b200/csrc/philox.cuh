@@ -22,15 +22,9 @@ enum : uint32_t {
 };
 constexpr uint32_t GLOBAL_ENV = 0xFFFFFFFFu;
 
-// OZL_PHILOX_NOINLINE (defined by a TU before including this header): keep ONE copy of the 10 rounds and call it.  The fused
-// EKFLeeLanded kernel has ~22 draw sites (~70 instructions each inlined); out of line its code shrinks by ~20 KB, which matters
-// there because the kernel is far larger than the 32 KB L1.5 instruction cache.  The step kernels keep it inline (measured).
-#ifdef OZL_PHILOX_NOINLINE
-#define OZL_PHILOX_ATTR __noinline__
-#else
-#define OZL_PHILOX_ATTR __forceinline__
-#endif
-static __device__ OZL_PHILOX_ATTR uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
+// Inline everywhere, including the fused EKFLeeLanded kernel, where one out-of-line copy would save ~20 KB of code but was
+// measured slower (ekf_lee_fused.cu).
+static __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
     constexpr uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
 #pragma unroll
     for (int r = 0; r < 10; ++r) {

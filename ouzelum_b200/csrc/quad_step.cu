@@ -5,7 +5,6 @@
 #include <cstring>
 #include <cstdlib>
 #include <cmath>
-#include <cuda.h>              // CUtensorMap (types only: the encoder is looked up through cudaGetDriverEntryPoint)
 #include "internal.h"
 #include "bulk_copy.cuh"
 #include "quad_io.cuh"
@@ -27,17 +26,20 @@ int check_cuda(cudaError_t e, const char* what) {
     if (e == cudaSuccess) return 0;
     return set_error("%s: %s", what, cudaGetErrorString(e));
 }
+PFN_cuTensorMapEncodeTiled tensor_map_encoder() {
+    static const PFN_cuTensorMapEncodeTiled fn = [] {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+            return (PFN_cuTensorMapEncodeTiled)p;
+        cudaGetLastError();
+        return (PFN_cuTensorMapEncodeTiled)nullptr;
+    }();
+    return fn;
+}
 
 // ------------------------------------------------------------------------------------------------ K1
-#ifndef OZL_OBS_BULK
-#define OZL_OBS_BULK 1
-#endif
-#ifndef OZL_STEP_BLOCK
-#define OZL_STEP_BLOCK 128
-#endif
-#ifndef OZL_STEP_MINB
-#define OZL_STEP_MINB 7
-#endif
+constexpr int kStepMinBlocks = 7;      // 128-env CTAs resident per SM (the one-wave limit behind tma_min_tiles)
 // FRONT selects what runs in front of the env step inside the same thread (one launch per control step for every task):
 //   FRONT_NONE     nothing: Ouzelum, Lando, the tracking / wrench variants fed from caller buffers
 //   FRONT_VEHICLE  the waypoint-following ground vehicle that carries the target (targets.cuh): Landing, Landed
@@ -146,11 +148,7 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
 #pragma unroll
         for (int j = 0; j < 13; ++j) s_obs[threadIdx.x * 13 + j] = o.obs[j];   // stride 13: conflict-free
     }
-#if OZL_OBS_BULK
     fence_proxy_async_smem();          // make the generic-proxy smem writes visible to the bulk-copy (async) proxy
-#else
-    if constexpr (STATES) fence_proxy_async_smem();
-#endif
     __syncthreads();
     // [N,13] row-major observation tile of this block is contiguous: write it with full 16-byte lanes
     const int64_t remaining = c.num_envs - base;
@@ -159,7 +157,6 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
         float* dst = obs + base * 13;
         const int nflt = n_here * 13;
         if ((nflt & 3) == 0) {   // base*13*4 bytes is 16-byte aligned whenever BLOCK % 4 == 0
-#if OZL_OBS_BULK
             if (obs_bulk) {
                 if (threadIdx.x == 0) bulk_store_s2g(dst, s_obs, (uint32_t)nflt * 4u);
             } else {
@@ -167,15 +164,6 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
                 const float4* s4 = reinterpret_cast<const float4*>(s_obs);
                 for (int k = threadIdx.x; k < nflt / 4; k += BLOCK) d4p[k] = s4[k];
             }
-#else
-            float4* d4p = reinterpret_cast<float4*>(dst);
-            const float4* s4 = reinterpret_cast<const float4*>(s_obs);
-#pragma unroll
-            for (int it = 0; it < (BLOCK * 13 / 4 + BLOCK - 1) / BLOCK; ++it) {
-                const int k = threadIdx.x + it * BLOCK;
-                if (k < nflt / 4) d4p[k] = s4[k];
-            }
-#endif
         } else {
             for (int k = threadIdx.x; k < nflt; k += BLOCK) dst[k] = s_obs[k];
         }
@@ -187,11 +175,7 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
     // one work unit per block; block 0 of the full-range launch also retires the padding (env0 != 0: ragged-tail launch
     // behind the TMA kernel, which has retired the padding already)
     block_epilogue<BLOCK>(c, pl, valid, o, n_here, 1ull + ((blockIdx.x == 0 && env0 == 0) ? (unsigned long long)c.step_pad : 0ull));
-#if OZL_OBS_BULK
     if (threadIdx.x == 0) bulk_wait_read_all();   // s_obs (and s_states) must stay alive until the bulk copies have read them
-#else
-    if constexpr (STATES) { if (threadIdx.x == 0) bulk_wait_read_all(); }
-#endif
     // Host consumer: completion word.  Every block orders its zero-copy result stores before a ticket (the barrier makes the
     // block's stores visible to thread 0, the system-scope fence orders them before the ticket); the block that draws the last
     // ticket writes the step's sequence number to pinned host memory, where the host is polling -- no stream synchronise, whose
@@ -212,12 +196,12 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
 }
 
 template <int BLOCK, int FRONT, bool STATES>
-__global__ void __launch_bounds__(BLOCK, OZL_STEP_MINB)
+__global__ void __launch_bounds__(BLOCK, kStepMinBlocks)
 quad_step_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
     quad_step_body<BLOCK, FRONT, STATES, false>(OZL_STEP_ARGS);
 }
 template <int BLOCK, int FRONT, bool STATES>
-__global__ void __launch_bounds__(BLOCK, OZL_STEP_MINB)
+__global__ void __launch_bounds__(BLOCK, kStepMinBlocks)
 quad_step_scn_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
     quad_step_body<BLOCK, FRONT, STATES, true>(OZL_STEP_ARGS);
 }
@@ -237,9 +221,7 @@ constexpr int kTmaProgOff = kTmaActOff + kTile * 16;              // progress [1
 constexpr int kTmaRstOff = kTmaProgOff + kTile * 8;               // reset    [128] int64    1024 B
 constexpr int kTmaStageBytes = kTmaRstOff + kTile * 8;            // 19456
 
-#ifndef OZL_TMA_MINB
-#define OZL_TMA_MINB 5
-#endif
+constexpr int kTmaMinBlocks = 5;       // CTAs per SM of the TMA kernel, and its persistent grid's slots per SM
 #define OZL_TMA_PARAMS                                                                                                          \
     const DevCfg c, const Planes pl, const float4* __restrict__ actions, float* __restrict__ obs, float* __restrict__ rew,       \
         int64_t* __restrict__ reset, int64_t* __restrict__ progress, uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, \
@@ -384,12 +366,12 @@ __device__ __forceinline__ void quad_step_tma_body(OZL_TMA_PARAMS, const CUtenso
 }
 
 template <bool STATES>
-__global__ void __launch_bounds__(kTile, OZL_TMA_MINB)
+__global__ void __launch_bounds__(kTile, kTmaMinBlocks)
 quad_step_tma_kernel(OZL_TMA_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
     quad_step_tma_body<STATES, false>(OZL_TMA_ARGS);
 }
 template <bool STATES>
-__global__ void __launch_bounds__(kTile, OZL_TMA_MINB)
+__global__ void __launch_bounds__(kTile, kTmaMinBlocks)
 quad_step_tma_scn_kernel(OZL_TMA_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
     quad_step_tma_body<STATES, true>(OZL_TMA_ARGS);
 }
@@ -800,22 +782,19 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
         //   163840 envs (1280 tiles, a second generic wave of 244 CTAs): generic warm 10.29, cold 13.51; 180224 envs on the TMA kernel 10.34 / 11.16
         // (round 1's kernels crossed over at ~400k envs; the lighter integrator moved the crossover down)
         // (override: OZL_TMA_MIN_TILES, 0 = never)
-        const char* pv = getenv("OZL_PDL");
-        e->use_pdl = pv ? atoi(pv) : 1;
         const char* ev = getenv("OZL_TMA_MIN_TILES");
-        e->tma_min_tiles = ev ? atoll(ev) : 7ll * prop.multiProcessorCount + 1;
+        e->tma_min_tiles = ev ? atoll(ev) : (long long)kStepMinBlocks * prop.multiProcessorCount + 1;
     }
     const size_t n = (size_t)cfg->num_envs;
     const size_t tiles = (n + kTile - 1) / kTile;
-    const size_t plane4 = align_up(tiles * kTile * sizeof(float4), 256), plane2 = align_up(tiles * kTile * sizeof(float2), 256);
-    const size_t state = OZL_TILED ? align_up(tiles * (size_t)kTileBytes, 256) : 7 * plane4 + plane2;
+    const size_t state = align_up(tiles * (size_t)kTileBytes, 256);
     const size_t ctrl = 256, metrics = align_up(sizeof(double) * kMetricSlots * kMetricStride, 256);
     const size_t tile_seq = align_up(tiles * 4 * sizeof(unsigned long long), 256);    // {started, done} per CTA of >= 64 envs
     e->arena_bytes = state + ctrl + metrics + tile_seq;
     if (check_cuda(cudaMalloc(&e->arena, e->arena_bytes), "cudaMalloc(state arena)")) { delete e; return 1; }
     if (check_cuda(cudaMemset(e->arena, 0, e->arena_bytes), "cudaMemset(state arena)")) { cudaFree(e->arena); delete e; return 1; }
     char* p = (char*)e->arena;
-    e->pl.base = p; e->pl.plane4 = (int64_t)plane4; e->pl.plane2 = (int64_t)plane2;
+    e->pl.base = p;
     p += state;
     e->pl.ctrl = (unsigned long long*)p; p += ctrl;
     e->pl.metrics = (double*)p; p += metrics;
@@ -826,15 +805,12 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
         e->chain_capture_id = 0;
         e->chain_last_node = nullptr;
         e->pv_tmap_ptr = nullptr;
-        e->pv_tmap_block = 0;
     }
     {
-        const char* hv = getenv("OZL_HOST_FLAG");
-        e->use_host_flag = hv ? atoi(hv) : 1;
         e->host_done = nullptr;
         e->host_seq = 0;
         void* hp = nullptr;
-        if (e->use_host_flag && cudaHostAlloc(&hp, 64, cudaHostAllocMapped | cudaHostAllocPortable) == cudaSuccess) {
+        if (cudaHostAlloc(&hp, 64, cudaHostAllocMapped | cudaHostAllocPortable) == cudaSuccess) {
             memset(hp, 0, 64);
             e->host_done = (volatile unsigned int*)hp;
         } else {
@@ -871,7 +847,7 @@ extern "C" int ozl_reset_all(ozl_env* env, uint64_t seed, void* stream) {
 }
 
 // Block size: 128 threads keeps >= 1 block on every SM down to ~19k envs and lets 16k-env launches use 128 SMs.
-constexpr int kStepBlock = OZL_STEP_BLOCK;
+constexpr int kStepBlock = 128;
 static_assert(kStepBlock == kTile, "the step counter retires one work unit per 128-env tile == one block of the generic kernel");
 
 // The states tensor map of the handle (zeros while no states buffer is registered: the STATES = false kernels never read it)
@@ -886,7 +862,7 @@ static int launch_step_t(ozl_env* env, const float* actions, const float* target
     if (((uintptr_t)actions & 15) || ((uintptr_t)obs & 15)) return set_error("%s: actions/obs must be 16-byte aligned", who);
     const int64_t n = env->cfg.num_envs;
     const int64_t full_tiles = n / kTile, tail = n % kTile;
-    const int64_t resident = (int64_t)env->sm_count * OZL_TMA_MINB;
+    const int64_t resident = (int64_t)env->sm_count * kTmaMinBlocks;
     const bool plain = (target_in == nullptr) && act_mode == ACT_ROTORS && done_u8 == nullptr && reset_mirror == nullptr && obs_bulk;
     const auto tma_kernel = SCN ? quad_step_tma_scn_kernel<STATES> : quad_step_tma_kernel<STATES>;
     const auto kernel = SCN ? quad_step_scn_kernel<kStepBlock, FRONT_NONE, STATES> : quad_step_kernel<kStepBlock, FRONT_NONE, STATES>;
@@ -895,7 +871,7 @@ static int launch_step_t(ozl_env* env, const float* actions, const float* target
         // large N: persistent TMA-pipelined kernel over the whole tiles, then one generic block for the ragged tail
         unsigned grid = (unsigned)(full_tiles < resident ? full_tiles : resident);
         while ((full_tiles + grid - 1) / grid > 8192) grid *= 2;     // 16-bit packed metric counters: keep tiles per CTA far below 65535
-        if (launch_pdl(env, tma_kernel, dim3(grid), dim3(kTile), st, env->dev, env->pl, (const float4*)actions, obs, rew,
+        if (launch_pdl(tma_kernel, dim3(grid), dim3(kTile), st, env->dev, env->pl, (const float4*)actions, obs, rew,
                        reset, progress, timeout, ep_ret, full_tiles, states_map(env), (const float*)env->scn))
             return check_cuda(cudaGetLastError(), "quad_step_tma_kernel");
         if (tail)
@@ -904,7 +880,7 @@ static int launch_step_t(ozl_env* env, const float* actions, const float* target
                                              (volatile unsigned int*)nullptr, 0u, states_map(env), (const float*)env->scn);
         return check_cuda(cudaGetLastError(), "quad_step_kernel(tail)");
     }
-    if (launch_pdl(env, kernel, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev,
+    if (launch_pdl(kernel, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev,
                    env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, target_in, act_mode, done_u8, reset_mirror,
                    obs_bulk, (int64_t)0, FrontArgs{}, (volatile unsigned int*)(host_flag ? env->host_done : nullptr),
                    host_flag ? ++env->host_seq : 0u, states_map(env), (const float*)env->scn))
@@ -942,7 +918,7 @@ static int launch_front_step(ozl_env* env, int front, const float* actions, cons
     const int64_t n = env->cfg.num_envs;
     cudaStream_t st = (cudaStream_t)stream;
 #define OZL_LAUNCH_FRONT(F, S, MODE)                                                                                            \
-    launch_pdl(env, env->scn ? quad_step_scn_kernel<kStepBlock, F, S> : quad_step_kernel<kStepBlock, F, S>, dim3(blocks_for(n, kStepBlock)), \
+    launch_pdl(env->scn ? quad_step_scn_kernel<kStepBlock, F, S> : quad_step_kernel<kStepBlock, F, S>, dim3(blocks_for(n, kStepBlock)), \
                dim3(kStepBlock), st, env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret,          \
                (const float*)nullptr, (int)MODE, (uint8_t*)nullptr, (int64_t*)nullptr, 1, (int64_t)0, fa,                           \
                (volatile unsigned int*)nullptr, 0u, states_map(env), (const float*)env->scn)
@@ -984,13 +960,13 @@ static int step_host_impl(ozl_env* env, const float* actions_host, float* obs_ho
     if (!done_host) return set_error("ozl_step_host: done_host is NULL");
     // host-mapped (pinned, UVA) buffers: plain coalesced stores over PCIe instead of the TMA bulk store (measured equal)
     return launch_step(env, actions_host, nullptr, ACT_ROTORS, obs_host, rew_host, reset, progress, timeout, ep_ret, stream,
-                       "ozl_step_host", done_host, 0, reset_host, env && env->use_host_flag && env->host_done);
+                       "ozl_step_host", done_host, 0, reset_host, env && env->host_done);
 }
 
-// Wait for the last host step: poll the completion word (see quad_step_kernel); if it does not flip within ~2 s -- or the word is
-// disabled -- synchronise the stream, which also surfaces any CUDA error.
+// Wait for the last host step: poll the completion word (see quad_step_kernel); if it does not flip within ~2 s -- or the handle
+// has no word because cudaHostAlloc failed -- synchronise the stream, which also surfaces any CUDA error.
 static int host_step_wait(ozl_env* env, void* stream) {
-    if (env->use_host_flag && env->host_done) {
+    if (env->host_done) {
         const unsigned int want = env->host_seq;
         for (long spins = 0; spins < 400000000L; ++spins) {
             if (*env->host_done == want) { __atomic_thread_fence(__ATOMIC_ACQUIRE); return 0; }
@@ -1068,19 +1044,8 @@ extern "C" int ozl_set_states_output(ozl_env* env, float* states, int32_t width)
         return 0;
     }
     if ((uintptr_t)states & 15) return set_error("ozl_set_states_output: states must be 16-byte aligned");
-    typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                 const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                 CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    static EncodeFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-            cudaGetLastError();
-            return set_error("ozl_set_states_output: cuTensorMapEncodeTiled is not available from the driver");
-        }
-        fn = (EncodeFn)p;
-    }
+    const PFN_cuTensorMapEncodeTiled fn = tensor_map_encoder();
+    if (!fn) return set_error("ozl_set_states_output: cuTensorMapEncodeTiled is not available from the driver");
     // [N][32] f32 rows of 128 bytes; box = one 128-env tile, 128-byte swizzle (stage_states_row writes the tile in that layout)
     const cuuint64_t gdim[2] = {(cuuint64_t)OZL_STATES_WIDTH, (cuuint64_t)env->cfg.num_envs};
     const cuuint64_t gstr[1] = {(cuuint64_t)OZL_STATES_WIDTH * sizeof(float)};
@@ -1205,7 +1170,7 @@ extern "C" int ozl_set_step_count(ozl_env* env, uint64_t value, void* stream) {
 extern "C" int ozl_metrics_read(ozl_env* env, double* out16, int32_t clear, void* stream) {
     OZL_ENV_CHECK("ozl_metrics_read");
     if (!out16) return set_error("ozl_metrics_read: out16 is NULL");
-    if (launch_pdl(env, metrics_read_kernel, dim3(1), dim3(16 * 32), st, env->pl, out16, (int)clear))
+    if (launch_pdl(metrics_read_kernel, dim3(1), dim3(16 * 32), st, env->pl, out16, (int)clear))
         return check_cuda(cudaGetLastError(), "metrics_read_kernel");
     return 0;
 }
