@@ -275,6 +275,7 @@ int ozl_set_step_count(ozl_env* env, uint64_t value, void* stream);
  *  [0] sum reward  [1] sum episode return of finished episodes  [2] episodes that ended after a landing  [3..7] reserved
  *  [8] env-steps  [9] finished episodes  [10] sum of finished episode lengths  [11] time-outs
  *  [12] dist>die_dist  [13] z<die_z  [14] env-steps with an active rotor fault  [15] resets applied
+ * Every step path fills every slot the same way: ozl_rollout(K) adds what K single steps add, landed episodes included.
  * Replaces RecordEpisodeStatisticsTorch + the trainer's Python scan (RPO-LSTM/utils.py:20-35, main.py:105-113). */
 int ozl_metrics_read(ozl_env* env, double* out16, int32_t clear, void* stream);
 

@@ -415,7 +415,7 @@ quad_rollout_kernel(const DevCfg c, const Planes pl, int K, float* __restrict__ 
         }
         if (k + 1 < K && c.collect_metrics) {
             // metrics for the intermediate steps (the last step goes through block_epilogue)
-            // -- same reduction, without the ticket
+            // -- same slots, landed episodes included, without the ticket
             const int lane = threadIdx.x & 31;
             const bool done = valid && o.reset;
             const double srew = warp_sum(valid ? (double)o.rew : 0.0);
@@ -427,10 +427,12 @@ quad_rollout_kernel(const DevCfg c, const Planes pl, int K, float* __restrict__ 
                                 __popc(__ballot_sync(0xffffffffu, valid && o.crash_z)),
                                 __popc(__ballot_sync(0xffffffffu, valid && o.fault_active))};
             const int n_rs = __popc(__ballot_sync(0xffffffffu, valid && o.did_reset));
+            const int n_ld = __popc(__ballot_sync(0xffffffffu, valid && o.landed_episode));
             if (lane == 0) {
                 double* m = pl.metrics + (blockIdx.x % kMetricSlots) * kMetricStride;
                 if (srew != 0.0) atomicAdd(m + 0, srew);
                 if (sret != 0.0) atomicAdd(m + 1, sret);
+                if (n_ld) atomicAdd(m + 2, (double)n_ld);
 #pragma unroll
                 for (int j = 0; j < 7; ++j)
                     if (cnt[j]) atomicAdd(m + 8 + j, (double)cnt[j]);
