@@ -1,7 +1,9 @@
 // Batched estimators, one env per thread (kernels K2 and K3): attitude-EKF state in registers, PV covariance in shared memory.
-//   K3  9-state position/velocity/accel-bias Kalman filter   CPU twin: oracle/pv_filter.py
+//   K3  9-state position/velocity/accel-bias Kalman filter   CPU twin: oracle/pv_filter.py, exact twin: tests/filters_ref.c
 //       reference: isaacgymenvs/PVFilter.py:25-64 (prediction_step), :67-110 (correction_step), :113-142
-//   K2  4-state attitude EKF, float64                          CPU twin: oracle/ahrs_ekf.py
+//   K2  4-state attitude EKF, float64                          CPU twin: oracle/ahrs_ekf.py, exact twin: tests/filters_ref.c
+// The exact twin restates these functions operation for operation in C; the kernels must equal it bit for bit (any change here
+// changes it too).
 //       reference: isaacgymenvs/ahrs_ekf.py:1072-1158, 1280-1337 (the `ang` branch)
 // The reference runs both as Python loops over envs (tasks/ekf_lee_landed.py:378-391, 417-444: N iterations of ~15 numpy
 // calls / ~40 tiny CUDA launches per step).  Here one launch handles all envs; HBM traffic is the filter state once in,
