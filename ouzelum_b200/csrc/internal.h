@@ -52,6 +52,7 @@ struct ozl_env {
     int device;
     int sm_count;
     long long tma_min_tiles;    // >= this many whole tiles: use the persistent TMA-pipelined step kernel
+    long long early_draw_max_envs;  // <= this many envs: the generic step launches run quad_step_subwave_kernel
     void* arena;                // single cudaMalloc backing all planes
     size_t arena_bytes;
     // host-consumer steps: completion word in pinned host memory, written by the last block of a step kernel after all its

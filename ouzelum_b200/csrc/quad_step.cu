@@ -70,6 +70,8 @@ __device__ __forceinline__ void stage_states_row(float* tile, int r, const float
 // STATES: also write the privileged critic state (ozl_set_states_output) through `states_map`; the STATES = false instantiations
 // are the kernels without that output.  SCN: lay the scenario table `scn` (ozl_set_scenarios) over the reset draws; the body
 // is instantiated by two kernels, quad_step_kernel (no table, `scn` unused) and quad_step_scn_kernel.
+// EARLY: the prologue of quad_step_subwave_kernel (below): branch-free loads, nothing loaded is read before the barrier, and
+// every env draws the reset-path Philox numbers (ResetDraws) between the barrier and the first use of its state.
 #define OZL_STEP_PARAMS                                                                                                         \
     const DevCfg c, const Planes pl, const float4* __restrict__ actions, float* __restrict__ obs, float* __restrict__ rew,       \
         int64_t* __restrict__ reset, int64_t* __restrict__ progress, uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, \
@@ -77,7 +79,7 @@ __device__ __forceinline__ void stage_states_row(float* tile, int r, const float
         const int obs_bulk, const int64_t env0, const FrontArgs fa, volatile unsigned int* host_done, const unsigned int host_seq
 #define OZL_STEP_ARGS c, pl, actions, obs, rew, reset, progress, timeout, ep_ret_out, target_in, act_mode, done_u8, reset_mirror, \
                       obs_bulk, env0, fa, host_done, host_seq, states_map, scn
-template <int BLOCK, int FRONT, bool STATES, bool SCN>
+template <int BLOCK, int FRONT, bool STATES, bool SCN, bool EARLY = false>
 __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMap& states_map, const float* __restrict__ scn) {
     __shared__ __align__(16) float s_obs[BLOCK * 13];
     __shared__ __align__(1024) float s_states[STATES ? BLOCK * OZL_STATES_WIDTH : 4];
@@ -99,7 +101,16 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
     float4 a4 = make_float4(0.f, 0.f, 0.f, 0.f);
     int64_t prog = 0;
     bool rst = false;
-    if (valid) {
+    int64_t rst_word = 0;
+    if constexpr (EARLY) {
+        // no branch around the loads (lanes past num_envs load the last env and never use it): the block barrier then waits
+        // for the leader's step record only, not for this thread's loads
+        const int64_t li = valid ? i : c.num_envs - 1;
+        load_env(pl, li, L);
+        if (FRONT != FRONT_LEE) a4 = __ldg(actions + li);
+        prog = progress[li];
+        rst_word = reset[li];
+    } else if (valid) {
         load_env(pl, i, L);
         if (FRONT != FRONT_LEE) a4 = __ldg(actions + i);
         prog = progress[i];
@@ -107,6 +118,20 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
     }
     __syncthreads();
     const uint64_t step = s_step;
+    ResetDraws pre = {};
+    if constexpr (EARLY) {
+        // the reset-path draws depend on (seed, env, step) only: ~270 instructions issued while the state is still arriving,
+        // and the reset / re-sample paths below become selects instead of divergent branches with ten Philox rounds each
+        const uint32_t genv = c.env_id_base + (uint32_t)i;
+        if (!c.target_fixed) pre.target = draw(c.seed, genv, step, P_TARGET);
+        pre.spawn = draw(c.seed, genv, step, P_SPAWN);
+        if (c.fault_mode) pre.fault = draw(c.seed, genv, step, P_FAULT);
+        // keep them here: left alone, the compiler sinks a draw into the one branch that reads it (the reset path)
+        asm volatile("" : "+r"(pre.target.x), "+r"(pre.target.y), "+r"(pre.target.z), "+r"(pre.spawn.x), "+r"(pre.spawn.y),
+                          "+r"(pre.spawn.z), "+r"(pre.fault.x), "+r"(pre.fault.y), "+r"(pre.fault.z));
+        rst = rst_word != 0;
+    }
+    const ResetDraws* pre_p = EARLY ? &pre : nullptr;
     if (valid) {
         Env e;
         unpack(L, e);
@@ -123,7 +148,7 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
         const uint32_t genv = c.env_id_base + (uint32_t)i;
         const float* scn_row = SCN ? scn + i * OZL_SCENARIO_WIDTH : nullptr;
         if (FRONT == FRONT_LEE) {
-            const int64_t prog1 = env_reset_phase<SCN>(e, prog, rst, genv, step, c, o, scn_row);
+            const int64_t prog1 = env_reset_phase<SCN>(e, prog, rst, genv, step, c, o, scn_row, pre_p);
             const float cmd[4] = {fa.cmd[0] * fa.g.scale[0], fa.cmd[1] * fa.g.scale[1], fa.cmd[2] * fa.g.scale[2], fa.cmd[3] * fa.g.scale[3]};
             float th, tq[3];
             lee_control(LEE_POSITION, e.p, e.q, e.v, e.w, cmd, fa.g, th, tq);                  // lee_landed.py:311
@@ -131,7 +156,7 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
             if (fa.wrench_out) fa.wrench_out[i] = make_float4(act[0], act[1], act[2], act[3]);
             env_act_phase(e, act, prog1, rst, genv, step, c, o, ACT_WRENCH, tptr, fa.cmd);       // detector on the controller target, :305,318-322
         } else {
-            env_step<SCN>(e, act, prog, rst, genv, step, c, o, act_mode, tptr, scn_row);
+            env_step<SCN>(e, act, prog, rst, genv, step, c, o, act_mode, tptr, scn_row, pre_p);
         }
         if constexpr (STATES) stage_states_row(s_states, threadIdx.x, o.obs, e, o, c);
         obs_epilogue(o.obs, genv, step, flicker_blackout(step, c), c);
@@ -204,6 +229,16 @@ template <int BLOCK, int FRONT, bool STATES>
 __global__ void __launch_bounds__(BLOCK, kStepMinBlocks)
 quad_step_scn_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
     quad_step_body<BLOCK, FRONT, STATES, true>(OZL_STEP_ARGS);
+}
+// Launches smaller than one wave of the kernels above (up to 4 CTAs per SM, ozl_env::early_draw_max_envs) are bound by the
+// latency of their slowest warp, not by issue or bandwidth.  This twin fills the warp's wait for its state with the reset-path
+// draws of every env (EARLY) and drops the 72-register cap: it needs 105-126 registers, which leaves room for 4 CTAs per SM.
+// Same results bit for bit.  Larger launches keep the kernels above: there the draws would be issued for every env instead of
+// for the ~2 % that reset, on a launch with 7 warps per scheduler that is issue-bound, and 4 CTAs per SM would need two waves.
+template <int BLOCK, int FRONT, bool STATES, bool SCN>
+__global__ void __launch_bounds__(BLOCK, 1)
+quad_step_subwave_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
+    quad_step_body<BLOCK, FRONT, STATES, SCN, true>(OZL_STEP_ARGS);
 }
 
 // ------------------------------------------------------------------------------------------------ K1, TMA-pipelined
@@ -787,6 +822,15 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
         const char* ev = getenv("OZL_TMA_MIN_TILES");
         e->tma_min_tiles = ev ? atoll(ev) : (long long)kStepMinBlocks * prop.multiProcessorCount + 1;
     }
+    {   // up to one wave of quad_step_subwave_kernel (4 x 128-env CTAs per SM: 75776 envs on 148 SMs) the generic launch runs it.
+        // Measured on B200 at 1000 W (us per step, default kernel -> sub-wave kernel, cold / warm L2; DESIGN.md section 6):
+        //   16384 envs  4.16-4.48 -> 3.85-4.06 / 3.76 -> 3.55      65536 envs  6.94-7.17 -> 6.24-6.35 / 5.34 -> 5.09
+        //   75776 envs  9.47-9.71 -> 6.65-6.70 / 7.66-7.79 -> 5.24     81920 envs (two waves of it)  9.58-9.84 -> 9.51-9.60 / 7.56-7.60 -> 8.38-8.40
+        //   131072 envs (two waves of it)  10.79-10.93 -> 11.31-11.37 / 7.81 -> 9.52
+        // (override: OZL_EARLY_DRAW_MAX_ENVS, 0 = never)
+        const char* ev = getenv("OZL_EARLY_DRAW_MAX_ENVS");
+        e->early_draw_max_envs = ev ? atoll(ev) : 4ll * kTile * prop.multiProcessorCount;
+    }
     const size_t n = (size_t)cfg->num_envs;
     const size_t tiles = (n + kTile - 1) / kTile;
     const size_t state = align_up(tiles * (size_t)kTileBytes, 256);
@@ -868,6 +912,7 @@ static int launch_step_t(ozl_env* env, const float* actions, const float* target
     const bool plain = (target_in == nullptr) && act_mode == ACT_ROTORS && done_u8 == nullptr && reset_mirror == nullptr && obs_bulk;
     const auto tma_kernel = SCN ? quad_step_tma_scn_kernel<STATES> : quad_step_tma_kernel<STATES>;
     const auto kernel = SCN ? quad_step_scn_kernel<kStepBlock, FRONT_NONE, STATES> : quad_step_kernel<kStepBlock, FRONT_NONE, STATES>;
+    const auto step_kernel = n <= env->early_draw_max_envs ? quad_step_subwave_kernel<kStepBlock, FRONT_NONE, STATES, SCN> : kernel;
     if (plain && env->tma_min_tiles > 0 && full_tiles >= env->tma_min_tiles &&
         !(((uintptr_t)progress | (uintptr_t)reset) & 15)) {
         // large N: persistent TMA-pipelined kernel over the whole tiles, then one generic block for the ragged tail
@@ -882,7 +927,7 @@ static int launch_step_t(ozl_env* env, const float* actions, const float* target
                                              (volatile unsigned int*)nullptr, 0u, states_map(env), (const float*)env->scn);
         return check_cuda(cudaGetLastError(), "quad_step_kernel(tail)");
     }
-    if (launch_pdl(kernel, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev,
+    if (launch_pdl(step_kernel, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev,
                    env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, target_in, act_mode, done_u8, reset_mirror,
                    obs_bulk, (int64_t)0, FrontArgs{}, (volatile unsigned int*)(host_flag ? env->host_done : nullptr),
                    host_flag ? ++env->host_seq : 0u, states_map(env), (const float*)env->scn))
@@ -918,10 +963,12 @@ static int launch_front_step(ozl_env* env, int front, const float* actions, cons
     fa.h.reset = reset;
     fa.h.step_ptr = env->pl.ctrl;            // the vehicle follows the handle's device step counter (graph-capturable)
     const int64_t n = env->cfg.num_envs;
+    const bool subwave = n <= env->early_draw_max_envs;
     cudaStream_t st = (cudaStream_t)stream;
 #define OZL_LAUNCH_FRONT(F, S, MODE)                                                                                            \
-    launch_pdl(env->scn ? quad_step_scn_kernel<kStepBlock, F, S> : quad_step_kernel<kStepBlock, F, S>, dim3(blocks_for(n, kStepBlock)), \
-               dim3(kStepBlock), st, env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret,          \
+    launch_pdl(subwave ? (env->scn ? quad_step_subwave_kernel<kStepBlock, F, S, true> : quad_step_subwave_kernel<kStepBlock, F, S, false>) \
+                       : (env->scn ? quad_step_scn_kernel<kStepBlock, F, S> : quad_step_kernel<kStepBlock, F, S>),                   \
+               dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret,          \
                (const float*)nullptr, (int)MODE, (uint8_t*)nullptr, (int64_t*)nullptr, 1, (int64_t)0, fa,                           \
                (volatile unsigned int*)nullptr, 0u, states_map(env), (const float*)env->scn)
     int rc;
