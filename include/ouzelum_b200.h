@@ -26,11 +26,14 @@
 extern "C" {
 #endif
 
-#define OZL_ABI_VERSION 6   /* 3: ozl_cfg.dr[] (domain-randomisation schema), per-env yaw_km (params8), wrench_warmup_steps,
+#define OZL_ABI_VERSION 7   /* 3: ozl_cfg.dr[] (domain-randomisation schema), per-env yaw_km (params8), wrench_warmup_steps,
                                ozl_ekf_lee_args.num_envs_total, i64 reset mirror in ozl_host_io
                                4: (additive) ozl_metrics_xchg_* / ozl_metrics_push / ozl_metrics_sum, ozl_noise_lambda_apply
                                5: (additive) ozl_set_states_output, OZL_STATE_* layout of the privileged critic state
-                               6: (additive) ozl_set_scenarios, OZL_SCN_* layout of a scenario row */
+                               6: (additive) ozl_set_scenarios, OZL_SCN_* layout of a scenario row
+                               7: (additive) fault_mode 2 (multi-rotor and gradual rotor faults): ozl_cfg.fault_rotors_lo / _hi /
+                                  fault_ramp_steps in the former reserved0 / reserved1 (same size), ozl_get_rotor_eff /
+                                  ozl_set_rotor_eff, scenario group OZL_SCN_RFAULT_* */
 
 /* sensor-fault model of isaacgymenvs/utils/POMDP.py:4-42 */
 enum { OZL_POMDP_NONE = 0, OZL_POMDP_FLICKER = 1, OZL_POMDP_NOISE = 2, OZL_POMDP_FLICKER_NOISE = 3 };
@@ -62,7 +65,8 @@ typedef struct ozl_dr_param {
  * reference counterpart (SURVEY.md section 8a row P). */
 typedef struct ozl_cfg {
     int32_t abi_version;          /* must be OZL_ABI_VERSION */
-    int32_t reserved0;
+    int16_t fault_rotors_lo;      /* fault_mode 2: number of faulted rotors drawn in [lo, hi], 0 <= lo <= hi <= 4 (default 1, 1);  */
+    int16_t fault_rotors_hi;      /* these two and fault_ramp_steps sit in what were reserved words, so sizeof(ozl_cfg) is unchanged */
     int64_t num_envs;             /* envs simulated by THIS handle (the local shard)            cfg env.numEnvs */
     int64_t env_id_base;          /* global id of local env 0: RNG is keyed by global id, so results do not depend on the sharding */
     uint64_t seed;
@@ -90,7 +94,8 @@ typedef struct ozl_cfg {
     /* extras (no reference counterpart; 0 => reference behaviour) */
     float lin_drag;               /* F = -k v (world)                                                             */
     float yaw_km;                 /* rotor reaction torque about body z per newton of thrust                      */
-    int32_t fault_mode;           /* 1: single-rotor loss of effectiveness, schedule drawn at reset               */
+    int32_t fault_mode;           /* 1: single-rotor loss of effectiveness, schedule drawn at reset
+                                     2: multi-rotor and gradual loss of effectiveness (see "Rotor faults, mode 2" below) */
     float fault_eff_lo, fault_eff_range;
     int32_t dr_enable;            /* 1: randomise the per-env parameters at reset according to dr[]               */
     ozl_dr_param dr[7];           /* indexed by OZL_DR_*; default: mass/Ixx/Iyy/Izz/arm/thrust-scale = scaling x uniform
@@ -107,8 +112,25 @@ typedef struct ozl_cfg {
     int32_t wrench_warmup_steps;  /* wrench-actuated steps with step counter < this value are the estimator warm-up of
                                      tasks/ekf_lee_landed.py:339,508-529: the wrench reaches EVERY env (no near-target cut, no
                                      zeroing for just-reset envs) and the landing flag is not raised.  0 = no warm-up      */
-    int32_t reserved1;
+    int32_t fault_ramp_steps;     /* fault_mode 2: steps over which the loss ramps in, 0 <= ramp < 2^24 (0 or 1: abrupt; default 0) */
 } ozl_cfg;
+
+/* Rotor faults, mode 2 (cfg.fault_mode = 2, "multi").  At every reset of env i, with Philox words keyed by (seed, global env id,
+ * step, purpose) like every other draw -- r0..r2 of the P_FAULT draw that mode 1 uses, w0..w3 of one more draw (P_RFAULT) --
+ *   k      = fault_rotors_lo + umulhi(r2, fault_rotors_hi - fault_rotors_lo + 1)          number of faulted rotors
+ *   rotors = the first k entries of permutation umulhi(r0, 24) of {0,1,2,3}, the 24 in lexicographic order
+ *   e_j    = fault_eff_lo + fault_eff_range * u01(w_j) for a faulted rotor j, 1.0f for a healthy one
+ *   onset  = umulhi(r1, max_episode_length) (mode 1's onset), or never (0x1FFFFFFF) when k = 0
+ * At progress p >= onset (progress after the reset phase of the step), with d = p - onset, rotor j's force is multiplied by
+ *   a_j = e_j                                                    if fault_ramp_steps <= 1 or d + 1 >= fault_ramp_steps
+ *   a_j = fmaf((float)(d + 1) * inv_ramp, e_j - 1.0f, 1.0f)      otherwise, inv_ramp = (float)(1.0 / fault_ramp_steps)
+ * (a healthy rotor gets exactly 1).  The fault is active (metrics slot 14) while p >= onset; OZL_STATE_EFF .. +3 report a_j (1 on
+ * wrench-actuated steps, where no fault is applied).  e_0..e_3 live in a per-env plane of the handle (ozl_get_rotor_eff /
+ * ozl_set_rotor_eff), the onset in the fault word (ozl_get_params fault2[:, 1]; the rotor id and the params8 effectiveness are
+ * unused).  Mode 2 applies on ozl_step, ozl_step_tracking, ozl_step_wrench, ozl_step_host*, ozl_landing_step,
+ * ozl_apply_resets and the initial state (no fault); ozl_rollout, ozl_lee_landed_step and ozl_ekf_lee_landed_step refuse to run.
+ * ozl_create checks 0 <= lo <= hi <= 4, 0 <= fault_ramp_steps < 2^24, fault_eff_lo in [0, 1] and fault_eff_lo + fault_eff_range
+ * in [fault_eff_lo, 1]. */
 
 typedef struct ozl_env ozl_env;   /* opaque */
 
@@ -225,7 +247,9 @@ int ozl_set_states_output(ozl_env* env, float* states, int32_t width);
  *                              in [0, 2^24)), effectiveness in [0, 1]                        group "fault"
  *   OZL_SCN_MASS .. _YAW_KM    mass, ixx, iyy, izz, arm, thrust_scale, yaw_km (absolute values, as params8 of ozl_set_params),
  *                              one group each
- *   OZL_SCN_RESERVED .. 31     must be NaN
+ *   OZL_SCN_RFAULT_ONSET, OZL_SCN_RFAULT_EFF .. +3   fault_mode 2 only: onset (an integer in [0, 2^24)) and e_0..e_3, each in
+ *                              [0, 1]; four 1s mean no fault in that episode                 group "rotor faults"
+ *   OZL_SCN_RESERVED .. 31     must be NaN (under fault_mode 2: slot 31 only, slots 26-30 are the rotor-faults group)
  * Slots 0-12 are laid out as root13 of ozl_set_state.  A group is either all NaN -- the env gets exactly what it gets without a
  * table: the draw, identity / zero for attitude and velocities, an unchanged value for a body parameter that is not randomised --
  * or all set, and then its values are used at every reset of the env.  An all-NaN table therefore gives results bit-identical to
@@ -236,13 +260,15 @@ int ozl_set_states_output(ozl_env* env, float* states, int32_t width);
  * ozl_lee_landed_step and ozl_apply_resets; the landed flag and the episode bookkeeping are unchanged. */
 enum { OZL_SCN_POS = 0, OZL_SCN_QUAT = 3, OZL_SCN_LINVEL = 7, OZL_SCN_ANGVEL = 10, OZL_SCN_TARGET = 13, OZL_SCN_FAULT_ROTOR = 16,
        OZL_SCN_FAULT_ONSET = 17, OZL_SCN_FAULT_EFF = 18, OZL_SCN_MASS = 19, OZL_SCN_IXX = 20, OZL_SCN_IYY = 21, OZL_SCN_IZZ = 22,
-       OZL_SCN_ARM = 23, OZL_SCN_THRUST_SCALE = 24, OZL_SCN_YAW_KM = 25, OZL_SCN_RESERVED = 26, OZL_SCENARIO_WIDTH = 32 };
+       OZL_SCN_ARM = 23, OZL_SCN_THRUST_SCALE = 24, OZL_SCN_YAW_KM = 25, OZL_SCN_RESERVED = 26, OZL_SCN_RFAULT_ONSET = 26,
+       OZL_SCN_RFAULT_EFF = 27, OZL_SCENARIO_WIDTH = 32 };
 
 /* Register the scenario table: `rows_host` is HOST memory, [N, OZL_SCENARIO_WIDTH] f32; `width` must be OZL_SCENARIO_WIDTH.
  * Every row is validated first and nothing is registered if one fails: reserved slots NaN; each group all NaN or all finite;
  * |x^2 + y^2 + z^2 + w^2 - 1| <= 1e-6 for the quaternion (the integrator keeps a unit quaternion unit with one Newton step and
  * needs a unit input); no target group when cfg.target_fixed is set (the target is driven by a vehicle or the caller); no fault
- * group unless cfg.fault_mode is set; rotor in {-1, 0, 1, 2, 3}, onset an integer in [0, 2^24), effectiveness in [0, 1]; mass
+ * group unless cfg.fault_mode is 1 (under mode 2 the rotor-faults group instead, with the rules above); rotor in {-1, 0, 1, 2, 3},
+ * onset an integer in [0, 2^24), effectiveness in [0, 1]; mass
  * and inertias in (1e-30, 1e30) (the step's reciprocals need positive normal floats), arm > 0, thrust_scale >= 0, yaw_km finite.
  * The rows are copied (stream-ordered on `stream`, which is then synchronised) into a device buffer the handle allocates on the
  * first registration and frees in ozl_destroy.  A later call overwrites the contents at the same address, so a CUDA graph
@@ -266,6 +292,10 @@ int ozl_set_state(ozl_env* env, const float* root13, const float* thrust4, const
  * Mass and inertia must be positive normal floats (the step evaluates their IEEE reciprocals on a range-checked fast path). */
 int ozl_get_params(ozl_env* env, float* params8, int32_t* fault2, void* stream);
 int ozl_set_params(ozl_env* env, const float* params8, const int32_t* fault2, void* stream);
+/* fault_mode 2: the per-rotor effectiveness e_0..e_3 of every env's current episode, eff4 [N,4] f32 device buffers (16-byte
+ * aligned).  Stream-ordered copies, CUDA-graph capturable.  Non-zero return unless cfg.fault_mode == 2. */
+int ozl_get_rotor_eff(ozl_env* env, float* eff4, void* stream);
+int ozl_set_rotor_eff(ozl_env* env, const float* eff4, void* stream);
 
 /* Step counter (the RNG's time axis): number of ozl_step's since ozl_reset_all.  Host-synchronising. */
 int ozl_get_step_count(ozl_env* env, uint64_t* out, void* stream);

@@ -9,7 +9,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("OUZELUM_B200_LIB") or os.path.join(_HERE, "libouzelum_b200.so")   # override: kernel experiments only
 
-OZL_ABI_VERSION = 6
+OZL_ABI_VERSION = 7
 
 
 def _header_enum(prefix):
@@ -46,7 +46,7 @@ class OzlDrParam(C.Structure):
 class OzlCfg(C.Structure):
     """Mirror of `struct ozl_cfg` (include/ouzelum_b200.h)."""
     _fields_ = [
-        ("abi_version", C.c_int32), ("reserved0", C.c_int32),
+        ("abi_version", C.c_int32), ("fault_rotors_lo", C.c_int16), ("fault_rotors_hi", C.c_int16),
         ("num_envs", C.c_int64), ("env_id_base", C.c_int64), ("seed", C.c_uint64),
         ("max_episode_length", C.c_int32), ("target_period", C.c_int32), ("target_fixed", C.c_int32),
         ("substeps", C.c_int32), ("control_freq_inv", C.c_int32),
@@ -62,13 +62,15 @@ class OzlCfg(C.Structure):
         ("dr_enable", C.c_int32), ("dr", OzlDrParam * 7),
         ("pomdp_mode", C.c_int32), ("pomdp_prob", C.c_float), ("noise_sigma", C.c_float),
         ("collect_metrics", C.c_int32), ("plate_enable", C.c_int32), ("plate_z", C.c_float), ("plate_radius", C.c_float), ("land_cutoff", C.c_float),
-        ("wrench_warmup_steps", C.c_int32), ("reserved1", C.c_int32),
+        ("wrench_warmup_steps", C.c_int32), ("fault_ramp_steps", C.c_int32),
     ]
+
+    _MULTI_FAULT = ("fault_rotors_lo", "fault_rotors_hi", "fault_ramp_steps")    # meaningful under fault_mode 2 only
 
     def to_dict(self):
         out = {}
         for name, typ in self._fields_:
-            if name.startswith("reserved") or name == "abi_version":
+            if name.startswith("reserved") or name == "abi_version" or (name in self._MULTI_FAULT and self.fault_mode != 2):
                 continue
             v = getattr(self, name)
             if name == "dr":
@@ -186,6 +188,8 @@ _SIGS = {
     "ozl_set_state": (C.c_int, [_P] * 6),
     "ozl_get_params": (C.c_int, [_P] * 4),
     "ozl_set_params": (C.c_int, [_P] * 4),
+    "ozl_get_rotor_eff": (C.c_int, [_P] * 3),
+    "ozl_set_rotor_eff": (C.c_int, [_P] * 3),
     "ozl_get_step_count": (C.c_int, [_P, C.POINTER(C.c_uint64), _P]),
     "ozl_set_step_count": (C.c_int, [_P, C.c_uint64, _P]),
     "ozl_metrics_read": (C.c_int, [_P, _P, C.c_int32, _P]),

@@ -11,7 +11,8 @@ import copy
 _SIM = {"dt": 0.01, "substeps": 2, "up_axis": "z", "use_gpu_pipeline": True, "gravity": [0.0, 0.0, -9.81]}
 
 _EXTRAS = {
-    "rotorFault": {"enable": False, "effLow": 0.0, "effHigh": 0.5},
+    # mode "multi": rotors [lo, hi] faulted rotors per episode, the loss ramping in over rampSteps steps (include/ouzelum_b200.h)
+    "rotorFault": {"enable": False, "mode": "single", "rotors": [1, 1], "effLow": 0.0, "effHigh": 0.5, "rampSteps": 0},
     "domainRandomization": {"enable": False, "low": 0.8, "high": 1.2},
     "linDrag": 0.0, "yawKm": 0.0,
     "POMDP": "none", "pomdp_prob": 0.0,

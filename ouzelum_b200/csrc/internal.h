@@ -52,6 +52,7 @@ struct ozl_env {
     int device;
     int sm_count;
     long long tma_min_tiles;    // >= this many whole tiles: use the persistent TMA-pipelined step kernel
+    long long tma_min_tiles_mf; // the same for the fault_mode 2 twins (the generic twin is resident 6 CTAs per SM, not 7)
     long long early_draw_max_envs;  // <= this many envs: the generic step launches run quad_step_subwave_kernel
     void* arena;                // single cudaMalloc backing all planes
     size_t arena_bytes;
@@ -75,6 +76,9 @@ struct ozl_env {
     // registered and NULL otherwise -- the step launches pick the kernels that read it by this pointer
     float* scn_buf;
     float* scn;
+    // fault_mode 2: the constants and the e_0..e_3 plane (MfCfg::eff4, in the arena) that the fault_mode 2 kernels take as
+    // their last argument; eff4 is NULL for the other modes
+    ozl::MfCfg mf;
 };
 
 // Step launches go through cudaLaunchKernelEx so that they can carry the programmatic-stream-serialization attribute (PDL):

@@ -8,13 +8,14 @@ namespace ozl {
 enum : uint32_t {
     P_TARGET = 0,    // r0,r1 -> target x,y ; r2 -> target z
     P_SPAWN = 1,     // r0,r1,r2 -> spawn offsets
-    P_FAULT = 2,     // r0 -> rotor ; r1 -> onset ; r2 -> effectiveness
+    P_FAULT = 2,     // r0 -> rotor ; r1 -> onset ; r2 -> effectiveness  (fault_mode 2: r0 -> permutation ; r1 -> onset ; r2 -> count)
     P_DR0 = 3,       // mass, Ixx, Iyy, Izz
     P_DR1 = 4,       // arm, thrust-scale, yaw_km
     P_DR2 = 24,      // second uniforms of gaussian draws (mass, Ixx, Iyy, Izz)
     P_DR3 = 25,      //                                   (arm, thrust-scale, yaw_km)
     P_QDOF0 = 5,     // Quadcopter task: initial DOF positions 0..3
     P_QDOF1 = 6,     //                  initial DOF positions 4..7
+    P_RFAULT = 7,    // fault_mode 2: w0..w3 -> effectiveness of rotors 0..3
     P_OBSNOISE = 8,  // +0..+3: 13 sensor-noise uniforms
     P_FLICKER = 12,  // global blackout draw (env word = GLOBAL_ENV)
     P_ACTION = 16,   // synthetic roll-out actions

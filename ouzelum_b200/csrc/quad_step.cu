@@ -66,12 +66,33 @@ __device__ __forceinline__ void stage_states_row(float* tile, int r, const float
 #pragma unroll
     for (int k = 0; k < OZL_STATES_WIDTH / 4; ++k) row[k ^ (r & 7)] = make_float4(s[4 * k], s[4 * k + 1], s[4 * k + 2], s[4 * k + 3]);
 }
+// fault_mode 2: the same row, then its EFF slots overwritten with the factors a_j applied this step (clamped like every slot; all 1
+// on a wrench-actuated step).  They are recomputed from e (re-read, see RotorEff) and the post-reset progress o.prog - 1 once the
+// row is out of registers, rather than kept live across the integrator.
+__device__ __forceinline__ void stage_states_row_mf(float* tile, int r, const float clean[13], const Env& e, const StepOut& o,
+                                                    const DevCfg& c, const RotorEff& rf, bool rotors) {
+    stage_states_row(tile, r, clean, e, o, c);
+    float a[4] = {1.0f, 1.0f, 1.0f, 1.0f};
+    if (rotors) {
+        RotorEff rr = rf;
+        rfault_load(rr);
+        rfault_factors(e, rr, o.prog - 1, a);
+    }
+    static_assert(OZL_STATE_EFF == 17, "EFF slots 17..20: elements 1..3 of 16-byte chunk 4 and element 0 of chunk 5");
+    float* row = tile + r * OZL_STATES_WIDTH;
+    row[4 * (4 ^ (r & 7)) + 1] = fminf(fmaxf(a[0], -c.clip_obs), c.clip_obs);
+    row[4 * (4 ^ (r & 7)) + 2] = fminf(fmaxf(a[1], -c.clip_obs), c.clip_obs);
+    row[4 * (4 ^ (r & 7)) + 3] = fminf(fmaxf(a[2], -c.clip_obs), c.clip_obs);
+    row[4 * (5 ^ (r & 7))] = fminf(fmaxf(a[3], -c.clip_obs), c.clip_obs);
+}
 
 // STATES: also write the privileged critic state (ozl_set_states_output) through `states_map`; the STATES = false instantiations
 // are the kernels without that output.  SCN: lay the scenario table `scn` (ozl_set_scenarios) over the reset draws; the body
 // is instantiated by two kernels, quad_step_kernel (no table, `scn` unused) and quad_step_scn_kernel.
 // EARLY: the prologue of quad_step_subwave_kernel (below): branch-free loads, nothing loaded is read before the barrier, and
 // every env draws the reset-path Philox numbers (ResetDraws) between the barrier and the first use of its state.
+// MF: fault_mode 2 (quad_step_mf_kernel / quad_step_mf_subwave_kernel): the env's lane of mf.eff4 (MfCfg, their last argument)
+// is read with its state and written back on a reset; the scenario row is read through `scn` when it is not NULL (SCN is true).
 #define OZL_STEP_PARAMS                                                                                                         \
     const DevCfg c, const Planes pl, const float4* __restrict__ actions, float* __restrict__ obs, float* __restrict__ rew,       \
         int64_t* __restrict__ reset, int64_t* __restrict__ progress, uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, \
@@ -79,8 +100,9 @@ __device__ __forceinline__ void stage_states_row(float* tile, int r, const float
         const int obs_bulk, const int64_t env0, const FrontArgs fa, volatile unsigned int* host_done, const unsigned int host_seq
 #define OZL_STEP_ARGS c, pl, actions, obs, rew, reset, progress, timeout, ep_ret_out, target_in, act_mode, done_u8, reset_mirror, \
                       obs_bulk, env0, fa, host_done, host_seq, states_map, scn
-template <int BLOCK, int FRONT, bool STATES, bool SCN, bool EARLY = false>
-__device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMap& states_map, const float* __restrict__ scn) {
+template <int BLOCK, int FRONT, bool STATES, bool SCN, bool EARLY = false, bool MF = false>
+__device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMap& states_map, const float* __restrict__ scn,
+                                               const MfCfg& mf = MfCfg{}) {
     __shared__ __align__(16) float s_obs[BLOCK * 13];
     __shared__ __align__(1024) float s_states[STATES ? BLOCK * OZL_STATES_WIDTH : 4];
     __shared__ uint64_t s_step;
@@ -102,16 +124,19 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
     int64_t prog = 0;
     bool rst = false;
     int64_t rst_word = 0;
+    float4 ef = make_float4(1.f, 1.f, 1.f, 1.f);
     if constexpr (EARLY) {
         // no branch around the loads (lanes past num_envs load the last env and never use it): the block barrier then waits
         // for the leader's step record only, not for this thread's loads
         const int64_t li = valid ? i : c.num_envs - 1;
         load_env(pl, li, L);
+        if constexpr (MF) ef = mf.eff4[li];
         if (FRONT != FRONT_LEE) a4 = __ldg(actions + li);
         prog = progress[li];
         rst_word = reset[li];
     } else if (valid) {
         load_env(pl, i, L);
+        if constexpr (MF) asm volatile("prefetch.global.L1 [%0];" ::"l"(mf.eff4 + i));   // read where it is used (RotorEff)
         if (FRONT != FRONT_LEE) a4 = __ldg(actions + i);
         prog = progress[i];
         rst = reset[i] != 0;
@@ -129,6 +154,10 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
         // keep them here: left alone, the compiler sinks a draw into the one branch that reads it (the reset path)
         asm volatile("" : "+r"(pre.target.x), "+r"(pre.target.y), "+r"(pre.target.z), "+r"(pre.spawn.x), "+r"(pre.spawn.y),
                           "+r"(pre.spawn.z), "+r"(pre.fault.x), "+r"(pre.fault.y), "+r"(pre.fault.z));
+        if constexpr (MF) {
+            pre.rfault = draw(c.seed, genv, step, P_RFAULT);
+            asm volatile("" : "+r"(pre.rfault.x), "+r"(pre.rfault.y), "+r"(pre.rfault.z), "+r"(pre.rfault.w));
+        }
         rst = rst_word != 0;
     }
     const ResetDraws* pre_p = EARLY ? &pre : nullptr;
@@ -146,23 +175,35 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
         }
         float act[4] = {a4.x, a4.y, a4.z, a4.w};
         const uint32_t genv = c.env_id_base + (uint32_t)i;
-        const float* scn_row = SCN ? scn + i * OZL_SCENARIO_WIDTH : nullptr;
+        const float* scn_row = SCN ? ((MF && !scn) ? nullptr : scn + i * OZL_SCENARIO_WIDTH) : nullptr;
+        RotorEff rf;
+        if constexpr (MF) {
+            rf.e[0] = ef.x; rf.e[1] = ef.y; rf.e[2] = ef.z; rf.e[3] = ef.w;
+            rf.in_mem = !EARLY;
+            rf.i = i;
+            rf.m = &mf;
+        }
+        RotorEff* rf_p = MF ? &rf : nullptr;
         if (FRONT == FRONT_LEE) {
-            const int64_t prog1 = env_reset_phase<SCN>(e, prog, rst, genv, step, c, o, scn_row, pre_p);
+            const int64_t prog1 = env_reset_phase<SCN, MF>(e, prog, rst, genv, step, c, o, scn_row, pre_p, rf_p);
             const float cmd[4] = {fa.cmd[0] * fa.g.scale[0], fa.cmd[1] * fa.g.scale[1], fa.cmd[2] * fa.g.scale[2], fa.cmd[3] * fa.g.scale[3]};
             float th, tq[3];
             lee_control(LEE_POSITION, e.p, e.q, e.v, e.w, cmd, fa.g, th, tq);                  // lee_landed.py:311
             act[0] = fa.mg * th; act[1] = tq[0]; act[2] = tq[1]; act[3] = tq[2];                 // :313-314
             if (fa.wrench_out) fa.wrench_out[i] = make_float4(act[0], act[1], act[2], act[3]);
-            env_act_phase(e, act, prog1, rst, genv, step, c, o, ACT_WRENCH, tptr, fa.cmd);       // detector on the controller target, :305,318-322
+            env_act_phase<MF>(e, act, prog1, rst, genv, step, c, o, ACT_WRENCH, tptr, fa.cmd, rf_p);   // detector on the controller target, :305,318-322
         } else {
-            env_step<SCN>(e, act, prog, rst, genv, step, c, o, act_mode, tptr, scn_row, pre_p);
+            env_step<SCN, MF>(e, act, prog, rst, genv, step, c, o, act_mode, tptr, scn_row, pre_p, rf_p);
         }
-        if constexpr (STATES) stage_states_row(s_states, threadIdx.x, o.obs, e, o, c);
+        if constexpr (STATES && MF) stage_states_row_mf(s_states, threadIdx.x, o.obs, e, o, c, rf, act_mode == ACT_ROTORS);
+        else if constexpr (STATES) stage_states_row(s_states, threadIdx.x, o.obs, e, o, c);
         obs_epilogue(o.obs, genv, step, flicker_blackout(step, c), c);
 
         store_dynamic(pl, i, e);
         if (o.static_dirty || tptr) store_static(pl, i, e);
+        if constexpr (MF) {
+            if (EARLY && o.did_reset) mf.eff4[i] = make_float4(rf.e[0], rf.e[1], rf.e[2], rf.e[3]);
+        }
         rew[i] = o.rew;
         reset[i] = o.reset ? 1 : 0;
         progress[i] = o.prog;
@@ -240,6 +281,24 @@ __global__ void __launch_bounds__(BLOCK, 1)
 quad_step_subwave_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
     quad_step_body<BLOCK, FRONT, STATES, SCN, true>(OZL_STEP_ARGS);
 }
+// fault_mode 2 twins of quad_step_kernel / quad_step_scn_kernel (one kernel for both: `scn` may be NULL) and of
+// quad_step_subwave_kernel, chosen by the launches whenever cfg.fault_mode == 2 (never for FRONT_LEE, which refuses mode 2).
+// The sub-wave twin keeps 4 CTAs per SM, its one-wave limit.
+// The generic twin is bounded to 6 CTAs per SM (85 registers): at 7 (72 registers) ptxas spills 8-48 bytes in every variant however
+// the mode-2 state is held, so mode-2 launches switch to the TMA twin one wave earlier (ozl_env::tma_min_tiles_mf).
+constexpr int kStepMfMinBlocks = 6;
+template <int BLOCK, int FRONT, bool STATES>
+__global__ void __launch_bounds__(BLOCK, kStepMfMinBlocks)
+quad_step_mf_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn,
+                    const __grid_constant__ MfCfg mf) {
+    quad_step_body<BLOCK, FRONT, STATES, true, false, true>(OZL_STEP_ARGS, mf);
+}
+template <int BLOCK, int FRONT, bool STATES>
+__global__ void __launch_bounds__(BLOCK, 4)
+quad_step_mf_subwave_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn,
+                            const __grid_constant__ MfCfg mf) {
+    quad_step_body<BLOCK, FRONT, STATES, true, true, true>(OZL_STEP_ARGS, mf);
+}
 
 // ------------------------------------------------------------------------------------------------ K1, TMA-pipelined
 // Persistent variant for large N (rotor-action mode, stored target): one CTA per (SM x 8) slot loops over tiles of
@@ -262,8 +321,12 @@ constexpr int kTmaMinBlocks = 5;       // CTAs per SM of the TMA kernel, and its
         int64_t* __restrict__ reset, int64_t* __restrict__ progress, uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, \
         const int64_t full_tiles
 #define OZL_TMA_ARGS c, pl, actions, obs, rew, reset, progress, timeout, ep_ret_out, full_tiles, states_map, scn
-template <bool STATES, bool SCN>
-__device__ __forceinline__ void quad_step_tma_body(OZL_TMA_PARAMS, const CUtensorMap& states_map, const float* __restrict__ scn) {
+// MF: fault_mode 2 (quad_step_tma_mf_kernel): thread 0 prefetches the next tile's 2 KiB of e_0..e_3 into L2 with one bulk prefetch
+// when it issues that tile's copies, and each thread reads its lane where it is used (RotorEff; a 2 KiB bulk copy into the stage
+// would leave room for 4 CTAs per SM, not 5, with the states tile); `scn` may be NULL.
+template <bool STATES, bool SCN, bool MF = false>
+__device__ __forceinline__ void quad_step_tma_body(OZL_TMA_PARAMS, const CUtensorMap& states_map, const float* __restrict__ scn,
+                                                   const MfCfg& mf = MfCfg{}) {
     __shared__ __align__(128) unsigned char s_stage[kTmaStageBytes];
     __shared__ __align__(16) float s_obs[kTile * 13];
     __shared__ __align__(1024) float s_states[STATES ? kTile * OZL_STATES_WIDTH : 4];   // 16 KB: 5 CTAs/SM still fit
@@ -295,6 +358,10 @@ __device__ __forceinline__ void quad_step_tma_body(OZL_TMA_PARAMS, const CUtenso
     unsigned long long tile_base = 0;
     if (tid == 0) {
         if (tile < full_tiles) issue(tile);
+        if constexpr (MF) {
+            if (tile < full_tiles)
+                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(mf.eff4 + tile * kTile), "r"(kTile * 16) : "memory");
+        }
         const unsigned long long v = atomicAdd(pl.ctrl + 4, 1ull);
         tile_base = (v / (unsigned long long)full_tiles) * (unsigned long long)full_tiles;
         nxt = (long long)gridDim.x + (long long)(v - tile_base);
@@ -331,6 +398,8 @@ __device__ __forceinline__ void quad_step_tma_body(OZL_TMA_PARAMS, const CUtenso
         if (tid == 0) {
             if (next < full_tiles) {
                 issue(next);
+                if constexpr (MF)   // the next tile's 2 KiB of e_0..e_3 into L2; each thread reads its lane where it is used
+                    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(mf.eff4 + next * kTile), "r"(kTile * 16) : "memory");
                 nxt = (long long)gridDim.x + (long long)(atomicAdd(pl.ctrl + 4, 1ull) - tile_base);
             }
         }
@@ -341,8 +410,16 @@ __device__ __forceinline__ void quad_step_tma_body(OZL_TMA_PARAMS, const CUtenso
         const float act[4] = {a4.x, a4.y, a4.z, a4.w};
         const uint32_t genv = c.env_id_base + (uint32_t)i;
         StepOut o;
-        env_step<SCN>(e, act, prog, rst, genv, step, c, o, ACT_ROTORS, nullptr, SCN ? scn + i * OZL_SCENARIO_WIDTH : nullptr);
-        if constexpr (STATES) stage_states_row(s_states, tid, o.obs, e, o, c);
+        RotorEff rf;
+        if constexpr (MF) {
+            rf.in_mem = true;
+            rf.i = i;
+            rf.m = &mf;
+        }
+        env_step<SCN, MF>(e, act, prog, rst, genv, step, c, o, ACT_ROTORS, nullptr,
+                          SCN ? ((MF && !scn) ? nullptr : scn + i * OZL_SCENARIO_WIDTH) : nullptr, nullptr, MF ? &rf : nullptr);
+        if constexpr (STATES && MF) stage_states_row_mf(s_states, tid, o.obs, e, o, c, rf, true);
+        else if constexpr (STATES) stage_states_row(s_states, tid, o.obs, e, o, c);
         obs_epilogue(o.obs, genv, step, blackout, c);
         store_dynamic(pl, i, e);
         if (o.static_dirty) store_static(pl, i, e);
@@ -409,6 +486,12 @@ template <bool STATES>
 __global__ void __launch_bounds__(kTile, kTmaMinBlocks)
 quad_step_tma_scn_kernel(OZL_TMA_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn) {
     quad_step_tma_body<STATES, true>(OZL_TMA_ARGS);
+}
+template <bool STATES>
+__global__ void __launch_bounds__(kTile, kTmaMinBlocks)
+quad_step_tma_mf_kernel(OZL_TMA_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn,
+                        const __grid_constant__ MfCfg mf) {
+    quad_step_tma_body<STATES, true, true>(OZL_TMA_ARGS, mf);
 }
 
 // ------------------------------------------------------------------------------------------------ mode B
@@ -570,8 +653,11 @@ __global__ void set_params_kernel(const Planes pl, int64_t n, const float* param
     store_static(pl, i, e);
 }
 
-// reset phase only (see ozl_apply_resets): same draws as env_step, no physics, no bookkeeping; `scn`: the scenario table or NULL
-__global__ void apply_resets_kernel(const DevCfg c, const Planes pl, const int64_t* __restrict__ reset, const float* __restrict__ scn) {
+// reset phase only (see ozl_apply_resets): same draws as env_step, no physics, no bookkeeping; `scn`: the scenario table or NULL.
+// MF: fault_mode 2 (apply_resets_mf_kernel), its draw and rotor-faults group in place of mode 1's.
+template <bool MF>
+__device__ __forceinline__ void apply_resets_body(const DevCfg& c, const Planes& pl, const int64_t* __restrict__ reset,
+                                                  const float* __restrict__ scn, const MfCfg& mf) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= c.num_envs || reset[i] == 0) return;
     const uint64_t step = read_step(pl.ctrl);
@@ -594,15 +680,36 @@ __global__ void apply_resets_kernel(const DevCfg c, const Planes pl, const int64
     e.p[2] = c.spawn_base[2] + (c.spawn_range[2] * u01(r.z) + c.spawn_lo[2]);
     e.q[0] = e.q[1] = e.q[2] = 0.0f; e.q[3] = 1.0f;
     for (int j = 0; j < 3; ++j) { e.v[j] = 0.0f; e.w[j] = 0.0f; }
-    if (c.fault_mode) {
+    RotorEff rf;
+    rf.in_mem = false;
+    rf.m = &mf;
+    if constexpr (MF) {
+        rfault_draw(e, rf, draw(c.seed, genv, step, P_FAULT), draw(c.seed, genv, step, P_RFAULT), c);
+    } else if (c.fault_mode) {
         const uint4 f = draw(c.seed, genv, step, P_FAULT);
         e.fault = (f.x & 3u) | (__umulhi(f.y, (uint32_t)c.max_episode_length) << 2) | landed;
         e.eff = c.fault_eff_lo + c.fault_eff_range * u01(f.z);
     }
     if (c.dr_enable) dr_draw_all(e, genv, step, c);
     if (scn) scn_respawn(e, scn + i * OZL_SCENARIO_WIDTH);
+    if constexpr (MF) {
+        if (scn) scn_rfault(e, rf, scn + i * OZL_SCENARIO_WIDTH);
+        mf.eff4[i] = make_float4(rf.e[0], rf.e[1], rf.e[2], rf.e[3]);
+    }
     store_dynamic(pl, i, e);
     store_static(pl, i, e);
+}
+__global__ void apply_resets_kernel(const DevCfg c, const Planes pl, const int64_t* __restrict__ reset, const float* __restrict__ scn) {
+    apply_resets_body<false>(c, pl, reset, scn, MfCfg{});
+}
+__global__ void apply_resets_mf_kernel(const DevCfg c, const Planes pl, const int64_t* __restrict__ reset, const float* __restrict__ scn,
+                                       const __grid_constant__ MfCfg mf) {
+    apply_resets_body<true>(c, pl, reset, scn, mf);
+}
+// fault_mode 2 part of ozl_reset_all: no fault in the initial episode (init_state_kernel writes onset never)
+__global__ void rfault_init_kernel(float4* eff4, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) eff4[i] = make_float4(1.0f, 1.0f, 1.0f, 1.0f);
 }
 
 __global__ void init_state_kernel(const DevCfg c, const Planes pl) {
@@ -757,6 +864,7 @@ extern "C" int ozl_cfg_default(ozl_cfg* c, int64_t num_envs) {
     c->arm = (float)arm;
     c->max_angvel = (float)(4.0 * M_PI);
     c->fault_eff_lo = 0.0f; c->fault_eff_range = 0.5f;
+    c->fault_rotors_lo = 1; c->fault_rotors_hi = 1; c->fault_ramp_steps = 0;
     for (int j = 0; j < OZL_DR_NUM; ++j) {       // isaacgymenvs/utils/dr_utils.py:121-130 (scaling, uniform); yaw_km: not randomised
         c->dr[j].distribution = j == OZL_DR_YAW_KM ? OZL_DR_NONE : OZL_DR_UNIFORM;
         c->dr[j].operation = OZL_DR_SCALING;
@@ -785,6 +893,18 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
         !(cfg->iyy > 1e-30f && cfg->iyy < 1e30f) || !(cfg->izz > 1e-30f && cfg->izz < 1e30f))
         return set_error("ozl_create: mass and inertia must be positive normal floats");
     if (cfg->wrench_warmup_steps < 0) return set_error("ozl_create: wrench_warmup_steps must be >= 0");
+    if (cfg->fault_mode == 2) {
+        if (!(0 <= cfg->fault_rotors_lo && cfg->fault_rotors_lo <= cfg->fault_rotors_hi && cfg->fault_rotors_hi <= 4))
+            return set_error("ozl_create: fault_mode 2 needs 0 <= fault_rotors_lo <= fault_rotors_hi <= 4 (got %d, %d)",
+                             (int)cfg->fault_rotors_lo, (int)cfg->fault_rotors_hi);
+        if (cfg->fault_ramp_steps < 0 || cfg->fault_ramp_steps >= (1 << 24))
+            return set_error("ozl_create: fault_ramp_steps %d is not in [0, 2^24)", (int)cfg->fault_ramp_steps);
+        if (!(cfg->fault_eff_lo >= 0.0f && cfg->fault_eff_lo <= 1.0f))
+            return set_error("ozl_create: fault_eff_lo %g is not in [0, 1]", (double)cfg->fault_eff_lo);
+        if (!(cfg->fault_eff_range >= 0.0f && (double)cfg->fault_eff_lo + (double)cfg->fault_eff_range <= 1.0))
+            return set_error("ozl_create: fault_eff_lo + fault_eff_range (%g + %g) is not in [fault_eff_lo, 1]",
+                             (double)cfg->fault_eff_lo, (double)cfg->fault_eff_range);
+    }
     for (int j = 0; j < OZL_DR_NUM; ++j) {
         const ozl_dr_param& d = cfg->dr[j];
         if (d.distribution < OZL_DR_NONE || d.distribution > OZL_DR_GAUSSIAN) return set_error("ozl_create: dr[%d].distribution %d unknown", j, d.distribution);
@@ -808,6 +928,7 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
     e->states = nullptr;
     memset(e->states_tmap, 0, sizeof(e->states_tmap));
     e->scn_buf = e->scn = nullptr;
+    e->mf = MfCfg{};
     derive_dev_cfg(*cfg, e->dev);
     e->device = device;
     e->sm_count = prop.multiProcessorCount;
@@ -821,6 +942,8 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
         // (override: OZL_TMA_MIN_TILES, 0 = never)
         const char* ev = getenv("OZL_TMA_MIN_TILES");
         e->tma_min_tiles = ev ? atoll(ev) : (long long)kStepMinBlocks * prop.multiProcessorCount + 1;
+        // fault_mode 2: the generic twin holds 6 CTAs per SM (kStepMfMinBlocks), so its one-wave limit is lower
+        e->tma_min_tiles_mf = ev ? atoll(ev) : (long long)kStepMfMinBlocks * prop.multiProcessorCount + 1;
     }
     {   // up to one wave of quad_step_subwave_kernel (4 x 128-env CTAs per SM: 75776 envs on 148 SMs) the generic launch runs it.
         // Measured on B200 at 1000 W (us per step, default kernel -> sub-wave kernel, cold / warm L2; DESIGN.md section 6):
@@ -836,7 +959,8 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
     const size_t state = align_up(tiles * (size_t)kTileBytes, 256);
     const size_t ctrl = 256, metrics = align_up(sizeof(double) * kMetricSlots * kMetricStride, 256);
     const size_t tile_seq = align_up(tiles * 4 * sizeof(unsigned long long), 256);    // {started, done} per CTA of >= 64 envs
-    e->arena_bytes = state + ctrl + metrics + tile_seq;
+    const size_t eff4 = cfg->fault_mode == 2 ? tiles * kTile * sizeof(float4) : 0;      // fault_mode 2: MfCfg::eff4
+    e->arena_bytes = state + ctrl + metrics + tile_seq + eff4;
     if (check_cuda(cudaMalloc(&e->arena, e->arena_bytes), "cudaMalloc(state arena)")) { delete e; return 1; }
     if (check_cuda(cudaMemset(e->arena, 0, e->arena_bytes), "cudaMemset(state arena)")) { cudaFree(e->arena); delete e; return 1; }
     char* p = (char*)e->arena;
@@ -844,7 +968,12 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
     p += state;
     e->pl.ctrl = (unsigned long long*)p; p += ctrl;
     e->pl.metrics = (double*)p; p += metrics;
-    e->pl.tile_seq = (unsigned long long*)p;
+    e->pl.tile_seq = (unsigned long long*)p; p += tile_seq;
+    e->mf.eff4 = eff4 ? (float4*)p : nullptr;
+    e->mf.rotors_lo = (uint32_t)cfg->fault_rotors_lo;
+    e->mf.rotors_span = (uint32_t)(cfg->fault_rotors_hi - cfg->fault_rotors_lo + 1);
+    e->mf.ramp_steps = cfg->fault_ramp_steps;
+    e->mf.inv_ramp = cfg->fault_ramp_steps > 0 ? (float)(1.0 / (double)cfg->fault_ramp_steps) : 0.0f;    // rounded once
     {
         const char* cv = getenv("OZL_EKF_CHAIN");
         e->chain_mode = cv ? atoi(cv) : 1;
@@ -889,6 +1018,7 @@ extern "C" int ozl_reset_all(ozl_env* env, uint64_t seed, void* stream) {
     int64_t n = env->cfg.num_envs;
     if (n < kMetricSlots * kMetricStride) n = kMetricSlots * kMetricStride;
     init_state_kernel<<<blocks_for(n, 256), 256, 0, st>>>(env->dev, env->pl);
+    if (env->mf.eff4) rfault_init_kernel<<<blocks_for(env->cfg.num_envs, 256), 256, 0, st>>>(env->mf.eff4, env->cfg.num_envs);
     return check_cuda(cudaGetLastError(), "init_state_kernel");
 }
 
@@ -910,28 +1040,43 @@ static int launch_step_t(ozl_env* env, const float* actions, const float* target
     const int64_t full_tiles = n / kTile, tail = n % kTile;
     const int64_t resident = (int64_t)env->sm_count * kTmaMinBlocks;
     const bool plain = (target_in == nullptr) && act_mode == ACT_ROTORS && done_u8 == nullptr && reset_mirror == nullptr && obs_bulk;
-    const auto tma_kernel = SCN ? quad_step_tma_scn_kernel<STATES> : quad_step_tma_kernel<STATES>;
+    // cfg.fault_mode 2: the twins, which take MfCfg as one more argument and read the scenario row when `scn` is set
+    const bool mf = env->cfg.fault_mode == 2;
     const auto kernel = SCN ? quad_step_scn_kernel<kStepBlock, FRONT_NONE, STATES> : quad_step_kernel<kStepBlock, FRONT_NONE, STATES>;
-    const auto step_kernel = n <= env->early_draw_max_envs ? quad_step_subwave_kernel<kStepBlock, FRONT_NONE, STATES, SCN> : kernel;
-    if (plain && env->tma_min_tiles > 0 && full_tiles >= env->tma_min_tiles &&
+    const bool subwave = n <= env->early_draw_max_envs;
+    const long long tma_min_tiles = mf ? env->tma_min_tiles_mf : env->tma_min_tiles;
+    if (plain && tma_min_tiles > 0 && full_tiles >= tma_min_tiles &&
         !(((uintptr_t)progress | (uintptr_t)reset) & 15)) {
         // large N: persistent TMA-pipelined kernel over the whole tiles, then one generic block for the ragged tail
         unsigned grid = (unsigned)(full_tiles < resident ? full_tiles : resident);
         while ((full_tiles + grid - 1) / grid > 8192) grid *= 2;     // 16-bit packed metric counters: keep tiles per CTA far below 65535
-        if (launch_pdl(tma_kernel, dim3(grid), dim3(kTile), st, env->dev, env->pl, (const float4*)actions, obs, rew,
-                       reset, progress, timeout, ep_ret, full_tiles, states_map(env), (const float*)env->scn))
+        const auto tma = [&](auto k, auto... mfa) {
+            return launch_pdl(k, dim3(grid), dim3(kTile), st, env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout,
+                              ep_ret, full_tiles, states_map(env), (const float*)env->scn, mfa...);
+        };
+        if (mf ? tma(quad_step_tma_mf_kernel<STATES>, env->mf) : tma(SCN ? quad_step_tma_scn_kernel<STATES> : quad_step_tma_kernel<STATES>))
             return check_cuda(cudaGetLastError(), "quad_step_tma_kernel");
-        if (tail)
-            kernel<<<1, kStepBlock, 0, st>>>(env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, nullptr,
-                                             ACT_ROTORS, nullptr, nullptr, 1, full_tiles * kTile, FrontArgs{},
-                                             (volatile unsigned int*)nullptr, 0u, states_map(env), (const float*)env->scn);
+        const auto tail_block = [&](auto k, auto... mfa) {
+            k<<<1, kStepBlock, 0, st>>>(env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, nullptr,
+                                        ACT_ROTORS, nullptr, nullptr, 1, full_tiles * kTile, FrontArgs{}, (volatile unsigned int*)nullptr,
+                                        0u, states_map(env), (const float*)env->scn, mfa...);
+        };
+        if (tail) {
+            if (mf) tail_block(quad_step_mf_kernel<kStepBlock, FRONT_NONE, STATES>, env->mf);
+            else tail_block(kernel);
+        }
         return check_cuda(cudaGetLastError(), "quad_step_kernel(tail)");
     }
-    if (launch_pdl(step_kernel, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev,
-                   env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, target_in, act_mode, done_u8, reset_mirror,
-                   obs_bulk, (int64_t)0, FrontArgs{}, (volatile unsigned int*)(host_flag ? env->host_done : nullptr),
-                   host_flag ? ++env->host_seq : 0u, states_map(env), (const float*)env->scn))
-        return check_cuda(cudaGetLastError(), "quad_step_kernel");
+    const auto gen = [&](auto k, auto... mfa) {
+        return launch_pdl(k, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev, env->pl, (const float4*)actions, obs, rew,
+                          reset, progress, timeout, ep_ret, target_in, act_mode, done_u8, reset_mirror, obs_bulk, (int64_t)0, FrontArgs{},
+                          (volatile unsigned int*)(host_flag ? env->host_done : nullptr), host_flag ? ++env->host_seq : 0u,
+                          states_map(env), (const float*)env->scn, mfa...);
+    };
+    const int rc = mf ? gen(subwave ? quad_step_mf_subwave_kernel<kStepBlock, FRONT_NONE, STATES> : quad_step_mf_kernel<kStepBlock, FRONT_NONE, STATES>,
+                            env->mf)
+                      : gen(subwave ? quad_step_subwave_kernel<kStepBlock, FRONT_NONE, STATES, SCN> : kernel);
+    if (rc) return check_cuda(cudaGetLastError(), "quad_step_kernel");
     return 0;
 }
 
@@ -965,18 +1110,25 @@ static int launch_front_step(ozl_env* env, int front, const float* actions, cons
     const int64_t n = env->cfg.num_envs;
     const bool subwave = n <= env->early_draw_max_envs;
     cudaStream_t st = (cudaStream_t)stream;
-#define OZL_LAUNCH_FRONT(F, S, MODE)                                                                                            \
-    launch_pdl(subwave ? (env->scn ? quad_step_subwave_kernel<kStepBlock, F, S, true> : quad_step_subwave_kernel<kStepBlock, F, S, false>) \
-                       : (env->scn ? quad_step_scn_kernel<kStepBlock, F, S> : quad_step_kernel<kStepBlock, F, S>),                   \
-               dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret,          \
-               (const float*)nullptr, (int)MODE, (uint8_t*)nullptr, (int64_t*)nullptr, 1, (int64_t)0, fa,                           \
-               (volatile unsigned int*)nullptr, 0u, states_map(env), (const float*)env->scn)
+#define OZL_PICK(F, S)                                                                                                          \
+    (subwave ? (env->scn ? quad_step_subwave_kernel<kStepBlock, F, S, true> : quad_step_subwave_kernel<kStepBlock, F, S, false>) \
+             : (env->scn ? quad_step_scn_kernel<kStepBlock, F, S> : quad_step_kernel<kStepBlock, F, S>))
+#define OZL_PICK_MF(F, S) (subwave ? quad_step_mf_subwave_kernel<kStepBlock, F, S> : quad_step_mf_kernel<kStepBlock, F, S>)
+    const auto go = [&](auto k, int mode, auto... mfa) {
+        return launch_pdl(k, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev, env->pl, (const float4*)actions, obs, rew,
+                          reset, progress, timeout, ep_ret, (const float*)nullptr, mode, (uint8_t*)nullptr, (int64_t*)nullptr, 1, (int64_t)0,
+                          fa, (volatile unsigned int*)nullptr, 0u, states_map(env), (const float*)env->scn, mfa...);
+    };
+    const bool mf = env->cfg.fault_mode == 2;          // the fault_mode 2 twins (FRONT_LEE: refused by ozl_lee_landed_step)
     int rc;
-    if (front == FRONT_VEHICLE)
-        rc = env->states ? OZL_LAUNCH_FRONT(FRONT_VEHICLE, true, ACT_ROTORS) : OZL_LAUNCH_FRONT(FRONT_VEHICLE, false, ACT_ROTORS);
+    if (front == FRONT_VEHICLE && mf)
+        rc = env->states ? go(OZL_PICK_MF(FRONT_VEHICLE, true), ACT_ROTORS, env->mf) : go(OZL_PICK_MF(FRONT_VEHICLE, false), ACT_ROTORS, env->mf);
+    else if (front == FRONT_VEHICLE)
+        rc = env->states ? go(OZL_PICK(FRONT_VEHICLE, true), ACT_ROTORS) : go(OZL_PICK(FRONT_VEHICLE, false), ACT_ROTORS);
     else
-        rc = env->states ? OZL_LAUNCH_FRONT(FRONT_LEE, true, ACT_WRENCH) : OZL_LAUNCH_FRONT(FRONT_LEE, false, ACT_WRENCH);
-#undef OZL_LAUNCH_FRONT
+        rc = env->states ? go(OZL_PICK(FRONT_LEE, true), ACT_WRENCH) : go(OZL_PICK(FRONT_LEE, false), ACT_WRENCH);
+#undef OZL_PICK_MF
+#undef OZL_PICK
     if (rc) return check_cuda(cudaGetLastError(), who);
     return 0;
 }
@@ -990,6 +1142,8 @@ extern "C" int ozl_landing_step(ozl_env* env, const float* actions, const ozl_hu
 extern "C" int ozl_lee_landed_step(ozl_env* env, const ozl_lee_landed_args* in, const ozl_husky_args* husky, float* obs, float* rew,
                                    int64_t* reset, int64_t* progress, uint8_t* timeout, float* ep_ret, void* stream) {
     if (!in || !in->gains16) return set_error("ozl_lee_landed_step: NULL argument");
+    if (env && env->cfg.fault_mode == 2)
+        return set_error("ozl_lee_landed_step: cfg.fault_mode 2 (multi-rotor faults) does not apply to the wrench-actuated step");
     if ((uintptr_t)in->wrench4 & 15) return set_error("ozl_lee_landed_step: wrench4 must be 16-byte aligned");
     FrontArgs fa{};
     for (int k = 0; k < 3; ++k) { fa.g.kP[k] = in->gains16[k]; fa.g.kV[k] = in->gains16[3 + k]; fa.g.kR[k] = in->gains16[6 + k]; fa.g.kO[k] = in->gains16[9 + k]; }
@@ -1066,13 +1220,17 @@ extern "C" int ozl_step_wrench(ozl_env* env, const float* wrench4, const float* 
 extern "C" int ozl_apply_resets(ozl_env* env, const int64_t* reset, void* stream) {
     OZL_ENV_CHECK("ozl_apply_resets");
     if (!reset) return set_error("ozl_apply_resets: reset is NULL");
-    apply_resets_kernel<<<blocks_for(env->cfg.num_envs, 256), 256, 0, st>>>(env->dev, env->pl, reset, env->scn);
+    if (env->mf.eff4)
+        apply_resets_mf_kernel<<<blocks_for(env->cfg.num_envs, 256), 256, 0, st>>>(env->dev, env->pl, reset, env->scn, env->mf);
+    else
+        apply_resets_kernel<<<blocks_for(env->cfg.num_envs, 256), 256, 0, st>>>(env->dev, env->pl, reset, env->scn);
     return check_cuda(cudaGetLastError(), "apply_resets_kernel");
 }
 
 extern "C" int ozl_rollout(ozl_env* env, int32_t K, float* obs, float* rew, int64_t* reset, int64_t* progress, void* stream) {
     OZL_ENV_CHECK("ozl_rollout");
     if (K <= 0) return set_error("ozl_rollout: K must be > 0");
+    if (env->cfg.fault_mode == 2) return set_error("ozl_rollout: cfg.fault_mode 2 (multi-rotor faults) is not applied by the K-step kernel");
     if (env->states) return set_error("ozl_rollout: a states output is registered (ozl_set_states_output) and the K-step kernel does not write it");
     if (env->scn) return set_error("ozl_rollout: a scenario table is registered (ozl_set_scenarios) and the K-step kernel does not apply it");
     if (!obs || !rew || !reset || !progress) return set_error("ozl_rollout: NULL buffer");
@@ -1119,8 +1277,31 @@ static int check_scenario_row(const ozl_cfg& cfg, const float* r, int64_t row) {
         {OZL_SCN_THRUST_SCALE, 1, "thrust_scale"}, {OZL_SCN_YAW_KM, 1, "yaw_km"}};
     const char* who = "ozl_set_scenarios";
     const long long k = (long long)row;
-    for (int j = OZL_SCN_RESERVED; j < OZL_SCENARIO_WIDTH; ++j)
-        if (!std::isnan(r[j])) return set_error("%s: row %lld: reserved slot %d must be NaN", who, k, j);
+    const bool mf = cfg.fault_mode == 2;
+    for (int j = OZL_SCN_RESERVED; j < OZL_SCENARIO_WIDTH; ++j) {
+        if (std::isnan(r[j])) continue;
+        if (j == OZL_SCENARIO_WIDTH - 1) return set_error("%s: row %lld: reserved slot %d must be NaN", who, k, j);
+        if (!mf)
+            return set_error("%s: row %lld: reserved slot %d must be NaN (slots 26-30 are the rotor-faults group, which needs "
+                             "cfg.fault_mode 2, rotorFault.mode \"multi\")", who, k, j);
+    }
+    if (mf) {       // the rotor-faults group: all NaN or all finite, as the groups below
+        int nan = 0;
+        for (int j = OZL_SCN_RFAULT_ONSET; j < OZL_SCN_RFAULT_EFF + 4; ++j) {
+            if (std::isnan(r[j])) ++nan;
+            else if (!std::isfinite(r[j])) return set_error("%s: row %lld: rotor faults group has a non-finite value in slot %d", who, k, j);
+        }
+        if (nan != 0 && nan != 5) return set_error("%s: row %lld: rotor faults group must be all NaN or all set", who, k);
+        if (nan == 0) {
+            const float onset = r[OZL_SCN_RFAULT_ONSET];
+            if (!(onset >= 0.0f && onset < 16777216.0f && onset == std::floor(onset)))
+                return set_error("%s: row %lld: rotor faults onset %g is not an integer in [0, 2^24)", who, k, (double)onset);
+            for (int j = 0; j < 4; ++j)
+                if (!(r[OZL_SCN_RFAULT_EFF + j] >= 0.0f && r[OZL_SCN_RFAULT_EFF + j] <= 1.0f))
+                    return set_error("%s: row %lld: rotor faults effectiveness %g of rotor %d is not in [0, 1]", who, k,
+                                     (double)r[OZL_SCN_RFAULT_EFF + j], j);
+        }
+    }
     for (const auto& g : groups) {
         int nan = 0;
         for (int j = g.first; j < g.first + g.count; ++j) {
@@ -1138,6 +1319,9 @@ static int check_scenario_row(const ozl_cfg& cfg, const float* r, int64_t row) {
     if (set(OZL_SCN_TARGET) && cfg.target_fixed)
         return set_error("%s: row %lld: target group set, but cfg.target_fixed is set (the target is driven by a vehicle or the caller)", who, k);
     if (set(OZL_SCN_FAULT_ROTOR)) {
+        if (mf)
+            return set_error("%s: row %lld: fault group (slots 16-18, one rotor) set, but cfg.fault_mode is 2: pin the faults with the "
+                             "rotor faults group (slots 26-30)", who, k);
         if (!cfg.fault_mode)
             return set_error("%s: row %lld: fault group set, but the handle has no rotor-fault model (cfg.fault_mode, rotorFault.enable)", who, k);
         const float rotor = r[OZL_SCN_FAULT_ROTOR], onset = r[OZL_SCN_FAULT_ONSET], eff = r[OZL_SCN_FAULT_EFF];
@@ -1198,6 +1382,26 @@ extern "C" int ozl_set_params(ozl_env* env, const float* params8, const int32_t*
     OZL_ENV_CHECK("ozl_set_params");
     set_params_kernel<<<blocks_for(env->cfg.num_envs, 256), 256, 0, st>>>(env->pl, env->cfg.num_envs, params8, fault2);
     return check_cuda(cudaGetLastError(), "set_params_kernel");
+}
+
+static int rotor_eff_check(ozl_env* env, const void* eff4, const char* who) {
+    if (!env) return set_error("%s: env is NULL", who);
+    if (env->cfg.fault_mode != 2)
+        return set_error("%s: the handle has no per-rotor effectiveness (cfg.fault_mode is %d, it needs 2)", who, (int)env->cfg.fault_mode);
+    if (!eff4) return set_error("%s: eff4 is NULL", who);
+    if ((uintptr_t)eff4 & 15) return set_error("%s: eff4 must be 16-byte aligned", who);
+    return 0;
+}
+// MfCfg::eff4 is row-major [N, 4] over the first N lanes: one stream-ordered copy each way
+extern "C" int ozl_get_rotor_eff(ozl_env* env, float* eff4, void* stream) {
+    if (rotor_eff_check(env, eff4, "ozl_get_rotor_eff")) return 1;
+    return check_cuda(cudaMemcpyAsync(eff4, env->mf.eff4, (size_t)env->cfg.num_envs * sizeof(float4), cudaMemcpyDeviceToDevice,
+                                      (cudaStream_t)stream), "cudaMemcpyAsync(rotor effectiveness)");
+}
+extern "C" int ozl_set_rotor_eff(ozl_env* env, const float* eff4, void* stream) {
+    if (rotor_eff_check(env, eff4, "ozl_set_rotor_eff")) return 1;
+    return check_cuda(cudaMemcpyAsync(env->mf.eff4, eff4, (size_t)env->cfg.num_envs * sizeof(float4), cudaMemcpyDeviceToDevice,
+                                      (cudaStream_t)stream), "cudaMemcpyAsync(rotor effectiveness)");
 }
 
 extern "C" int ozl_get_step_count(ozl_env* env, uint64_t* out, void* stream) {

@@ -14,6 +14,7 @@ import torch
 from ._lib import SCENARIO_LAYOUT, SCENARIO_WIDTH
 
 _ROTOR, _ONSET, _EFF = (SCENARIO_LAYOUT[k] for k in ("OZL_SCN_FAULT_ROTOR", "OZL_SCN_FAULT_ONSET", "OZL_SCN_FAULT_EFF"))
+_RONSET, _REFF = SCENARIO_LAYOUT["OZL_SCN_RFAULT_ONSET"], SCENARIO_LAYOUT["OZL_SCN_RFAULT_EFF"]
 
 
 def empty(n):
@@ -31,6 +32,21 @@ def fault_grid(n, rotors, onsets, effectiveness):
     grid = torch.tensor(combos, dtype=torch.float32)
     rows = empty(n)
     rows[:, _ROTOR:_EFF + 1] = grid[torch.arange(int(n)) % len(combos)]
+    return rows
+
+
+def multi_fault_grid(n, effectiveness, onsets):
+    """Rows whose rotor-faults group (rotorFault.mode "multi") runs through effectiveness x onsets (the last one fastest), tiled
+    over the n envs like `fault_grid`: `effectiveness` is a list of 4-tuples (e_0..e_3, each in [0, 1]; (1, 1, 1, 1) means no
+    fault in that episode).  Every other group is NaN."""
+    combos = [tuple(float(x) for x in e) + (float(o),) for e, o in itertools.product(effectiveness, onsets)]
+    if not combos:
+        raise ValueError("multi_fault_grid: effectiveness and onsets must not be empty")
+    if any(len(c) != 5 for c in combos):
+        raise ValueError("multi_fault_grid: every effectiveness entry must have four values (rotors 0..3)")
+    grid = torch.tensor([(c[4],) + c[:4] for c in combos], dtype=torch.float32)       # onset, e_0..e_3 (slot order)
+    rows = empty(n)
+    rows[:, _RONSET:_REFF + 4] = grid[torch.arange(int(n)) % len(combos)]
     return rows
 
 

@@ -146,6 +146,20 @@ class QuadSim:
         check(lib.ozl_set_params(self._h, ptr(params7), ptr(fault2), _stream()))
         torch.cuda.current_stream().synchronize()
 
+    def get_rotor_eff(self):
+        """fault_mode 2: e_0..e_3 of every env's current episode, [N, 4] float32 CUDA tensor (ozl_get_rotor_eff)."""
+        out = self._new(self.num_envs, 4)
+        check(lib.ozl_get_rotor_eff(self._h, out.data_ptr(), _stream()), ValueError)
+        return out
+
+    def set_rotor_eff(self, eff4):
+        """fault_mode 2: replace e_0..e_3 of every env ([N, 4]; the faulted rotors and the onset stay as drawn)."""
+        eff4 = eff4.to(device=self.device, dtype=torch.float32).contiguous()
+        if tuple(eff4.shape) != (self.num_envs, 4):
+            raise ValueError(f"expected shape {(self.num_envs, 4)}, got {tuple(eff4.shape)}")
+        check(lib.ozl_set_rotor_eff(self._h, eff4.data_ptr(), _stream()), ValueError)
+        torch.cuda.current_stream().synchronize()   # the input may be a temporary
+
     @property
     def step_count(self):
         out = C.c_uint64()

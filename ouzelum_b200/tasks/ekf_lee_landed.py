@@ -24,7 +24,7 @@ from ..ahrs_ekf import EKFBank
 from ..controllers import Controller, control
 from ..pv_filter import PVFilterBank
 from .landing import TARGET_Z, _VehicleTargetTask
-from .ouzelum import _POMDP, x500_cfg_from_task
+from .ouzelum import _POMDP, refuse_multi_fault, x500_cfg_from_task
 
 
 class EKFLeeLanded(_VehicleTargetTask):
@@ -53,6 +53,7 @@ class EKFLeeLanded(_VehicleTargetTask):
     def _native_cfg(self):
         # the observation itself also goes through the sensor-fault model env-side (ekf_lee_landed.py:659)
         # wrench_warmup_steps: during the estimator warm-up the hover force reaches every env and no landing is flagged (:508-529)
+        refuse_multi_fault(type(self).__name__, self.cfg["env"])
         return x500_cfg_from_task(self.cfg, self.num_envs, target_fixed=1, die_z=self.die_z, plate_enable=1,
                                   plate_z=TARGET_Z, plate_radius=0.35, land_cutoff=self.land_cutoff,
                                   wrench_warmup_steps=int(self.ConvergenceTime))

@@ -13,7 +13,7 @@ import torch
 
 from ..controllers import Controller, control
 from .landing import TARGET_Z, _VehicleTargetTask
-from .ouzelum import x500_cfg_from_task
+from .ouzelum import refuse_multi_fault, x500_cfg_from_task
 
 
 class LeeLanded(_VehicleTargetTask):
@@ -24,6 +24,7 @@ class LeeLanded(_VehicleTargetTask):
         # the landing detector of this task measures the distance to the CONTROLLER target (0,0,1), which is also what the
         # stored target is set to below; the reward's target rides on the Husky (post_physics_step, lee_landed.py:339-340)
         # (the detector distance is measured to the controller target: the step kernels take it as `det_tgt`)
+        refuse_multi_fault(type(self).__name__, self.cfg["env"])
         return x500_cfg_from_task(self.cfg, self.num_envs, target_fixed=1, die_z=self.die_z, plate_enable=1,
                                   plate_z=TARGET_Z, plate_radius=0.35,
                                   land_cutoff=self.land_cutoff if bool(self.cfg["env"].get("fusedStep", True)) else 0.0)

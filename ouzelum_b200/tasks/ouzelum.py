@@ -69,6 +69,34 @@ def dr_from_task_cfg(cfg):
     return enable, out
 
 
+def rotor_fault_cfg(fault):
+    """env["rotorFault"] = {enable, mode: "single" | "multi", rotors: [lo, hi], effLow, effHigh, rampSteps} -> ozl_cfg fields.
+    "single" (the default) is fault_mode 1; "multi" is fault_mode 2 (several rotors, gradual loss: include/ouzelum_b200.h)."""
+    fault = fault or {}
+    mode = fault.get("mode", "single")
+    if mode not in ("single", "multi"):
+        raise ValueError(f"rotorFault.mode must be 'single' or 'multi', got {mode!r}")
+    lo_e, hi_e = float(fault.get("effLow", 0.0)), float(fault.get("effHigh", 0.5))
+    kw = dict(fault_mode=(2 if mode == "multi" else 1) if fault.get("enable", False) else 0, fault_eff_lo=lo_e, fault_eff_range=hi_e - lo_e)
+    rotors, ramp = fault.get("rotors", [1, 1]), fault.get("rampSteps", 0)
+    if mode == "multi":
+        if len(rotors) != 2 or any(int(r) != r for r in rotors) or not 0 <= rotors[0] <= rotors[1] <= 4:
+            raise ValueError(f"rotorFault.rotors must be [lo, hi] with integers 0 <= lo <= hi <= 4, got {rotors!r}")
+        if int(ramp) != ramp or not 0 <= ramp < 1 << 24:
+            raise ValueError(f"rotorFault.rampSteps must be an integer in [0, 2^24), got {ramp!r}")
+        if not 0.0 <= lo_e <= hi_e <= 1.0:
+            raise ValueError(f"rotorFault: multi needs 0 <= effLow <= effHigh <= 1, got {lo_e}, {hi_e}")
+    kw.update(fault_rotors_lo=int(rotors[0]), fault_rotors_hi=int(rotors[1]), fault_ramp_steps=int(ramp))
+    return kw
+
+
+def refuse_multi_fault(task_name, env_cfg):
+    """rotorFault.mode "multi" (fault_mode 2) is applied by the rotor-actuated step kernels only: a task whose step is
+    wrench-actuated or has a kernel of its own raises ValueError for it."""
+    if (env_cfg.get("rotorFault", {}) or {}).get("mode", "single") == "multi":
+        raise ValueError(f"{task_name}: rotorFault.mode 'multi' is not supported (its step does not apply per-rotor faults)")
+
+
 def x500_cfg_from_task(cfg, num_envs, **over):
     """Translate the reference-style nested task dict into the C `ozl_cfg`."""
     env, sim = cfg["env"], cfg.get("sim", {})
@@ -88,9 +116,7 @@ def x500_cfg_from_task(cfg, num_envs, **over):
         clip_obs=float(min(env.get("clipObservations", math.inf), 3.0e38)),
         thrust_rate=dt * 2000,                         # ouzelum.py:237-238
         lin_drag=float(env.get("linDrag", 0.0)), yaw_km=float(env.get("yawKm", 0.0)),
-        fault_mode=1 if fault.get("enable", False) else 0,
-        fault_eff_lo=float(fault.get("effLow", 0.0)),
-        fault_eff_range=float(fault.get("effHigh", 0.5)) - float(fault.get("effLow", 0.0)),
+        **rotor_fault_cfg(fault),
         dr_enable=1 if dr_enable else 0, dr=dr,
         pomdp_mode=_POMDP[pomdp], pomdp_prob=float(env.get("pomdp_prob", 0.0)),
         noise_sigma=float(env.get("pomdp_prob", 0.0)),  # POMDP.py:8-9: one knob feeds both
@@ -300,12 +326,14 @@ class X500Task(VecTask):
         """Everything needed to continue bit-identically: private state, per-env parameters, RNG time axis, surface buffers."""
         st = self.sim.get_state()
         params, fault = self.sim.get_params()
+        rotor_eff = self.sim.get_rotor_eff() if self.native_cfg.fault_mode == 2 else None
         torch.cuda.current_stream().synchronize()
         return {"root": st["root"].cpu(), "thrust": st["thrust"].cpu(), "target": st["target"].cpu(), "ep_ret": st["ep_ret"].cpu(),
                 "params": params.cpu(), "fault": fault.cpu(), "step_count": self.sim.step_count,
                 "reset_buf": self.reset_buf.cpu(), "progress_buf": self.progress_buf.cpu(), "obs_buf": self.obs_buf.cpu(),
                 "rew_buf": self.rew_buf.cpu(), "timeout_buf": self._timeout_u8.cpu(), "episode_return_buf": self.episode_return_buf.cpu(),
                 "seed": int(self.native_cfg.seed), "num_envs": self.num_envs, "task": type(self).__name__,
+                **({"rotor_eff": rotor_eff.cpu()} if rotor_eff is not None else {}),
                 "scenarios": None if self.scenarios is None else self.scenarios.clone(),
                 **({"states_buf": self.states_buf.cpu()} if self.num_states > 0 else {})}
 
@@ -314,8 +342,12 @@ class X500Task(VecTask):
             raise ValueError(f"checkpoint has {sd['num_envs']} envs, this env has {self.num_envs}")
         if sd["seed"] != int(self.native_cfg.seed):
             raise ValueError("checkpoint was taken with a different RNG seed")
+        if (self.native_cfg.fault_mode == 2) != ("rotor_eff" in sd):     # refused before anything is loaded
+            raise ValueError("checkpoint and env disagree on rotorFault.mode 'multi' (the per-rotor effectiveness)")
         self.sim.set_state(root=sd["root"], thrust=sd["thrust"], target=sd["target"], ep_ret=sd["ep_ret"])
         self.sim.set_params(sd["params"], sd["fault"])
+        if "rotor_eff" in sd:
+            self.sim.set_rotor_eff(sd["rotor_eff"])
         self.sim.step_count = sd["step_count"]
         self.reset_buf.copy_(sd["reset_buf"])
         self.progress_buf.copy_(sd["progress_buf"])

@@ -12,7 +12,7 @@ import torch
 
 from .._lib import OzlQuadcopterArgs, check, lib
 from ..vec_task import VecTask
-from .ouzelum import asymmetric_states
+from .ouzelum import asymmetric_states, refuse_multi_fault
 
 
 def vehicle_constants():
@@ -39,6 +39,7 @@ class Quadcopter(VecTask):
         self.cfg["env"]["numObservations"] = 21          # quadcopter.py:57-60
         self.cfg["env"]["numActions"] = 12
         asymmetric_states(type(self).__name__, self.cfg["env"], supported=False)      # its 21-obs vehicle has no states output
+        refuse_multi_fault(type(self).__name__, self.cfg["env"])
         super().__init__(config=self.cfg, rl_device=rl_device, sim_device=sim_device, graphics_device_id=graphics_device_id,
                          headless=headless, virtual_screen_capture=virtual_screen_capture, force_render=force_render)
         self._timeout_u8 = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
