@@ -33,7 +33,8 @@ extern "C" {
                                6: (additive) ozl_set_scenarios, OZL_SCN_* layout of a scenario row
                                7: (additive) fault_mode 2 (multi-rotor and gradual rotor faults): ozl_cfg.fault_rotors_lo / _hi /
                                   fault_ramp_steps in the former reserved0 / reserved1 (same size), ozl_get_rotor_eff /
-                                  ozl_set_rotor_eff, scenario group OZL_SCN_RFAULT_* */
+                                  ozl_set_rotor_eff, scenario group OZL_SCN_RFAULT_*
+                                  (additive, still 7) ozl_set_episode_log, OZL_EPLOG_* layout of an episode record */
 
 /* sensor-fault model of isaacgymenvs/utils/POMDP.py:4-42 */
 enum { OZL_POMDP_NONE = 0, OZL_POMDP_FLICKER = 1, OZL_POMDP_NOISE = 2, OZL_POMDP_FLICKER_NOISE = 3 };
@@ -276,6 +277,45 @@ enum { OZL_SCN_POS = 0, OZL_SCN_QUAT = 3, OZL_SCN_LINVEL = 7, OZL_SCN_ANGVEL = 1
  * unregistering after a capture is not seen by that graph (it keeps the kernels it captured), as for ozl_set_states_output.
  * While a table is registered, ozl_rollout and ozl_ekf_lee_landed_step refuse to run (non-zero return, ozl_last_error()). */
 int ozl_set_scenarios(ozl_env* env, const float* rows_host, int32_t width, void* stream);
+
+/* Episode log: the step kernels append one record per episode that ends (reset flag raised) to a caller-owned buffer, with its
+ * termination cause and its conditions, so that survival can be studied as a function of the fault and body parameters of each
+ * episode -- which the next reset overwrites in the env's state.  A record is OZL_EPLOG_WIDTH four-byte slots (128 bytes), every
+ * value from the registers of the step that ended the episode, after the step (the state an OZL_STATE_* row shows for an env
+ * flagged for reset):
+ *   OZL_EPLOG_ENV              global env id (env_id_base + local index), uint32 bits
+ *   OZL_EPLOG_LENGTH           episode length: progress written by that step, int32 bits
+ *   OZL_EPLOG_STEP .. +1       step index of that step (the RNG's time axis), uint64, low word first
+ *   OZL_EPLOG_RETURN           episode return (the ep_ret output of that step)
+ *   OZL_EPLOG_FLAGS            uint32: bit 0 time-out, bit 1 dist > die_dist, bit 2 z < die_z, bit 3 the env landed in this
+ *                              episode (landed flag; metrics slot 2 counts it at the next step's reset), bit 4 rotor fault active
+ *                              in that step (metrics slot 14)
+ *   OZL_EPLOG_ONSET            fault onset (progress step), int32 bits; -1 when the episode had no fault scheduled
+ *   OZL_EPLOG_DIST             final distance to the target, the float32 that was compared with die_dist
+ *   OZL_EPLOG_EFF .. +3        per-rotor effectiveness of the episode: fault_mode 2 e_0..e_3 as drawn (not ramped); fault_mode 1
+ *                              1 except the faulted rotor's effectiveness; no fault scheduled: all 1
+ *   OZL_EPLOG_MASS .. _YAW_KM  mass, ixx, iyy, izz, arm, thrust_scale, yaw_km (absolute, the order of OZL_SCN_MASS ..)
+ *   OZL_EPLOG_POS .. +2        final root position
+ *   OZL_EPLOG_LINVEL .. +2     final linear velocity (world)
+ *   OZL_EPLOG_TARGET .. +2     target of that step
+ *   OZL_EPLOG_RESERVED .. 31   written 0
+ * The contents of a record are deterministic (every draw is keyed by global env id and step: the same bits on every kernel and
+ * sharding); the ORDER of the records is not. */
+enum { OZL_EPLOG_ENV = 0, OZL_EPLOG_LENGTH = 1, OZL_EPLOG_STEP = 2, OZL_EPLOG_RETURN = 4, OZL_EPLOG_FLAGS = 5, OZL_EPLOG_ONSET = 6,
+       OZL_EPLOG_DIST = 7, OZL_EPLOG_EFF = 8, OZL_EPLOG_MASS = 12, OZL_EPLOG_IXX = 13, OZL_EPLOG_IYY = 14, OZL_EPLOG_IZZ = 15,
+       OZL_EPLOG_ARM = 16, OZL_EPLOG_THRUST_SCALE = 17, OZL_EPLOG_YAW_KM = 18, OZL_EPLOG_POS = 19, OZL_EPLOG_LINVEL = 22,
+       OZL_EPLOG_TARGET = 25, OZL_EPLOG_RESERVED = 28, OZL_EPLOG_WIDTH = 32 };
+
+/* Register the episode log: `records` is caller-owned device memory [capacity, OZL_EPLOG_WIDTH] f32 (16-byte aligned), `head` one
+ * device uint64 the caller zeroes.  Every later launch of ozl_step, ozl_step_tracking, ozl_step_wrench, ozl_step_host*,
+ * ozl_landing_step and ozl_lee_landed_step adds the records of the episodes it ends to *head atomically; record k (in the order
+ * the additions hand them out) goes to row k if k < capacity and is dropped otherwise, but still counted: min(*head, capacity)
+ * rows are valid, *head - capacity records were dropped.  Clearing the log is the caller's stream-ordered zeroing of *head, so
+ * step, read and clear can all sit in one CUDA graph.  records = NULL unregisters (the steps then run the kernels without the
+ * log).  Refused: env NULL, width != OZL_EPLOG_WIDTH, capacity < 1, misaligned records, head NULL.  A captured CUDA graph keeps
+ * the log that was registered when it was captured.  While a log is registered, ozl_rollout and ozl_ekf_lee_landed_step refuse
+ * to run (their kernels write no records); ozl_apply_resets ends no episode and writes none. */
+int ozl_set_episode_log(ozl_env* env, float* records, int64_t capacity, uint64_t* head, int32_t width);
 
 /* Mode-B throughput entry: K steps in ONE launch, state held in registers, actions a = 2u-1 drawn
  * in-kernel from the counter RNG; obs/rew are written for the LAST step only, reset/progress are

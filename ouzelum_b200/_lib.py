@@ -26,6 +26,9 @@ STATES_WIDTH = STATES_LAYOUT["OZL_STATES_WIDTH"]
 # scenario rows applied at every reset (ozl_set_scenarios): slot indices OZL_SCN_* and the row width OZL_SCENARIO_WIDTH
 SCENARIO_LAYOUT = _header_enum("OZL_SC")
 SCENARIO_WIDTH = SCENARIO_LAYOUT["OZL_SCENARIO_WIDTH"]
+# episode records appended by the step kernels (ozl_set_episode_log): slot indices OZL_EPLOG_* and the record width
+EPLOG_LAYOUT = _header_enum("OZL_EPLOG")
+EPLOG_WIDTH = EPLOG_LAYOUT["OZL_EPLOG_WIDTH"]
 
 
 DR_NONE, DR_UNIFORM, DR_LOGUNIFORM, DR_GAUSSIAN = 0, 1, 2, 3
@@ -184,6 +187,7 @@ _SIGS = {
     "ozl_rollout": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P]),
     "ozl_set_states_output": (C.c_int, [_P, _P, C.c_int32]),
     "ozl_set_scenarios": (C.c_int, [_P, _P, C.c_int32, _P]),
+    "ozl_set_episode_log": (C.c_int, [_P, _P, C.c_int64, _P, C.c_int32]),
     "ozl_get_state": (C.c_int, [_P] * 6),
     "ozl_set_state": (C.c_int, [_P] * 6),
     "ozl_get_params": (C.c_int, [_P] * 4),

@@ -436,6 +436,8 @@ extern "C" int ozl_ekf_lee_landed_step(ozl_env* env, const ozl_ekf_lee_args* in,
         return set_error("ozl_ekf_lee_landed_step: a states output is registered (ozl_set_states_output) and the fused estimator step does not write it");
     if (env && env->scn)
         return set_error("ozl_ekf_lee_landed_step: a scenario table is registered (ozl_set_scenarios) and the fused estimator step does not apply it");
+    if (env && env->log.rec)
+        return set_error("ozl_ekf_lee_landed_step: an episode log is registered (ozl_set_episode_log) and the fused estimator step writes no records");
     if (env && env->cfg.fault_mode == 2)
         return set_error("ozl_ekf_lee_landed_step: cfg.fault_mode 2 (multi-rotor faults) does not apply to the wrench-actuated step");
     return launch_ekf_lee(env, in, husky, StepIo{obs, rew, reset, progress, timeout, ep_ret}, stream);

@@ -52,7 +52,7 @@ struct ozl_env {
     int device;
     int sm_count;
     long long tma_min_tiles;    // >= this many whole tiles: use the persistent TMA-pipelined step kernel
-    long long tma_min_tiles_mf; // the same for the fault_mode 2 twins (the generic twin is resident 6 CTAs per SM, not 7)
+    long long tma_min_tiles_mf; // the same for the fault_mode 2 and episode-log twins (their generic twins are resident 6 CTAs per SM, not 7)
     long long early_draw_max_envs;  // <= this many envs: the generic step launches run quad_step_subwave_kernel
     void* arena;                // single cudaMalloc backing all planes
     size_t arena_bytes;
@@ -79,6 +79,9 @@ struct ozl_env {
     // fault_mode 2: the constants and the e_0..e_3 plane (MfCfg::eff4, in the arena) that the fault_mode 2 kernels take as
     // their last argument; eff4 is NULL for the other modes
     ozl::MfCfg mf;
+    // episode log (ozl_set_episode_log): the caller's records / head / capacity that the log twins take as their last argument;
+    // rec is NULL while no log is registered -- the step launches pick the log twins by this pointer
+    ozl::LogCfg log;
 };
 
 // Step launches go through cudaLaunchKernelEx so that they can carry the programmatic-stream-serialization attribute (PDL):

@@ -86,6 +86,69 @@ __device__ __forceinline__ void stage_states_row_mf(float* tile, int r, const fl
     row[4 * (5 ^ (r & 7))] = fminf(fmaxf(a[3], -c.clip_obs), c.clip_obs);
 }
 
+// Episode log (ozl_set_episode_log): the record of every env in `lanes` whose episode ended this step (`done`), from the post-step
+// registers; layout OZL_EPLOG_* (include/ouzelum_b200.h), CPU twin tests/episode_log_ref.py.  Every lane of `lanes` calls it: one
+// ballot, one atomic per warp on the head (its leader), each ending lane's row = the warp's base + its rank among them; the record
+// is eight 16-byte stores, one full 128-byte line.  MF: e_0..e_3 from `rf` (re-read from the lane where it is kept in memory).
+// RELOAD: the record's state fields are read back from the env's planes (pl, i), which this thread has just written with the step's
+// results -- so the generic twin need not keep them live in registers across its stores (at 72 / 85 registers it spilled otherwise).
+__device__ __forceinline__ float4 ld_own_v4(const float4* p) {   // after this thread's own stores to p: "memory" keeps the order
+    float4 v;
+    asm volatile("ld.global.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p) : "memory");
+    return v;
+}
+template <bool MF, bool RELOAD = false>
+__device__ __forceinline__ void log_episode(const LogCfg& lg, unsigned lanes, bool done, uint32_t genv, uint64_t step, const Env& e_reg,
+                                            const StepOut& o, const DevCfg& c, const RotorEff& rf, const Planes* pl = nullptr,
+                                            int64_t i = 0) {
+    const unsigned m = __ballot_sync(lanes, done);
+    if (m == 0u) return;
+    unsigned lt;
+    asm("mov.u32 %0, %%lanemask_lt;" : "=r"(lt));
+    const int leader = __ffs(m) - 1;
+    unsigned long long base = 0ull;
+    if ((lt & m) == 0u && done) base = atomicAdd(lg.head, (unsigned long long)__popc(m));
+    base = __shfl_sync(lanes, base, leader);
+    if (!done) return;
+    const unsigned long long row = base + (unsigned long long)__popc(m & lt);
+    if (row >= (unsigned long long)lg.cap) return;
+    Env e = e_reg;
+    if constexpr (RELOAD) {      // plane layout: internal.h (d0 {px,py,pz,qx} d1 {..,vx} d2 {vy,vz,..} s0 {tgt, eff} s1 s2)
+        const float4 d0 = ld_own_v4(plane4_ptr(*pl, 0, i)), d1 = ld_own_v4(plane4_ptr(*pl, 1, i)), d2 = ld_own_v4(plane4_ptr(*pl, 2, i));
+        const float4 s0 = ld_own_v4(plane4_ptr(*pl, 4, i)), s1 = ld_own_v4(plane4_ptr(*pl, 5, i)), s2 = ld_own_v4(plane4_ptr(*pl, 6, i));
+        e.p[0] = d0.x; e.p[1] = d0.y; e.p[2] = d0.z; e.v[0] = d1.w; e.v[1] = d2.x; e.v[2] = d2.y;
+        e.tgt[0] = s0.x; e.tgt[1] = s0.y; e.tgt[2] = s0.z; e.eff = s0.w;
+        e.mass = s1.x; e.ixx = s1.y; e.iyy = s1.z; e.izz = s1.w; e.arm = s2.x; e.ks = s2.y; e.fault = __float_as_uint(s2.z); e.km = s2.w;
+    }
+    const uint32_t onset = (e.fault & ~LANDED_BIT) >> 2;
+    float eff[4] = {1.0f, 1.0f, 1.0f, 1.0f};
+    if constexpr (MF) {
+        RotorEff rr = rf;
+        rfault_load(rr);
+        eff[0] = rr.e[0]; eff[1] = rr.e[1]; eff[2] = rr.e[2]; eff[3] = rr.e[3];
+    } else if (c.fault_mode && onset != FAULT_NEVER) {
+        const uint32_t rotor = e.fault & 3u;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) eff[j] = rotor == (uint32_t)j ? e.eff : 1.0f;
+    }
+    const float dx = e.tgt[0] - e.p[0], dy = e.tgt[1] - e.p[1], dz = e.tgt[2] - e.p[2];
+    const float dist = sqrtf((dx * dx + dy * dy) + dz * dz);              // as env_act_phase computes it
+    const uint32_t flags = (uint32_t)o.timeout | ((uint32_t)o.crash_dist << 1) | ((uint32_t)o.crash_z << 2) |
+                           ((e.fault & LANDED_BIT) ? 8u : 0u) | ((uint32_t)o.fault_active << 4);
+    static_assert(OZL_EPLOG_WIDTH == 32 && OZL_EPLOG_EFF == 8 && OZL_EPLOG_MASS == 12 && OZL_EPLOG_POS == 19 &&
+                  OZL_EPLOG_LINVEL == 22 && OZL_EPLOG_TARGET == 25 && OZL_EPLOG_RESERVED == 28, "record layout of the stores below");
+    float4* r = lg.rec + row * (OZL_EPLOG_WIDTH / 4);
+    r[0] = make_float4(__uint_as_float(genv), __int_as_float((int)o.prog), __uint_as_float((uint32_t)step),
+                       __uint_as_float((uint32_t)(step >> 32)));
+    r[1] = make_float4(o.ep_ret_done, __uint_as_float(flags), __int_as_float(onset == FAULT_NEVER ? -1 : (int)onset), dist);
+    r[2] = make_float4(eff[0], eff[1], eff[2], eff[3]);
+    r[3] = make_float4(e.mass, e.ixx, e.iyy, e.izz);
+    r[4] = make_float4(e.arm, e.ks, e.km, e.p[0]);
+    r[5] = make_float4(e.p[1], e.p[2], e.v[0], e.v[1]);
+    r[6] = make_float4(e.v[2], e.tgt[0], e.tgt[1], e.tgt[2]);
+    r[7] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+}
+
 // STATES: also write the privileged critic state (ozl_set_states_output) through `states_map`; the STATES = false instantiations
 // are the kernels without that output.  SCN: lay the scenario table `scn` (ozl_set_scenarios) over the reset draws; the body
 // is instantiated by two kernels, quad_step_kernel (no table, `scn` unused) and quad_step_scn_kernel.
@@ -93,6 +156,8 @@ __device__ __forceinline__ void stage_states_row_mf(float* tile, int r, const fl
 // every env draws the reset-path Philox numbers (ResetDraws) between the barrier and the first use of its state.
 // MF: fault_mode 2 (quad_step_mf_kernel / quad_step_mf_subwave_kernel): the env's lane of mf.eff4 (MfCfg, their last argument)
 // is read with its state and written back on a reset; the scenario row is read through `scn` when it is not NULL (SCN is true).
+// LOG: the episode log (quad_step_log_* kernels, LogCfg their last argument): the record of every episode that ends (log_episode);
+// the scenario row is read through `scn` when it is not NULL, as for MF.
 #define OZL_STEP_PARAMS                                                                                                         \
     const DevCfg c, const Planes pl, const float4* __restrict__ actions, float* __restrict__ obs, float* __restrict__ rew,       \
         int64_t* __restrict__ reset, int64_t* __restrict__ progress, uint8_t* __restrict__ timeout, float* __restrict__ ep_ret_out, \
@@ -100,9 +165,9 @@ __device__ __forceinline__ void stage_states_row_mf(float* tile, int r, const fl
         const int obs_bulk, const int64_t env0, const FrontArgs fa, volatile unsigned int* host_done, const unsigned int host_seq
 #define OZL_STEP_ARGS c, pl, actions, obs, rew, reset, progress, timeout, ep_ret_out, target_in, act_mode, done_u8, reset_mirror, \
                       obs_bulk, env0, fa, host_done, host_seq, states_map, scn
-template <int BLOCK, int FRONT, bool STATES, bool SCN, bool EARLY = false, bool MF = false>
+template <int BLOCK, int FRONT, bool STATES, bool SCN, bool EARLY = false, bool MF = false, bool LOG = false>
 __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMap& states_map, const float* __restrict__ scn,
-                                               const MfCfg& mf = MfCfg{}) {
+                                               const MfCfg& mf = MfCfg{}, const LogCfg& lg = LogCfg{}) {
     __shared__ __align__(16) float s_obs[BLOCK * 13];
     __shared__ __align__(1024) float s_states[STATES ? BLOCK * OZL_STATES_WIDTH : 4];
     __shared__ uint64_t s_step;
@@ -161,6 +226,9 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
         rst = rst_word != 0;
     }
     const ResetDraws* pre_p = EARLY ? &pre : nullptr;
+    constexpr bool OPT = MF || LOG;    // `scn` may be NULL
+    unsigned log_lanes = 0u;           // LOG: the warp's lanes with an env, which all enter the branch below
+    if constexpr (LOG) log_lanes = __ballot_sync(0xffffffffu, valid);
     if (valid) {
         Env e;
         unpack(L, e);
@@ -175,7 +243,7 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
         }
         float act[4] = {a4.x, a4.y, a4.z, a4.w};
         const uint32_t genv = c.env_id_base + (uint32_t)i;
-        const float* scn_row = SCN ? ((MF && !scn) ? nullptr : scn + i * OZL_SCENARIO_WIDTH) : nullptr;
+        const float* scn_row = SCN ? ((OPT && !scn) ? nullptr : scn + i * OZL_SCENARIO_WIDTH) : nullptr;
         RotorEff rf;
         if constexpr (MF) {
             rf.e[0] = ef.x; rf.e[1] = ef.y; rf.e[2] = ef.z; rf.e[3] = ef.w;
@@ -185,7 +253,7 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
         }
         RotorEff* rf_p = MF ? &rf : nullptr;
         if (FRONT == FRONT_LEE) {
-            const int64_t prog1 = env_reset_phase<SCN, MF>(e, prog, rst, genv, step, c, o, scn_row, pre_p, rf_p);
+            const int64_t prog1 = env_reset_phase<SCN, MF, OPT>(e, prog, rst, genv, step, c, o, scn_row, pre_p, rf_p);
             const float cmd[4] = {fa.cmd[0] * fa.g.scale[0], fa.cmd[1] * fa.g.scale[1], fa.cmd[2] * fa.g.scale[2], fa.cmd[3] * fa.g.scale[3]};
             float th, tq[3];
             lee_control(LEE_POSITION, e.p, e.q, e.v, e.w, cmd, fa.g, th, tq);                  // lee_landed.py:311
@@ -193,7 +261,7 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
             if (fa.wrench_out) fa.wrench_out[i] = make_float4(act[0], act[1], act[2], act[3]);
             env_act_phase<MF>(e, act, prog1, rst, genv, step, c, o, ACT_WRENCH, tptr, fa.cmd, rf_p);   // detector on the controller target, :305,318-322
         } else {
-            env_step<SCN, MF>(e, act, prog, rst, genv, step, c, o, act_mode, tptr, scn_row, pre_p, rf_p);
+            env_step<SCN, MF, OPT>(e, act, prog, rst, genv, step, c, o, act_mode, tptr, scn_row, pre_p, rf_p);
         }
         if constexpr (STATES && MF) stage_states_row_mf(s_states, threadIdx.x, o.obs, e, o, c, rf, act_mode == ACT_ROTORS);
         else if constexpr (STATES) stage_states_row(s_states, threadIdx.x, o.obs, e, o, c);
@@ -204,6 +272,7 @@ __device__ __forceinline__ void quad_step_body(OZL_STEP_PARAMS, const CUtensorMa
         if constexpr (MF) {
             if (EARLY && o.did_reset) mf.eff4[i] = make_float4(rf.e[0], rf.e[1], rf.e[2], rf.e[3]);
         }
+        if constexpr (LOG) log_episode<MF, !EARLY && !MF>(lg, log_lanes, o.reset, genv, step, e, o, c, rf, &pl, i);
         rew[i] = o.rew;
         reset[i] = o.reset ? 1 : 0;
         progress[i] = o.prog;
@@ -299,6 +368,35 @@ quad_step_mf_subwave_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap
                             const __grid_constant__ MfCfg mf) {
     quad_step_body<BLOCK, FRONT, STATES, true, true, true>(OZL_STEP_ARGS, mf);
 }
+// Episode-log twins of the four kernels above (ozl_set_episode_log), chosen by the launches exactly where they would choose their
+// counterpart whenever a log is registered; each serves with and without a scenario table (`scn` may be NULL).  The sub-wave and
+// mode-2 twins keep their counterparts' occupancy.  The generic twin re-reads the record's fields from the state it has just stored
+// (log_episode, RELOAD) and is bounded to 6 CTAs per SM like the mode-2 twin: at 7 (72 registers) it spills 12-44 bytes even so.
+// Launches with a log therefore switch to the TMA twin at the mode-2 threshold (ozl_env::tma_min_tiles_mf).
+template <int BLOCK, int FRONT, bool STATES>
+__global__ void __launch_bounds__(BLOCK, kStepMfMinBlocks)
+quad_step_log_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn,
+                     const __grid_constant__ LogCfg lg) {
+    quad_step_body<BLOCK, FRONT, STATES, true, false, false, true>(OZL_STEP_ARGS, MfCfg{}, lg);
+}
+template <int BLOCK, int FRONT, bool STATES>
+__global__ void __launch_bounds__(BLOCK, 1)
+quad_step_log_subwave_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn,
+                             const __grid_constant__ LogCfg lg) {
+    quad_step_body<BLOCK, FRONT, STATES, true, true, false, true>(OZL_STEP_ARGS, MfCfg{}, lg);
+}
+template <int BLOCK, int FRONT, bool STATES>
+__global__ void __launch_bounds__(BLOCK, kStepMfMinBlocks)
+quad_step_log_mf_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn,
+                        const __grid_constant__ MfCfg mf, const __grid_constant__ LogCfg lg) {
+    quad_step_body<BLOCK, FRONT, STATES, true, false, true, true>(OZL_STEP_ARGS, mf, lg);
+}
+template <int BLOCK, int FRONT, bool STATES>
+__global__ void __launch_bounds__(BLOCK, 4)
+quad_step_log_mf_subwave_kernel(OZL_STEP_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn,
+                                const __grid_constant__ MfCfg mf, const __grid_constant__ LogCfg lg) {
+    quad_step_body<BLOCK, FRONT, STATES, true, true, true, true>(OZL_STEP_ARGS, mf, lg);
+}
 
 // ------------------------------------------------------------------------------------------------ K1, TMA-pipelined
 // Persistent variant for large N (rotor-action mode, stored target): one CTA per (SM x 8) slot loops over tiles of
@@ -324,9 +422,10 @@ constexpr int kTmaMinBlocks = 5;       // CTAs per SM of the TMA kernel, and its
 // MF: fault_mode 2 (quad_step_tma_mf_kernel): thread 0 prefetches the next tile's 2 KiB of e_0..e_3 into L2 with one bulk prefetch
 // when it issues that tile's copies, and each thread reads its lane where it is used (RotorEff; a 2 KiB bulk copy into the stage
 // would leave room for 4 CTAs per SM, not 5, with the states tile); `scn` may be NULL.
-template <bool STATES, bool SCN, bool MF = false>
+// LOG: the episode log (quad_step_tma_log_kernel / quad_step_tma_log_mf_kernel); `scn` may be NULL.
+template <bool STATES, bool SCN, bool MF = false, bool LOG = false>
 __device__ __forceinline__ void quad_step_tma_body(OZL_TMA_PARAMS, const CUtensorMap& states_map, const float* __restrict__ scn,
-                                                   const MfCfg& mf = MfCfg{}) {
+                                                   const MfCfg& mf = MfCfg{}, const LogCfg& lg = LogCfg{}) {
     __shared__ __align__(128) unsigned char s_stage[kTmaStageBytes];
     __shared__ __align__(16) float s_obs[kTile * 13];
     __shared__ __align__(1024) float s_states[STATES ? kTile * OZL_STATES_WIDTH : 4];   // 16 KB: 5 CTAs/SM still fit
@@ -416,10 +515,12 @@ __device__ __forceinline__ void quad_step_tma_body(OZL_TMA_PARAMS, const CUtenso
             rf.i = i;
             rf.m = &mf;
         }
-        env_step<SCN, MF>(e, act, prog, rst, genv, step, c, o, ACT_ROTORS, nullptr,
-                          SCN ? ((MF && !scn) ? nullptr : scn + i * OZL_SCENARIO_WIDTH) : nullptr, nullptr, MF ? &rf : nullptr);
+        env_step<SCN, MF, MF || LOG>(e, act, prog, rst, genv, step, c, o, ACT_ROTORS, nullptr,
+                                     SCN ? (((MF || LOG) && !scn) ? nullptr : scn + i * OZL_SCENARIO_WIDTH) : nullptr, nullptr,
+                                     MF ? &rf : nullptr);
         if constexpr (STATES && MF) stage_states_row_mf(s_states, tid, o.obs, e, o, c, rf, true);
         else if constexpr (STATES) stage_states_row(s_states, tid, o.obs, e, o, c);
+        if constexpr (LOG) log_episode<MF>(lg, 0xffffffffu, o.reset, genv, step, e, o, c, rf);
         obs_epilogue(o.obs, genv, step, blackout, c);
         store_dynamic(pl, i, e);
         if (o.static_dirty) store_static(pl, i, e);
@@ -492,6 +593,19 @@ __global__ void __launch_bounds__(kTile, kTmaMinBlocks)
 quad_step_tma_mf_kernel(OZL_TMA_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn,
                         const __grid_constant__ MfCfg mf) {
     quad_step_tma_body<STATES, true, true>(OZL_TMA_ARGS, mf);
+}
+// episode-log twins (ozl_set_episode_log) of quad_step_tma_kernel / _scn_kernel and of quad_step_tma_mf_kernel
+template <bool STATES>
+__global__ void __launch_bounds__(kTile, kTmaMinBlocks)
+quad_step_tma_log_kernel(OZL_TMA_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn,
+                         const __grid_constant__ LogCfg lg) {
+    quad_step_tma_body<STATES, true, false, true>(OZL_TMA_ARGS, MfCfg{}, lg);
+}
+template <bool STATES>
+__global__ void __launch_bounds__(kTile, kTmaMinBlocks)
+quad_step_tma_log_mf_kernel(OZL_TMA_PARAMS, const __grid_constant__ CUtensorMap states_map, const float* __restrict__ scn,
+                            const __grid_constant__ MfCfg mf, const __grid_constant__ LogCfg lg) {
+    quad_step_tma_body<STATES, true, true, true>(OZL_TMA_ARGS, mf, lg);
 }
 
 // ------------------------------------------------------------------------------------------------ mode B
@@ -929,6 +1043,7 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
     memset(e->states_tmap, 0, sizeof(e->states_tmap));
     e->scn_buf = e->scn = nullptr;
     e->mf = MfCfg{};
+    e->log = LogCfg{};
     derive_dev_cfg(*cfg, e->dev);
     e->device = device;
     e->sm_count = prop.multiProcessorCount;
@@ -942,7 +1057,7 @@ extern "C" int ozl_create(const ozl_cfg* cfg, int device, ozl_env** out) {
         // (override: OZL_TMA_MIN_TILES, 0 = never)
         const char* ev = getenv("OZL_TMA_MIN_TILES");
         e->tma_min_tiles = ev ? atoll(ev) : (long long)kStepMinBlocks * prop.multiProcessorCount + 1;
-        // fault_mode 2: the generic twin holds 6 CTAs per SM (kStepMfMinBlocks), so its one-wave limit is lower
+        // fault_mode 2 or an episode log: the generic twins hold 6 CTAs per SM (kStepMfMinBlocks), so their one-wave limit is lower
         e->tma_min_tiles_mf = ev ? atoll(ev) : (long long)kStepMfMinBlocks * prop.multiProcessorCount + 1;
     }
     {   // up to one wave of quad_step_subwave_kernel (4 x 128-env CTAs per SM: 75776 envs on 148 SMs) the generic launch runs it.
@@ -1042,9 +1157,11 @@ static int launch_step_t(ozl_env* env, const float* actions, const float* target
     const bool plain = (target_in == nullptr) && act_mode == ACT_ROTORS && done_u8 == nullptr && reset_mirror == nullptr && obs_bulk;
     // cfg.fault_mode 2: the twins, which take MfCfg as one more argument and read the scenario row when `scn` is set
     const bool mf = env->cfg.fault_mode == 2;
+    // a registered episode log: the log twin of the kernel chosen otherwise, with LogCfg as its last argument
+    const bool lg = env->log.rec != nullptr;
     const auto kernel = SCN ? quad_step_scn_kernel<kStepBlock, FRONT_NONE, STATES> : quad_step_kernel<kStepBlock, FRONT_NONE, STATES>;
     const bool subwave = n <= env->early_draw_max_envs;
-    const long long tma_min_tiles = mf ? env->tma_min_tiles_mf : env->tma_min_tiles;
+    const long long tma_min_tiles = (mf || lg) ? env->tma_min_tiles_mf : env->tma_min_tiles;
     if (plain && tma_min_tiles > 0 && full_tiles >= tma_min_tiles &&
         !(((uintptr_t)progress | (uintptr_t)reset) & 15)) {
         // large N: persistent TMA-pipelined kernel over the whole tiles, then one generic block for the ragged tail
@@ -1054,16 +1171,20 @@ static int launch_step_t(ozl_env* env, const float* actions, const float* target
             return launch_pdl(k, dim3(grid), dim3(kTile), st, env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout,
                               ep_ret, full_tiles, states_map(env), (const float*)env->scn, mfa...);
         };
-        if (mf ? tma(quad_step_tma_mf_kernel<STATES>, env->mf) : tma(SCN ? quad_step_tma_scn_kernel<STATES> : quad_step_tma_kernel<STATES>))
-            return check_cuda(cudaGetLastError(), "quad_step_tma_kernel");
+        const int rc = !lg ? (mf ? tma(quad_step_tma_mf_kernel<STATES>, env->mf)
+                                 : tma(SCN ? quad_step_tma_scn_kernel<STATES> : quad_step_tma_kernel<STATES>))
+                           : (mf ? tma(quad_step_tma_log_mf_kernel<STATES>, env->mf, env->log) : tma(quad_step_tma_log_kernel<STATES>, env->log));
+        if (rc) return check_cuda(cudaGetLastError(), "quad_step_tma_kernel");
         const auto tail_block = [&](auto k, auto... mfa) {
             k<<<1, kStepBlock, 0, st>>>(env->dev, env->pl, (const float4*)actions, obs, rew, reset, progress, timeout, ep_ret, nullptr,
                                         ACT_ROTORS, nullptr, nullptr, 1, full_tiles * kTile, FrontArgs{}, (volatile unsigned int*)nullptr,
                                         0u, states_map(env), (const float*)env->scn, mfa...);
         };
         if (tail) {
-            if (mf) tail_block(quad_step_mf_kernel<kStepBlock, FRONT_NONE, STATES>, env->mf);
-            else tail_block(kernel);
+            if (!lg && mf) tail_block(quad_step_mf_kernel<kStepBlock, FRONT_NONE, STATES>, env->mf);
+            else if (!lg) tail_block(kernel);
+            else if (mf) tail_block(quad_step_log_mf_kernel<kStepBlock, FRONT_NONE, STATES>, env->mf, env->log);
+            else tail_block(quad_step_log_kernel<kStepBlock, FRONT_NONE, STATES>, env->log);
         }
         return check_cuda(cudaGetLastError(), "quad_step_kernel(tail)");
     }
@@ -1073,9 +1194,17 @@ static int launch_step_t(ozl_env* env, const float* actions, const float* target
                           (volatile unsigned int*)(host_flag ? env->host_done : nullptr), host_flag ? ++env->host_seq : 0u,
                           states_map(env), (const float*)env->scn, mfa...);
     };
-    const int rc = mf ? gen(subwave ? quad_step_mf_subwave_kernel<kStepBlock, FRONT_NONE, STATES> : quad_step_mf_kernel<kStepBlock, FRONT_NONE, STATES>,
-                            env->mf)
-                      : gen(subwave ? quad_step_subwave_kernel<kStepBlock, FRONT_NONE, STATES, SCN> : kernel);
+    int rc;
+    if (!lg)
+        rc = mf ? gen(subwave ? quad_step_mf_subwave_kernel<kStepBlock, FRONT_NONE, STATES> : quad_step_mf_kernel<kStepBlock, FRONT_NONE, STATES>,
+                      env->mf)
+                : gen(subwave ? quad_step_subwave_kernel<kStepBlock, FRONT_NONE, STATES, SCN> : kernel);
+    else if (mf)
+        rc = gen(subwave ? quad_step_log_mf_subwave_kernel<kStepBlock, FRONT_NONE, STATES> : quad_step_log_mf_kernel<kStepBlock, FRONT_NONE, STATES>,
+                 env->mf, env->log);
+    else
+        rc = gen(subwave ? quad_step_log_subwave_kernel<kStepBlock, FRONT_NONE, STATES> : quad_step_log_kernel<kStepBlock, FRONT_NONE, STATES>,
+                 env->log);
     if (rc) return check_cuda(cudaGetLastError(), "quad_step_kernel");
     return 0;
 }
@@ -1114,19 +1243,31 @@ static int launch_front_step(ozl_env* env, int front, const float* actions, cons
     (subwave ? (env->scn ? quad_step_subwave_kernel<kStepBlock, F, S, true> : quad_step_subwave_kernel<kStepBlock, F, S, false>) \
              : (env->scn ? quad_step_scn_kernel<kStepBlock, F, S> : quad_step_kernel<kStepBlock, F, S>))
 #define OZL_PICK_MF(F, S) (subwave ? quad_step_mf_subwave_kernel<kStepBlock, F, S> : quad_step_mf_kernel<kStepBlock, F, S>)
+#define OZL_PICK_LOG(F, S) (subwave ? quad_step_log_subwave_kernel<kStepBlock, F, S> : quad_step_log_kernel<kStepBlock, F, S>)
+#define OZL_PICK_LOG_MF(F, S) (subwave ? quad_step_log_mf_subwave_kernel<kStepBlock, F, S> : quad_step_log_mf_kernel<kStepBlock, F, S>)
     const auto go = [&](auto k, int mode, auto... mfa) {
         return launch_pdl(k, dim3(blocks_for(n, kStepBlock)), dim3(kStepBlock), st, env->dev, env->pl, (const float4*)actions, obs, rew,
                           reset, progress, timeout, ep_ret, (const float*)nullptr, mode, (uint8_t*)nullptr, (int64_t*)nullptr, 1, (int64_t)0,
                           fa, (volatile unsigned int*)nullptr, 0u, states_map(env), (const float*)env->scn, mfa...);
     };
     const bool mf = env->cfg.fault_mode == 2;          // the fault_mode 2 twins (FRONT_LEE: refused by ozl_lee_landed_step)
+    const bool lg = env->log.rec != nullptr;           // the episode-log twins
     int rc;
-    if (front == FRONT_VEHICLE && mf)
+    if (!lg && front == FRONT_VEHICLE && mf)
         rc = env->states ? go(OZL_PICK_MF(FRONT_VEHICLE, true), ACT_ROTORS, env->mf) : go(OZL_PICK_MF(FRONT_VEHICLE, false), ACT_ROTORS, env->mf);
-    else if (front == FRONT_VEHICLE)
+    else if (!lg && front == FRONT_VEHICLE)
         rc = env->states ? go(OZL_PICK(FRONT_VEHICLE, true), ACT_ROTORS) : go(OZL_PICK(FRONT_VEHICLE, false), ACT_ROTORS);
-    else
+    else if (!lg)
         rc = env->states ? go(OZL_PICK(FRONT_LEE, true), ACT_WRENCH) : go(OZL_PICK(FRONT_LEE, false), ACT_WRENCH);
+    else if (front == FRONT_VEHICLE && mf)
+        rc = env->states ? go(OZL_PICK_LOG_MF(FRONT_VEHICLE, true), ACT_ROTORS, env->mf, env->log)
+                         : go(OZL_PICK_LOG_MF(FRONT_VEHICLE, false), ACT_ROTORS, env->mf, env->log);
+    else if (front == FRONT_VEHICLE)
+        rc = env->states ? go(OZL_PICK_LOG(FRONT_VEHICLE, true), ACT_ROTORS, env->log) : go(OZL_PICK_LOG(FRONT_VEHICLE, false), ACT_ROTORS, env->log);
+    else
+        rc = env->states ? go(OZL_PICK_LOG(FRONT_LEE, true), ACT_WRENCH, env->log) : go(OZL_PICK_LOG(FRONT_LEE, false), ACT_WRENCH, env->log);
+#undef OZL_PICK_LOG_MF
+#undef OZL_PICK_LOG
 #undef OZL_PICK_MF
 #undef OZL_PICK
     if (rc) return check_cuda(cudaGetLastError(), who);
@@ -1233,6 +1374,7 @@ extern "C" int ozl_rollout(ozl_env* env, int32_t K, float* obs, float* rew, int6
     if (env->cfg.fault_mode == 2) return set_error("ozl_rollout: cfg.fault_mode 2 (multi-rotor faults) is not applied by the K-step kernel");
     if (env->states) return set_error("ozl_rollout: a states output is registered (ozl_set_states_output) and the K-step kernel does not write it");
     if (env->scn) return set_error("ozl_rollout: a scenario table is registered (ozl_set_scenarios) and the K-step kernel does not apply it");
+    if (env->log.rec) return set_error("ozl_rollout: an episode log is registered (ozl_set_episode_log) and the K-step kernel writes no records");
     if (!obs || !rew || !reset || !progress) return set_error("ozl_rollout: NULL buffer");
     quad_rollout_kernel<kStepBlock><<<blocks_for(env->cfg.num_envs, kStepBlock), kStepBlock, 0, st>>>(
         env->dev, env->pl, K, obs, rew, reset, progress);
@@ -1265,6 +1407,23 @@ extern "C" int ozl_set_states_output(ozl_env* env, float* states, int32_t width)
     if (r != CUDA_SUCCESS) return set_error("ozl_set_states_output: cuTensorMapEncodeTiled failed (%d)", (int)r);
     memcpy(env->states_tmap, m, sizeof(m));
     env->states = states;
+    return 0;
+}
+
+extern "C" int ozl_set_episode_log(ozl_env* env, float* records, int64_t capacity, uint64_t* head, int32_t width) {
+    if (!env) return set_error("ozl_set_episode_log: env is NULL");
+    if (width != OZL_EPLOG_WIDTH)
+        return set_error("ozl_set_episode_log: width %d != OZL_EPLOG_WIDTH (%d)", (int)width, (int)OZL_EPLOG_WIDTH);
+    if (!records) {
+        env->log = LogCfg{};
+        return 0;
+    }
+    if (capacity < 1) return set_error("ozl_set_episode_log: capacity %lld must be >= 1", (long long)capacity);
+    if ((uintptr_t)records & 15) return set_error("ozl_set_episode_log: records must be 16-byte aligned");
+    if (!head) return set_error("ozl_set_episode_log: head is NULL");
+    env->log.rec = reinterpret_cast<float4*>(records);
+    env->log.head = reinterpret_cast<unsigned long long*>(head);
+    env->log.cap = capacity;
     return 0;
 }
 

@@ -6,6 +6,7 @@ C ABI `ozl_set_scenarios`; row layout OZL_SCN_* in include/ouzelum_b200.h, `_lib
     result = scenarios.evaluate(env, lambda obs: policy(obs["obs"]), steps=4000)
 
 Two policies evaluated on the same table see the same faults, spawn poses and body parameters in every episode.
+`run_episodes(env, act_fn, steps)` returns the episode-log record (termination cause and conditions) of every episode of a run.
 """
 import itertools
 
@@ -48,6 +49,32 @@ def multi_fault_grid(n, effectiveness, onsets):
     rows = empty(n)
     rows[:, _RONSET:_REFF + 4] = grid[torch.arange(int(n)) % len(combos)]
     return rows
+
+
+def run_episodes(env, act_fn, steps, capacity=None):
+    """Run `steps` steps of `env` with actions `act_fn(obs_dict)` and return the episode-log records (`X500Task.episode_log`) of
+    every episode that ended during the run, concatenated in (step, env) order, with "dropped" 0.  An env ends at most one episode
+    per step, so the log (of `capacity` records, default 64 per env) is drained every capacity // num_envs steps and loses none.
+    A log the env had enabled is replaced by this run's and disabled at the end."""
+    n = env.num_envs
+    capacity = 64 * n if capacity is None else int(capacity)
+    if capacity < n:
+        raise ValueError(f"run_episodes: capacity {capacity} is below one record per env ({n})")
+    every = capacity // n
+    env.enable_episode_log(capacity)
+    parts = []
+    try:
+        obs = env.obs_dict if env.obs_dict else {"obs": env.obs_buf}
+        for t in range(int(steps)):
+            obs, _, _, _ = env.step(act_fn(obs))
+            if (t + 1) % every == 0:
+                parts.append(env.episode_log(clear=True))
+        parts.append(env.episode_log(clear=True))
+    finally:
+        env.disable_episode_log()
+    out = {k: torch.cat([p[k] for p in parts]) for k in parts[0] if k != "dropped"}
+    out["dropped"] = sum(p["dropped"] for p in parts)
+    return out
 
 
 def evaluate(env, act_fn, steps):

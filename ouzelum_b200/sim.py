@@ -88,6 +88,20 @@ class QuadSim:
         host = rows.detach().to("cpu").contiguous()
         check(lib.ozl_set_scenarios(self._h, host.data_ptr(), _lib.SCENARIO_WIDTH, _stream()), ValueError)
 
+    def set_episode_log(self, records, head):
+        """ozl_set_episode_log: every later step launch appends the record of each episode it ends to `records` ([capacity,
+        EPLOG_WIDTH] f32 CUDA tensor) and counts it in `head` (one int64 CUDA tensor, zeroed by the caller); both kept alive by the
+        caller.  records = None unregisters."""
+        if records is None:
+            check(lib.ozl_set_episode_log(self._h, None, 0, None, _lib.EPLOG_WIDTH), ValueError)
+            return
+        if records.dim() != 2 or records.shape[1] != _lib.EPLOG_WIDTH or records.dtype != torch.float32 \
+                or not records.is_contiguous() or records.device != self.device:
+            raise ValueError(f"records must be a contiguous float32 [capacity, {_lib.EPLOG_WIDTH}] tensor on {self.device}")
+        if head.numel() != 1 or head.dtype != torch.int64 or head.device != self.device:
+            raise ValueError(f"head must be one int64 element on {self.device}")
+        check(lib.ozl_set_episode_log(self._h, records.data_ptr(), records.shape[0], head.data_ptr(), _lib.EPLOG_WIDTH), ValueError)
+
     def rollout(self, k, obs, rew, reset, progress):
         check(lib.ozl_rollout(self._h, int(k), obs.data_ptr(), rew.data_ptr(), reset.data_ptr(), progress.data_ptr(),
                               _stream()))

@@ -32,6 +32,7 @@ class EKFLeeLanded(_VehicleTargetTask):
     land_cutoff = 0.25                                 # ekf_lee_landed.py:508
     supports_states = False                            # the fused estimator step kernel has no states output
     supports_scenarios = False                         # ... and does not apply a scenario table
+    supports_episode_log = False                       # ... and writes no episode records
 
     def __init__(self, cfg, *a, **k):
         env = cfg["env"]

@@ -97,6 +97,27 @@ def refuse_multi_fault(task_name, env_cfg):
         raise ValueError(f"{task_name}: rotorFault.mode 'multi' is not supported (its step does not apply per-rotor faults)")
 
 
+def decode_episode_records(rows):
+    """[k, EPLOG_WIDTH] float32 records (layout OZL_EPLOG_* in include/ouzelum_b200.h) -> dict of named tensors, sorted by (step,
+    env).  The row contents are deterministic; their order in the buffer is not."""
+    L = _lib.EPLOG_LAYOUT
+    bits = rows.view(torch.int32)
+    env = bits[:, L["OZL_EPLOG_ENV"]].long() & 0xFFFFFFFF
+    s = L["OZL_EPLOG_STEP"]
+    step = (bits[:, s + 1].long() << 32) | (bits[:, s].long() & 0xFFFFFFFF)
+    order = torch.argsort(env, stable=True)                    # two stable passes: env, then step (a packed key would overflow)
+    order = order[torch.argsort(step[order], stable=True)]
+    rows, bits, env, step = rows[order], bits[order], env[order], step[order]
+    flags = bits[:, L["OZL_EPLOG_FLAGS"]]
+    col = lambda name, k=1: rows[:, L[name]:L[name] + k].clone()
+    return {"env": env, "length": bits[:, L["OZL_EPLOG_LENGTH"]].long(), "step": step,
+            "return": rows[:, L["OZL_EPLOG_RETURN"]].clone(),
+            "timeout": (flags & 1) != 0, "crash_dist": (flags & 2) != 0, "crash_z": (flags & 4) != 0, "landed": (flags & 8) != 0,
+            "fault_active": (flags & 16) != 0, "onset": bits[:, L["OZL_EPLOG_ONSET"]].long(), "dist": rows[:, L["OZL_EPLOG_DIST"]].clone(),
+            "eff": col("OZL_EPLOG_EFF", 4), "params": col("OZL_EPLOG_MASS", 7), "pos": col("OZL_EPLOG_POS", 3),
+            "linvel": col("OZL_EPLOG_LINVEL", 3), "target": col("OZL_EPLOG_TARGET", 3)}
+
+
 def x500_cfg_from_task(cfg, num_envs, **over):
     """Translate the reference-style nested task dict into the C `ozl_cfg`."""
     env, sim = cfg["env"], cfg.get("sim", {})
@@ -148,6 +169,7 @@ class X500Task(VecTask):
     num_x500_actions = 4
     supports_states = True             # the step kernels can write the privileged critic state (ozl_set_states_output)
     supports_scenarios = True          # the step kernels can apply a scenario table at resets (ozl_set_scenarios)
+    supports_episode_log = True        # the step kernels can append a record per finished episode (ozl_set_episode_log)
 
     def __init__(self, cfg, rl_device, sim_device, graphics_device_id, headless,
                  virtual_screen_capture=False, force_render=False):
@@ -172,6 +194,7 @@ class X500Task(VecTask):
         self._graph = None
         self._static_actions = None
         self.scenarios = None          # the registered scenario table (CPU copy), see set_scenarios
+        self._eplog = None             # (records, head) of the episode log, see enable_episode_log
         self.use_cuda_graph = bool(self.cfg["env"].get("useCudaGraph", False))
 
     # ---- overridable pieces --------------------------------------------------------------------------
@@ -315,6 +338,47 @@ class X500Task(VecTask):
 
     def _check_scenarios(self, rows):
         """Task-specific refusals of a scenario table (the library validates the rows themselves)."""
+
+    # ---- episode log -------------------------------------------------------------------------------------------------------
+    def enable_episode_log(self, capacity):
+        """From now on every step appends one record per episode that ends -- termination cause, length, return, and the episode's
+        conditions (fault onset and per-rotor effectiveness, body parameters, final position, velocity and target) -- to a device
+        buffer of `capacity` records; `episode_log()` reads and clears it.  Records beyond the capacity are counted and dropped.
+        Re-captures this task's own step graph.  The log is not env state: checkpoints do not carry it."""
+        if not self.supports_episode_log:
+            raise ValueError(f"{type(self).__name__}: the episode log is not supported (its step kernel writes no records)")
+        capacity = int(capacity)
+        if capacity < 1:
+            raise ValueError(f"episode log capacity must be >= 1, got {capacity}")
+        records = torch.zeros(capacity, _lib.EPLOG_WIDTH, dtype=torch.float32, device=self.device)
+        head = torch.zeros(1, dtype=torch.int64, device=self.device)
+        self.sim.set_episode_log(records, head)
+        self._eplog = (records, head)
+        self._graph = None             # the captured step holds the kernels without (or with another) log
+
+    def disable_episode_log(self):
+        if self._eplog is None:
+            return
+        self.sim.set_episode_log(None, None)
+        self._eplog = None
+        self._graph = None
+
+    def episode_log(self, clear=True):
+        """The records since the last clearing read, as a dict of tensors on the env's device sorted by (step, env): "env",
+        "length", "step" (int64 [k]), "return", "dist" (float32 [k]), the causes "timeout", "crash_dist", "crash_z", "landed" and
+        "fault_active" (bool [k]), "onset" (int64 [k], -1: no fault scheduled), "eff" [k, 4], "params" [k, 7] (mass, ixx, iyy, izz,
+        arm, thrust scale, yaw_km), "pos", "linvel", "target" [k, 3]; and "dropped", the number of records the capacity lost.  One
+        host synchronisation; `clear` zeroes the count (stream-ordered)."""
+        if self._eplog is None:
+            raise ValueError("the episode log is not enabled (enable_episode_log)")
+        records, head = self._eplog
+        total = int(head.item())
+        k = min(total, records.shape[0])
+        out = decode_episode_records(records[:k])
+        if clear:
+            head.zero_()
+        out["dropped"] = total - k
+        return out
 
     def reset_idx(self, env_ids):
         """ouzelum.py:192-216.  The re-initialisation itself happens inside the next step's kernel (exactly when

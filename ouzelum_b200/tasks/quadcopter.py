@@ -45,8 +45,13 @@ class Quadcopter(VecTask):
         self._timeout_u8 = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
         self.timeout_buf = self._timeout_u8.view(torch.bool)
 
+    supports_episode_log = False       # its step kernel writes no episode records
+
     def set_scenarios(self, rows):
         raise ValueError("Quadcopter: scenario tables are not supported (its step kernel does not apply them)")
+
+    def enable_episode_log(self, capacity):
+        raise ValueError("Quadcopter: the episode log is not supported (its step kernel writes no records)")
 
     def create_sim(self):
         n, dev = self.num_envs, self.device
